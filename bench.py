@@ -329,6 +329,19 @@ def run_reference(args, rank, world):
     emit(line)
 
 
+def dump_last_step(out_dir, record, groups, frames, total, suffix=""):
+    """What lvo_step_batch_dev returned for the frames of the last timed step, as float64 .npy files: status[frame, context] and
+    odometry_pose / mapping_pose[frame, lane, 7] (q x, y, z, w, t x, y, z; lanes in context order).  Two builds run with the same
+    arguments see the same seeded sweeps, so their files can be compared array for array."""
+    ks = range(total - frames, total)
+    out = {"status": np.array([[record[(g, k)][0] for g in range(groups)] for k in ks], np.float64),
+           "odometry_pose": np.stack([np.concatenate([record[(g, k)][1] for g in range(groups)]) for k in ks]).astype(np.float64),
+           "mapping_pose": np.stack([np.concatenate([record[(g, k)][2] for g in range(groups)]) for k in ks]).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -383,6 +396,8 @@ def main():
     ap.add_argument("--only-knn", action="store_true", help="profiling aid: only the throughput-mode 5-NN measurement")
     ap.add_argument("--profile-iso", type=int, default=0, help="profiling aid: bracket this many of the isolated frames after the timed region with "
                     "cudaProfilerStart / cudaProfilerStop (use with `ncu --profile-from-start off`: nothing before them is profiled or serialised)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the status and poses the device-resident arm returned in its last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     F = max(1, args.frames_per_step)
@@ -562,18 +577,23 @@ def main():
             cs[g].set_option(L.LVO_OPT_FIXPOINT_SKIP, fixpoint_skip)
         return cs
 
-    def dev_stepper(cs):
+    def dev_stepper(cs, record=None):
         def step_dev(g, k):
             ptrs = [dev[(s_, k + o)].data_ptr() for s_, o in gplan[g]]
             ns = [dev[(s_, k + o)].shape[0] for s_, o in gplan[g]]
             st, odo, mp = cs[g].step_batch_dev(ptrs, ns)
             assert st >= 0
+            if record is not None and total - F <= k < total:
+                record[(g, k)] = (st, odo, mp)
         return step_dev
 
+    last_step = {} if args.dump_outputs else None
     ctx_d = make_dev_contexts(args.fixpoint_skip)
-    step_dev = dev_stepper(ctx_d)
+    step_dev = dev_stepper(ctx_d, last_step)
 
     ms_d, wall_d, launches, knn_ms_situ, knn_launches_situ, knn_bytes_situ = timed_run(step_dev, ctx_d)
+    if args.dump_outputs:
+        dump_last_step(args.dump_outputs, last_step, G, F, total, f"_rank{rank}" if world > 1 else "")
     st0 = ctx_d[0].stats(0)
     # outer iterations that ran in the last timed frame, mean over all lanes (10 = the reference's full schedule)
     ex = [(c.stats(l).odo_outer_executed, c.stats(l).map_outer_executed) for c in ctx_d for l in range(per)]
