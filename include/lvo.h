@@ -171,6 +171,26 @@ int lvo_step_batch_dev(lvo_ctx* ctx, const lvo_point* const* d_sweeps, const siz
                        lvo_pose* T_wmap_curr);
 int lvo_lane_status(const lvo_ctx* ctx, int lane);
 
+/* ---- per-lane lifecycle: sequences of unequal length, or started at different times, share one context ----- */
+
+/* Lane activity (default: every lane active).  The lvo_step_batch* calls skip an idle lane entirely: its sweep view / device
+ * pointer / count is not read, validated or uploaded (may be NULL / 0); its poses, odometry state and "last" clouds, map
+ * (both generations as seen through lvo_map_export / lvo_map_cloud), map correction, lvo_stats, probes, lvo_lane_status and
+ * skip_frame phase are left exactly as they were; its entries of T_wodom_curr / T_wmap_curr are not written; it does not
+ * contribute to the returned status.  A step in which no lane is active returns LVO_OK.  Resuming the lane continues its
+ * sequence bit for bit as if the idle steps had not happened.  Each lane maps on its own frames 0, skip_frame, 2 skip_frame, ...
+ * An idle lane is not free: its odometry grids are rebuilt and its map is copied into the other generation.  Measured on a B200
+ * (1000 W, 128 lanes): with 1/4, 1/2, 3/4 of the lanes idle a step takes 0.95, 0.77, 0.64 of its all-active time
+ * (profiles/lane_lifecycle.md); the cost of an idle lane by itself is not measured.
+ * LVO_E_STATE while an *_async step is in flight, LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid. */
+int lvo_set_lane_active(lvo_ctx* ctx, int lane, int active);
+/* Return `lane` to the state of a freshly created context: next active step is its first frame (LVO_W_FIRST_FRAME), empty map,
+ * identity poses and map correction, cen = (10, 10, 5), zero lvo_stats, status LVO_OK, skip_frame phase 0.  Other lanes are
+ * untouched, and so is the lane's activity.  Stream-ordered (returns when done); LVO_E_STATE while an *_async step is in flight,
+ * LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid.  To start a sequence from a pre-built map, follow it with
+ * lvo_map_import / lvo_set_odometry_state. */
+int lvo_lane_reset(lvo_ctx* ctx, int lane);
+
 /* ---- state export / import (SURVEY §5 "Checkpoint / resume"; needed to start from a pre-filled map) ------- */
 
 /* Replace the map of `lane` with the given cubes.  cube_ind[i] is the reference's array index

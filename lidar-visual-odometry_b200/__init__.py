@@ -87,7 +87,8 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_scan_to_map", "lvo_step_batch", "lvo_step_batch_dev", "lvo_lane_status", "lvo_map_import", "lvo_map_export",
            "lvo_get_map_correction", "lvo_set_map_correction", "lvo_set_odometry_state", "lvo_probe_fetch", "lvo_voxel_downsample", "lvo_knn",
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
-           "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait"]
+           "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
+           "lvo_lane_reset"]
 
 
 def load_library():
@@ -112,6 +113,8 @@ def load_library():
     L.lvo_step_batch_async.argtypes = [vp, C.POINTER(CloudView)]
     L.lvo_step_batch_dev_async.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.lvo_wait.argtypes = [vp, C.POINTER(Pose), C.POINTER(Pose)]
+    L.lvo_set_lane_active.argtypes = [vp, ip, ip]
+    L.lvo_lane_reset.argtypes = [vp, ip]
     L.lvo_map_import.argtypes = [vp, ip, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
     L.lvo_map_export.argtypes = [vp, ip, ip, C.POINTER(CloudOut), vp]
     L.lvo_map_cloud.argtypes = [vp, ip, ip, C.POINTER(CloudOut)]
@@ -241,13 +244,22 @@ class Lvo:
         r = self._check(self.lib.lvo_scan_to_map(self.h, *[v[0] for v in vs], C.byref(pin), C.byref(pout), C.byref(reg[0]) if reg else None))
         return r, pose_to_np(pout), (reg[1][:reg[0].n].copy() if reg else None)
 
-    # ---- batched device-resident pipeline
+    # ---- batched device-resident pipeline.  sweeps[l] may be None for an idle lane (set_lane_active); its pose rows come back NaN.
+    def _poses(self):
+        """Pose arrays for one step over NaN-filled numpy buffers (the library does not write the entries of idle lanes).  Filled
+        and read back as whole arrays: a per-pose Python loop would cost the timing loops of bench.py host time on every step."""
+        return tuple((Pose * self.lanes).from_buffer(np.full((self.lanes, 7), np.nan)) for _ in range(2))
+
+    @staticmethod
+    def _rows(po, pm):
+        return tuple(np.frombuffer(p, np.float64).reshape(-1, 7).copy() for p in (po, pm))
+
     def step_batch(self, sweeps):
         views = [view_of(s) for s in sweeps]
         arr = (CloudView * self.lanes)(*[v[0] for v in views])
-        po, pm = (Pose * self.lanes)(), (Pose * self.lanes)()
+        po, pm = self._poses()
         r = self._check(self.lib.lvo_step_batch(self.h, arr, po, pm))
-        return r, np.stack([pose_to_np(p) for p in po]), np.stack([pose_to_np(p) for p in pm])
+        return (r,) + self._rows(po, pm)
 
     def step_batch_async(self, sweeps):
         """Enqueue one frame and return; the arrays must stay alive and unchanged until wait()."""
@@ -256,10 +268,10 @@ class Lvo:
         return self._check(self.lib.lvo_step_batch_async(self.h, arr))
 
     def wait(self):
-        po, pm = (Pose * self.lanes)(), (Pose * self.lanes)()
+        po, pm = self._poses()
         r = self._check(self.lib.lvo_wait(self.h, po, pm))
         self._async_keep = None
-        return r, np.stack([pose_to_np(p) for p in po]), np.stack([pose_to_np(p) for p in pm])
+        return (r,) + self._rows(po, pm)
 
     def stage_timings(self):
         """{reference TicToc name: milliseconds} of the last plain-launch call, plus the three whole-stage times."""
@@ -277,19 +289,29 @@ class Lvo:
         if next_sweeps is not None:
             nviews = [view_of(s) for s in next_sweeps]
             nxt = (CloudView * self.lanes)(*[v[0] for v in nviews])
-        po, pm = (Pose * self.lanes)(), (Pose * self.lanes)()
+        po, pm = self._poses()
         r = self._check(self.lib.lvo_step_batch_pipelined(self.h, arr, nxt, po, pm))
-        return r, np.stack([pose_to_np(p) for p in po]), np.stack([pose_to_np(p) for p in pm])
+        return (r,) + self._rows(po, pm)
 
     def step_batch_dev(self, dev_ptrs, counts):
-        ptrs = (C.c_void_p * self.lanes)(*[int(p) for p in dev_ptrs])
-        ns = (C.c_size_t * self.lanes)(*[int(n) for n in counts])
-        po, pm = (Pose * self.lanes)(), (Pose * self.lanes)()
+        """dev_ptrs[l] / counts[l] may be None for an idle lane."""
+        ptrs = (C.c_void_p * self.lanes)(*[int(p or 0) for p in dev_ptrs])
+        ns = (C.c_size_t * self.lanes)(*[int(n or 0) for n in counts])
+        po, pm = self._poses()
         r = self._check(self.lib.lvo_step_batch_dev(self.h, ptrs, ns, po, pm))
-        return r, np.stack([pose_to_np(p) for p in po]), np.stack([pose_to_np(p) for p in pm])
+        return (r,) + self._rows(po, pm)
 
     def lane_status(self, lane):
         return self.lib.lvo_lane_status(self.h, lane)
+
+    # ---- per-lane lifecycle
+    def set_lane_active(self, lane, active):
+        """An idle lane is skipped by every step (its sweep may be None) and resumes its sequence bit for bit."""
+        self._check(self.lib.lvo_set_lane_active(self.h, lane, int(bool(active))))
+
+    def lane_reset(self, lane):
+        """Return `lane` to the first-frame state of a new context (empty map, identity poses, skip_frame phase 0)."""
+        self._check(self.lib.lvo_lane_reset(self.h, lane))
 
     # ---- state
     def map_import(self, lane, corner, corner_cube, surf, surf_cube):

@@ -28,7 +28,8 @@
 struct ExtractArgs {
   // input
   const unsigned char* const* in_ptr;  // [lanes] device pointers to raw point records
-  const int* in_n;                     // [lanes]
+  const int* in_n;                     // [lanes] (0 for an idle lane)
+  const int* lane_flags;               // [lanes] LVO_LANE_* of the step: the kernels below leave an idle lane's state alone
   int in_stride, in_off_xyz;
   int n_scans;
   float thres;                         // (float)MINIMUM_RANGE
@@ -82,7 +83,7 @@ __device__ __forceinline__ float3 load_xyz(const unsigned char* base, int stride
 
 __global__ void k_extract_reset(ExtractArgs a) {
   LaneState& s = a.ls[blockIdx.x];
-  if (threadIdx.x == 0) {
+  if (threadIdx.x == 0 && lane_active(a.lane_flags, blockIdx.x)) {
     s.n_in = a.in_n[blockIdx.x];
     s.first_kept = INT_MAX; s.last_kept = -1; s.switch_idx = INT_MAX; s.n_kept = 0;
     s.n_sharp = s.n_less_sharp = s.n_flat = s.n_less_flat = 0;
@@ -166,6 +167,7 @@ __global__ void k_ring_offsets(ExtractArgs a) {
   const int lane = blockIdx.x;
   LaneState& s = a.ls[lane];
   const int n = a.in_n[lane];
+  if (!lane_active(a.lane_flags, lane)) return;
   const int nblk = (n + LVO_EX_THREADS - 1) / LVO_EX_THREADS;
   const int r = threadIdx.x;  // 64 threads
   int run = 0;
@@ -233,9 +235,10 @@ __global__ void __launch_bounds__(LVO_EX_THREADS) k_ring_scatter(ExtractArgs a) 
 
 __global__ void __launch_bounds__(LVO_EX_THREADS) k_curvature(ExtractArgs a) {
   const int lane = blockIdx.y;
-  const int n = a.ls[lane].n_kept;
+  const int n = a.ls[lane].n_kept;                   // an idle lane's n_kept is its last frame's
+  const bool active = lane_active(a.lane_flags, lane);   // (loaded together with n_kept: no extra latency on the way to the work)
   const int i = blockIdx.x * LVO_EX_THREADS + threadIdx.x;
-  if (i >= n) return;
+  if (i >= n || !active) return;
   const float4* P = a.full + (size_t)lane * a.P;
   float c = 0.f;
   const float4 p0 = P[i];
@@ -402,6 +405,7 @@ __global__ void __launch_bounds__(LVO_SECSORT_THREADS, 4) k_sector_sort(ExtractA
   const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int S = s.scan_start[ring], E = s.scan_end[ring];
+  if (!lane_active(a.lane_flags, lane)) return;
   if (threadIdx.x == 0) a.lf_cnt[lane * LVO_MAX_RINGS + ring] = 0;
   if (threadIdx.x < LVO_SECTORS * 3) a.slot_cnt[sbase * 3 + threadIdx.x] = 0;
   const int RL = (E + 6) - (S - 5) + 1;          // the ring occupies [S - 5, E + 6]
@@ -449,7 +453,8 @@ __global__ void __launch_bounds__(LVO_PICKW_THREADS) k_sector_pick_warp(ExtractA
   if (ring >= a.n_scans) return;
   const LaneState& s = a.ls[lane];
   const int S = s.scan_start[ring], E = s.scan_end[ring];
-  if (E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
+  const bool active = lane_active(a.lane_flags, lane);
+  if (!active || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
   const size_t lo = (size_t)lane * a.P;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int R0 = S - 5, RL = (E + 6) - R0 + 1;
@@ -557,7 +562,8 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 5 : 3) k_lessflat_voxel(Extrac
   const int lane = blockIdx.y, ring = blockIdx.x;
   const LaneState& s = a.ls[lane];
   const int S = s.scan_start[ring], E = s.scan_end[ring];
-  if (E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
+  const bool active = lane_active(a.lane_flags, lane);
+  if (!active || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
   if (NT == 256 && E - S <= 2048) return;       // candidates come from [S, E - 1]: at most 2048 of them, the other instantiation's ring
   const size_t lo = (size_t)lane * a.P;
   const float4* P = a.full + lo;
@@ -699,6 +705,7 @@ __global__ void __launch_bounds__(LVO_PICK_THREADS) k_sector_pick(ExtractArgs a)
   __shared__ unsigned s_scan[33];
   __shared__ unsigned char s_picked[LVO_PICK_RING_SMEM];   // cloudNeighborPicked of this ring while the greedy picks run
   const int lane = blockIdx.y, ring = blockIdx.x;
+  const bool active = lane_active(a.lane_flags, lane);
   LaneState& s = a.ls[lane];
   const size_t lo = (size_t)lane * a.P;
   const float4* P = a.full + lo;
@@ -710,7 +717,7 @@ __global__ void __launch_bounds__(LVO_PICK_THREADS) k_sector_pick(ExtractArgs a)
   const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int S = s.scan_start[ring], E = s.scan_end[ring];
-  if (a.ring_done[lane * LVO_MAX_RINGS + ring]) return;   // handled by k_sector_pick_fast
+  if (!active || a.ring_done[lane * LVO_MAX_RINGS + ring]) return;   // idle lane / handled by k_sector_pick_fast
   if (threadIdx.x == 0) a.lf_cnt[lane * LVO_MAX_RINGS + ring] = 0;
   if (threadIdx.x < LVO_SECTORS * 3) a.slot_cnt[sbase * 3 + threadIdx.x] = 0;
   if (E - S < 6) return;  // :279-280
@@ -928,6 +935,7 @@ __global__ void __launch_bounds__(512) k_feature_compact(ExtractArgs a) {
   const size_t sb = (size_t)(lane * LVO_MAX_RINGS + r) * LVO_SECTORS;
   int c0 = 0, c1 = 0, c2 = 0;
   if (k < nsec) { const int* c = a.slot_cnt + (sb + j) * 3; c0 = c[0]; c1 = c[1]; c2 = c[2]; }
+  if (!lane_active(a.lane_flags, lane)) return;
   unsigned t0, t1, t2, tl;
   const unsigned o0 = block_excl_scan((unsigned)c0, sm, &t0);
   const unsigned o1 = block_excl_scan((unsigned)c1, sm, &t1);

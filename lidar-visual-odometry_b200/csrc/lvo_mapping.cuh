@@ -34,6 +34,7 @@
 struct MapArgs {
   LaneState* ls;
   int lanes, outer, from_odo;
+  const int* lane_flags;             // [lanes] LVO_LANE_* of the step: a lane without LVO_LANE_MAPS keeps its map, poses and counters
   float leaf[2];                     // lineRes, planeRes as float (setLeafSize takes floats)
   // inputs: corner_last / surf_last / full-res of this frame
   const float4* in_pts[2]; int in_cap[2];   // less_sharp [cap_lsharp], less_flat [P]; counts n_less_sharp / n_less_flat
@@ -74,6 +75,9 @@ __global__ void k_map_begin(MapArgs a) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
   if (lane >= a.lanes) return;
   LaneState& s = a.ls[lane];
+  // a lane that does not map in this step (idle, or off its skip_frame phase): k-NN, fit and solve return for it, the gather / stack /
+  // refilter / finish / register kernels see no items, and the rebuild carries its map into the other generation unchanged
+  if (!lane_maps(a.lane_flags, lane)) { s.map_done = 1; return; }
   if (a.from_odo) { for (int k = 0; k < 4; ++k) s.q_wodom[k] = s.q_w[k]; for (int k = 0; k < 3; ++k) s.t_wodom[k] = s.t_w[k]; }
   // transformAssociateToMap
   quat_mul(s.q_wmap_wodom, s.q_wodom, s.map_x);
@@ -120,7 +124,8 @@ __global__ void k_map_begin(MapArgs a) {
 __global__ void k_map_gather(MapArgs a) {
   const int v = blockIdx.x, lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
-  if (v >= s.n_valid) return;
+  const bool maps = lane_maps(a.lane_flags, lane);
+  if (v >= s.n_valid || !maps) return;
   const int c = s.valid_cube[v];
   const int i = c % LVO_CUBE_W - s.shift[0], j = (c / LVO_CUBE_W) % LVO_CUBE_H - s.shift[1], k = c / (LVO_CUBE_W * LVO_CUBE_H) - s.shift[2];
   if (!(i >= 0 && i < LVO_CUBE_W && j >= 0 && j < LVO_CUBE_H && k >= 0 && k < LVO_CUBE_D)) return;
@@ -140,7 +145,11 @@ __global__ void __launch_bounds__(256) k_stack_offsets(MapArgs a) {
   for (int base = 0; base < L2; base += blockDim.x) {
     const int lt = base + threadIdx.x;
     unsigned v = 0;
-    if (lt < L2) { const LaneState& s = a.ls[lt >> 1]; v = (unsigned)((lt & 1) ? s.n_less_flat : s.n_less_sharp); a.vx.seg_leaf[lt] = a.leaf[lt & 1]; }
+    if (lt < L2) {
+      const LaneState& s = a.ls[lt >> 1];
+      if (lane_maps(a.lane_flags, lt >> 1)) v = (unsigned)((lt & 1) ? s.n_less_flat : s.n_less_sharp);
+      a.vx.seg_leaf[lt] = a.leaf[lt & 1];
+    }
     unsigned tot;
     const unsigned ex = block_excl_scan(v, sm, &tot);
     if (lt < L2) a.item_off[lt] = acc + ex;
@@ -152,6 +161,7 @@ __global__ void k_stack_gather(MapArgs a) {
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
   const int n = t ? s.n_less_flat : s.n_less_sharp;
+  if (!lane_maps(a.lane_flags, lane)) return;
   const float4* src = a.in_pts[t] + (size_t)lane * a.in_cap[t];
   const unsigned off = a.item_off[lt];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -164,6 +174,7 @@ __global__ void k_stack_scatter(MapArgs a) {
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   LaneState& s = a.ls[lane];
   const unsigned b = a.vx.seg_out_start[lt], n = a.vx.seg_out_cnt[lt];
+  if (!lane_maps(a.lane_flags, lane)) return;   // keeps n_stack and the stack (parity probes) of the lane's last mapping step
   float4* dst = a.stack[t] + (size_t)lane * a.in_cap[t];
   for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = a.vx.out_pts[b + i];
   if (blockIdx.x == 0 && threadIdx.x == 0) {
@@ -580,7 +591,7 @@ __global__ void __launch_bounds__(512) k_map_qsort(MapArgs a) {
   const LaneState& s = a.ls[lane];
   const int n = s.n_stack[t];
   int* order = a.qorder[t] + (size_t)lane * a.in_cap[t];
-  if (s.map_too_small) return;
+  if (s.map_too_small || !lane_maps(a.lane_flags, lane)) return;
   if (n > LVO_QSORT_MAX) { for (int i = threadIdx.x; i < n; i += blockDim.x) order[i] = i; return; }
   const GridView g = grid_view(a.grid, 2 * lane + t);
   const float4* Q = a.stack[t] + (size_t)lane * a.in_cap[t];
@@ -672,7 +683,7 @@ __global__ void __launch_bounds__(128) k_map_fit(MapArgs a) {
 
 __global__ void k_map_finish(MapArgs a) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
-  if (lane >= a.lanes) return;
+  if (lane >= a.lanes || !lane_maps(a.lane_flags, lane)) return;
   LaneState& s = a.ls[lane];
   // transformUpdate :148-152: q_wmap_wodom = q_w_curr * q_wodom_curr.inverse(); t_wmap_wodom = t_w_curr - q_wmap_wodom * t_wodom_curr
   const double* q = s.q_wodom;
@@ -692,7 +703,7 @@ __global__ void __launch_bounds__(256) k_refilter_offsets(MapArgs a) {
   for (int base = 0; base < L2; base += blockDim.x) {
     const int lt = base + threadIdx.x;
     unsigned v = 0;
-    if (lt < L2) { const LaneState& s = a.ls[lt >> 1]; v = (unsigned)(s.from_off[lt & 1][LVO_MAX_VALID] + s.n_stack[lt & 1]); }
+    if (lt < L2 && lane_maps(a.lane_flags, lt >> 1)) { const LaneState& s = a.ls[lt >> 1]; v = (unsigned)(s.from_off[lt & 1][LVO_MAX_VALID] + s.n_stack[lt & 1]); }
     unsigned tot;
     const unsigned ex = block_excl_scan(v, sm, &tot);
     if (lt < L2) a.item_off[lt] = acc + ex;
@@ -704,6 +715,7 @@ __global__ void k_refilter_gather(MapArgs a) {
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
   const int nfrom = s.from_off[t][LVO_MAX_VALID], nst = s.n_stack[t];
+  if (!lane_maps(a.lane_flags, lane)) return;
   const unsigned off = a.item_off[lt];
   const float4* FM = a.from_map[t] + (size_t)lane * a.map_cap[t];
   const float4* ST = a.stack[t] + (size_t)lane * a.in_cap[t];
@@ -745,15 +757,17 @@ __global__ void k_rebuild_appended(MapArgs a) {
     atomicMin(&a.app_first[(size_t)lt * LVO_NCUBES + cube], b + i);
   }
 }
-// one block per (lane, type): new per-cube counts and their exclusive scan
+// one block per (lane, type): new per-cube counts and their exclusive scan.  A lane that does not map in this step counts as having
+// no valid cube (its n_valid / valid_cube stay for lvo_map_cloud) and no shift (k_map_end left it 0): its map passes through unchanged.
 __global__ void __launch_bounds__(256) k_rebuild_offsets(MapArgs a) {
   __shared__ unsigned sm[33];
   __shared__ signed char vrank[LVO_NCUBES];
   const int lt = blockIdx.x, lane = lt >> 1, t = lt & 1;
   LaneState& s = a.ls[lane];
+  const bool maps = lane_maps(a.lane_flags, lane);
   for (int c = threadIdx.x; c < LVO_NCUBES; c += blockDim.x) vrank[c] = -1;
   __syncthreads();
-  if (threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
+  if (maps && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
   __syncthreads();
   const unsigned* cs = a.cube_start[a.gen][t] + (size_t)lane * (LVO_NCUBES + 1);
   unsigned* ncs = a.cube_start[a.gen ^ 1][t] + (size_t)lane * (LVO_NCUBES + 1);
@@ -780,6 +794,7 @@ __global__ void __launch_bounds__(256) k_rebuild_offsets(MapArgs a) {
   if (threadIdx.x == 0) {
     const unsigned kept = min(carry, (unsigned)a.map_cap[t]);
     ncs[LVO_NCUBES] = kept;
+    if (!maps) return;
     s.n_map[t] = (int)kept;
     if (t == 0) s.stats.map_corner_total = (int)kept; else s.stats.map_surf_total = (int)kept;
     if (carry > (unsigned)a.map_cap[t]) s.map_status = LVO_E_CAPACITY;
@@ -790,9 +805,10 @@ __global__ void __launch_bounds__(256) k_rebuild_copy(MapArgs a) {
   __shared__ signed char vrank[LVO_NCUBES];
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
+  const bool maps = lane_maps(a.lane_flags, lane);   // see k_rebuild_offsets
   for (int c = threadIdx.x; c < LVO_NCUBES; c += blockDim.x) vrank[c] = -1;
   __syncthreads();
-  if (threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
+  if (maps && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
   __syncthreads();
   const unsigned* cs = a.cube_start[a.gen][t] + (size_t)lane * (LVO_NCUBES + 1);
   const unsigned* ncs = a.cube_start[a.gen ^ 1][t] + (size_t)lane * (LVO_NCUBES + 1);
@@ -827,6 +843,7 @@ __global__ void k_register(MapArgs a) {
   const int lane = blockIdx.y;
   const LaneState& s = a.ls[lane];
   const int n = s.n_kept;
+  if (!lane_maps(a.lane_flags, lane)) return;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
     a.registered[(size_t)lane * a.P + i] = transform_point(s.map_x, s.map_x + 4, a.full[(size_t)lane * a.P + i]);
 }

@@ -26,6 +26,7 @@ struct OdoArgs {
   int fast_h;        // widest azimuth half-window (buckets) the thread-per-feature kernel scans itself (16; LVO_FAST_H overrides)
   int lane0;         // first lane of an association launch (chunked outer loop, see lvo_launch_odometry)
   int distortion;    // 0 | 1 | 2, see the header comment
+  const int* lane_flags;   // [lanes] LVO_LANE_* of the step: an idle lane's pose, "last" clouds, status and stats are left alone
   // current features (stride caps)
   const float4* sharp; float4* less_sharp; const float4* flat; float4* less_flat;
   float4* full;      // [lanes][P] ring-ordered full-resolution cloud (only touched by k_odo_to_end)
@@ -101,6 +102,7 @@ __global__ void k_odo_begin(OdoArgs a) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
   if (lane >= a.lanes) return;
   LaneState& s = a.ls[lane];
+  if (!lane_active(a.lane_flags, lane)) { s.odo_done = 1; return; }   // idle: the association and solve kernels return at once
   s.odo_status = s.odo_inited ? LVO_OK : LVO_W_FIRST_FRAME;
   s.odo_done = 0; s.stats.odo_outer_executed = 0;
   for (int o = 0; o < LVO_MAX_OUTER; ++o) { s.stats.odo_corner_corr[o] = 0; s.stats.odo_plane_corr[o] = 0; s.stats.odo_lm_iters[o] = 0; s.stats.odo_final_cost[o] = 0; s.stats.odo_slow[o] = 0; s.stats.odo_certified[o] = 0; }
@@ -723,7 +725,7 @@ __global__ void __launch_bounds__(256, 4) k_odo_assoc(OdoArgs a) {
 // after the outer loop: few-correspondence warning (:566-568), pose integration (:581-582)
 __global__ void k_odo_integrate(OdoArgs a, int outer_iters) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
-  if (lane >= a.lanes) return;
+  if (lane >= a.lanes || !lane_active(a.lane_flags, lane)) return;
   LaneState& s = a.ls[lane];
   if (s.odo_inited) {
     for (int o = 0; o < outer_iters; ++o)
@@ -745,6 +747,7 @@ __global__ void k_odo_to_end(OdoArgs a) {
   const int lane = blockIdx.y;
   const LaneState& s = a.ls[lane];
   const int n0 = s.n_less_sharp, n1 = s.n_less_flat, n2 = s.n_kept;
+  if (!lane_active(a.lane_flags, lane)) return;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n0 + n1 + n2; i += gridDim.x * blockDim.x) {
     float4* p = i < n0 ? a.less_sharp + (size_t)lane * a.cap_lsharp + i
                        : (i < n0 + n1 ? a.less_flat + (size_t)lane * a.P + (i - n0) : a.full + (size_t)lane * a.P + (i - n0 - n1));
@@ -757,6 +760,7 @@ __global__ void k_odo_swap(OdoArgs a) {
   const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
   const int nc = s.n_corner_last, nsf = s.n_surf_last;
+  if (!lane_active(a.lane_flags, lane)) return;
   const int stride = gridDim.x * blockDim.x;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nc + nsf; i += stride) {
     const bool corner = i < nc;
@@ -814,5 +818,6 @@ static inline void lvo_launch_odometry(cudaStream_t st, OdoArgs a, const SolveAr
   if (a.distortion == 2) { k_odo_to_end<<<dim3(64, lanes), 256, 0, st>>>(a); if (launches) *launches += 1; }
   k_odo_swap<<<dim3(32, lanes), 256, 0, st>>>(a);
   if (launches) *launches += 2;
+  // every lane's grids, an idle lane's included (rebuilt from its unchanged "last" clouds: the problem offsets are shared by all lanes)
   lvo_grid_build(st, a.grid, launches);
 }
