@@ -19,7 +19,6 @@ LVO_W_FIRST_FRAME, LVO_W_FEW_CORR, LVO_W_MAP_TOO_SMALL = 1, 2, 3
 LVO_OPT_GRAPHS = 1
 LVO_OPT_FIXPOINT_SKIP = 2
 LVO_OPT_STAGE_TIMING = 3
-LVO_OPT_KNN_TILE = 4
 LVO_OPT_KNN_REUSE = 5
 LVO_OPT_ODO_REUSE = 6
 

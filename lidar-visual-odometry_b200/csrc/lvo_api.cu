@@ -475,7 +475,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   od.factor_cap = std::max(c->cap_sharp + c->cap_flat, c->cap_lsharp + P);
   LVO_TRY(dalloc(c, &od.factors, (size_t)L * od.factor_cap));
   LVO_TRY(dalloc(c, &od.slow_list, (size_t)L * (c->cap_sharp + c->cap_flat))); LVO_TRY(dalloc(c, &od.slow_cnt, (size_t)L));
-  { const char* e = getenv("LVO_ODO_REUSE"); od.reuse = e ? atoi(e) : 1; }   // default: correspondences carried across the outer iterations with a certificate
+  od.reuse = 1;   // default: correspondences carried across the outer iterations with a certificate
   LVO_TRY(dalloc(c, &od.ref, (size_t)L * (c->cap_sharp + c->cap_flat))); LVO_TRY(dalloc(c, &od.guard, (size_t)L * (c->cap_sharp + c->cap_flat)));
   LVO_TRY(dalloc(c, &od.sel, (size_t)L * (c->cap_sharp + c->cap_flat)));
   LVO_TRY(dalloc(c, &od.corner_corr, (size_t)L * slots * c->cap_sharp * 2));
@@ -490,9 +490,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   mp.ls = c->d_ls; mp.lanes = L; mp.lane_flags = ex.lane_flags; mp.leaf[0] = (float)cfg->line_res; mp.leaf[1] = (float)cfg->plane_res;
   mp.in_pts[0] = ex.less_sharp; mp.in_pts[1] = ex.less_flat; mp.in_cap[0] = c->cap_lsharp; mp.in_cap[1] = P;
   mp.full = ex.full; mp.P = P; mp.gen = 0; mp.slots = slots;
-  { const char* e = getenv("LVO_KNN_TILE"); mp.knn_tile = e ? atoi(e) : 0; }   // default: thread-per-query search (faster on sweep-shaped query sets, profiles/r2_summary.md)
-  { const char* e = getenv("LVO_KNN_REUSE"); mp.knn_reuse = e ? atoi(e) : 1; }   // default: neighbour sets carried across the outer iterations with a certificate
-  lvo_mapping_kernel_attributes();
+  mp.knn_reuse = 1;   // default: neighbour sets carried across the outer iterations with a certificate
   lvo_extract_kernel_attributes();
   for (int t = 0; t < 2; ++t) {
     mp.map_cap[t] = mapc[t];
@@ -504,7 +502,6 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
     LVO_TRY(dalloc(c, &mp.stack[t], (size_t)L * mp.in_cap[t]));
     LVO_TRY(dalloc(c, &mp.knn_ind[t], (size_t)L * slots * mp.in_cap[t] * 5));
     LVO_TRY(dalloc(c, &mp.fac_valid[t], (size_t)L * slots * mp.in_cap[t]));
-    LVO_TRY(dalloc(c, &mp.qorder[t], (size_t)L * mp.in_cap[t]));
     LVO_TRY(dalloc(c, &mp.knn_ref[t], (size_t)L * mp.in_cap[t], false));
     LVO_TRY(dalloc(c, &mp.knn_sel[t], (size_t)L * mp.in_cap[t] * 5, false));
     LVO_TRY(dalloc(c, &mp.knn_flag[t], (size_t)L * mp.in_cap[t], false));
@@ -574,12 +571,6 @@ int lvo_set_option(lvo_ctx* c, int option, int value) {
   if (!c) return LVO_E_BADARG;
   if (option == LVO_OPT_GRAPHS) { c->opt_graphs = value; return LVO_OK; }
   if (option == LVO_OPT_STAGE_TIMING) { c->opt_stage_timing = value ? 1 : 0; return LVO_OK; }
-  if (option == LVO_OPT_KNN_TILE) {   // a kernel choice baked into captured graphs
-    if (c->st) cudaStreamSynchronize(c->st);
-    destroy_graphs(c);
-    c->map.knn_tile = value ? 1 : 0;
-    return LVO_OK;
-  }
   if (option == LVO_OPT_ODO_REUSE) {
     if (c->st) cudaStreamSynchronize(c->st);
     destroy_graphs(c);
@@ -740,15 +731,11 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
   if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
   c->launches = 0;
   LVO_TRY(enqueue_prefetch(c));
-  // LVO_STAGE_MASK (profiling aid, environment only): bit 0 extract, bit 1 scan-to-scan, bit 2 scan-to-map; stages left out are not
-  // enqueued, so the saturated throughput of a prefix of the chain can be measured (results are only meaningful with the default 7)
-  static int stage_mask = -1;
-  if (stage_mask < 0) { const char* e = getenv("LVO_STAGE_MASK"); stage_mask = e ? atoi(e) : 7; }
   // a lane maps on its own frames 0, skip_frame, 2 skip_frame, ... (laserOdometry.cpp:643); the mapping stage is enqueued when any
   // lane maps, and the kernels pass the others through (LVO_LANE_MAPS)
   bool do_map = false;
   for (int l = 0; l < c->lanes; ++l) {
-    const bool maps = c->lane_active[l] && (c->lane_frame[l] % c->cfg.skip_frame) == 0 && (stage_mask & 4);
+    const bool maps = c->lane_active[l] && (c->lane_frame[l] % c->cfg.skip_frame) == 0;
     lane_flags(c)[l] = (c->lane_active[l] ? LVO_LANE_ACTIVE : 0) | (maps ? LVO_LANE_MAPS : 0);
     do_map = do_map || maps;
   }
@@ -785,10 +772,10 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
   } else {
     LvoStageTimer* tm = stage_timer_begin(c, c->opt_stage_timing != 0);
     cudaEventRecord(c->ev[0], c->st);
-    if (stage_mask & 1) enqueue_extract(c, stride, off_xyz, max_n, tm);
+    enqueue_extract(c, stride, off_xyz, max_n, tm);
     cudaEventRecord(c->ev[1], c->st);
     c->solve.trace = c->d_trace[0];
-    if (stage_mask & 2) enqueue_odometry(c, tm);
+    enqueue_odometry(c, tm);
     cudaEventRecord(c->ev[2], c->st);
     if (do_map) { c->solve.trace = c->d_trace[1]; enqueue_mapping(c, 1, true, tm); }
     c->stage_tm.stop(c->st);

@@ -23,7 +23,6 @@
 #pragma once
 #include "lvo_internal.h"
 #include "lvo_knn.cuh"
-#include "lvo_knn_tile.cuh"
 #include "lvo_solver.cuh"
 #include "lvo_voxel.cuh"
 
@@ -57,8 +56,6 @@ struct MapArgs {
   int* knn_ind[2];                   // [type] -> [lanes][slots][in_cap[type]][5]
   int* fac_valid[2];                 // [type] -> [lanes][slots][in_cap[type]]
   int slots;                         // outer-iteration slots kept (LVO_MAX_OUTER with lvo_config::debug_probes, else 2)
-  int* qorder[2];                    // [type] -> [lanes][in_cap[type]] stack indices in map-cell order (k_map_qsort)
-  int knn_tile;                      // LVO_OPT_KNN_TILE
   // LVO_OPT_KNN_REUSE: certified reuse of a query's neighbour set across the outer iterations of a frame (k_map_knn_reuse)
   int knn_reuse;
   float4* knn_ref[2];                // [type] -> [lanes][in_cap[type]] query position of the last full search (x, y, z) and its guard radius (w)
@@ -583,70 +580,6 @@ __global__ void __launch_bounds__(128) k_map_fit_reuse(MapArgs a) {
   }
 }
 
-// Order of the queries for the tiled search: stack indices sorted by the map-grid cell (z, y, x) of the point under the frame's INITIAL
-// pose.  One CTA per (lane, type), register bitonic sort of (cell key, index); stacks beyond LVO_QSORT_MAX keep their order.
-__global__ void __launch_bounds__(512) k_map_qsort(MapArgs a) {
-  extern __shared__ unsigned long long qs_buf[];   // pad16(LVO_QSORT_MAX) exchange buffer of bitonic_regs16
-  const int t = blockIdx.x, lane = blockIdx.y;
-  const LaneState& s = a.ls[lane];
-  const int n = s.n_stack[t];
-  int* order = a.qorder[t] + (size_t)lane * a.in_cap[t];
-  if (s.map_too_small || !lane_maps(a.lane_flags, lane)) return;
-  if (n > LVO_QSORT_MAX) { for (int i = threadIdx.x; i < n; i += blockDim.x) order[i] = i; return; }
-  const GridView g = grid_view(a.grid, 2 * lane + t);
-  const float4* Q = a.stack[t] + (size_t)lane * a.in_cap[t];
-  int npad = 16; while (npad < n) npad <<= 1;
-  unsigned long long k[16];
-  const int e0 = (int)threadIdx.x * 16;
-#pragma unroll
-  for (int r = 0; r < 16; ++r) {
-    const int i = e0 + r;
-    unsigned long long key = ~0ull;
-    if (i < n) {
-      const float4 sel = transform_point(s.map_x, s.map_x + 4, Q[i]);
-      int cx = cell_coord(sel.x, g.inv_cell) - g.org[0], cy = cell_coord(sel.y, g.inv_cell) - g.org[1], cz = cell_coord(sel.z, g.inv_cell_z) - g.org[2];
-      cx = min(max(cx, 0), max(g.dim[0] - 1, 0)); cy = min(max(cy, 0), max(g.dim[1] - 1, 0)); cz = min(max(cz, 0), max(g.dim[2] - 1, 0));
-      key = ((unsigned long long)(unsigned)((cz * g.dim[1] + cy) * g.dim[0] + cx) << 32) | (unsigned)i;
-    }
-    k[r] = key;
-  }
-  bitonic_regs16<false>(k, npad, qs_buf);
-#pragma unroll
-  for (int r = 0; r < 16; ++r) if (e0 + r < n) order[e0 + r] = (int)(unsigned)(k[r] & 0xffffffffull);
-}
-
-// The graded 5-NN kernel, tiled form (lvo_knn_tile.cuh): a warp per 32 queries of the cell-sorted order, candidates staged in shared
-// memory by bulk asynchronous copies.  Same index sets as k_map_knn bit for bit.
-__global__ void __launch_bounds__(LVO_KT_WARPS * 32, 2) k_map_knn_tile(MapArgs a) {
-  extern __shared__ __align__(16) unsigned char kt_raw[];
-  KtWarpSmem& sm = *kt_setup(kt_raw);
-  unsigned phase = 0;
-  const int lane = blockIdx.y;
-  const LaneState& s = a.ls[lane];
-  if (s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
-  const int n0 = s.n_stack[0], n1 = s.n_stack[1];
-  const int c0 = (n0 + 31) >> 5, c1 = (n1 + 31) >> 5;
-  const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
-  for (int c = blockIdx.x * LVO_KT_WARPS + (int)w; c < c0 + c1; c += gridDim.x * LVO_KT_WARPS) {
-    const int t = c >= c0 ? 1 : 0;
-    const int i = ((t ? c - c0 : c) << 5) + (int)ln;
-    const bool have = i < (t ? n1 : n0);
-    int qi = 0;
-    float4 sel = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (have) {
-      qi = a.qorder[t][(size_t)lane * a.in_cap[t] + i];
-      sel = transform_point(s.map_x, s.map_x + 4, a.stack[t][(size_t)lane * a.in_cap[t] + qi]);
-    }
-    TopK<5> tk;
-    bool ok;
-    kt_warp_search(grid_view(a.grid, 2 * lane + t), sm, phase, have, sel.x, sel.y, sel.z, 1.0f, tk, ok);
-    if (have) {
-      int* ki = a.knn_ind[t] + (((size_t)lane * a.slots + a.outer % a.slots) * a.in_cap[t] + qi) * 5;
-#pragma unroll
-      for (int k = 0; k < 5; ++k) ki[k] = ok ? tk.id[k] : -1;
-    }
-  }
-}
 // line / plane fit of every accepted query (one thread per query) -> factor records
 __global__ void __launch_bounds__(128) k_map_fit(MapArgs a) {
   const int lane = blockIdx.y;
@@ -848,12 +781,6 @@ __global__ void k_register(MapArgs a) {
     a.registered[(size_t)lane * a.P + i] = transform_point(s.map_x, s.map_x + 4, a.full[(size_t)lane * a.P + i]);
 }
 
-// once per process and device, before the first launch (dynamic shared memory above 48 KB needs the opt-in)
-static inline void lvo_mapping_kernel_attributes() {
-  cudaFuncSetAttribute(k_map_qsort, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((LVO_QSORT_MAX + LVO_QSORT_MAX / 16) * sizeof(unsigned long long)));
-  cudaFuncSetAttribute(k_map_knn_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LVO_KT_SMEM_BYTES);
-}
-
 static inline void lvo_launch_mapping(cudaStream_t st, MapArgs a, const SolveArgs& solve_proto, int outer_iters, int lanes, bool want_registered,
                                       long long* launches, LvoStageTimer* tm = nullptr) {
   const int L2 = 2 * lanes;
@@ -869,30 +796,22 @@ static inline void lvo_launch_mapping(cudaStream_t st, MapArgs a, const SolveArg
   if (launches) *launches += 1;
   LVO_MARK(tm, LVO_ST_MAP_TREE, st);
   lvo_grid_build(st, a.grid, launches);
-  // a.knn_tile (LVO_OPT_KNN_TILE): the shared-memory tiled search instead of the thread-per-query one (same results bit for bit)
-  const int knn_tile = a.knn_tile;
-  if (knn_tile) {
-    k_map_qsort<<<dim3(2, lanes), 512, (LVO_QSORT_MAX + LVO_QSORT_MAX / 16) * sizeof(unsigned long long), st>>>(a);
-    if (launches) *launches += 1;
-  }
   const int nstack_cap = a.in_cap[0] + a.in_cap[1];
   dim3 ga(max(1, min(lvo_div_up(nstack_cap, 128), 128)), lanes);
-  dim3 gt(max(20, min(lvo_div_up(lvo_div_up(nstack_cap, 32) + 1, LVO_KT_WARPS), 592 / lanes)), lanes);
   // The reuse kernels loop over a lane's queries with few blocks: a stack holds ~4 k points (capacity 139 k), and every block of a
   // capacity-sized grid pays the dependent loads of the lane state before it can exit (16 384 blocks cost ~50 us when all of them are idle).
   dim3 gr(max(1, min(lvo_div_up(nstack_cap, 128), 32)), lanes), gf(max(1, min(lvo_div_up(nstack_cap, 128), 8)), lanes), gf2(max(1, min(lvo_div_up(nstack_cap, 128), 16)), lanes);
   for (int o = 0; o < outer_iters; ++o) {
     a.outer = o;
     LVO_MARK(tm, LVO_ST_MAP_KNN, st);
-    if (knn_tile) k_map_knn_tile<<<gt, LVO_KT_WARPS * 32, LVO_KT_SMEM_BYTES, st>>>(a);
-    else if (a.knn_reuse) k_map_knn_reuse<<<gr, 128, 0, st>>>(a);
+    if (a.knn_reuse) k_map_knn_reuse<<<gr, 128, 0, st>>>(a);
     else k_map_knn<<<ga, 128, 0, st>>>(a);
     LVO_MARK(tm, LVO_ST_MAP_FIT, st);
-    if (!knn_tile && a.knn_reuse) k_map_fit_reuse<<<o == 0 ? gr : (o <= 2 ? gf2 : gf), 128, 0, st>>>(a);   // ~25 % / 8 % / < 3 % of the rows change in iterations 1 / 2 / later
+    if (a.knn_reuse) k_map_fit_reuse<<<o == 0 ? gr : (o <= 2 ? gf2 : gf), 128, 0, st>>>(a);   // ~25 % / 8 % / < 3 % of the rows change in iterations 1 / 2 / later
     else k_map_fit<<<ga, 128, 0, st>>>(a);
     if (launches) *launches += 1;
     SolveArgs sa = solve_proto;
-    sa.which = 1; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = 0; sa.lane0 = 0; sa.reset_cnt = nullptr;  // LidarEdgeFactor(..., 1.0), :610
+    sa.which = 1; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = 0; sa.reset_cnt = nullptr;  // LidarEdgeFactor(..., 1.0), :610
     LVO_MARK(tm, LVO_ST_MAP_SOLVER, st);
     lvo_launch_lm(st, sa, lanes, 16384);
     if (launches) *launches += 2;

@@ -18,13 +18,12 @@
 #include "lvo_knn.cuh"
 #include "lvo_solver.cuh"
 
-#define LVO_ODO_GRIDS 6   // search structures per lane over the previous sweep's two clouds
+#define LVO_ODO_GRIDS 6         // search structures per lane over the previous sweep's two clouds
+#define LVO_ODO_FAST_AZ_HALF 16 // widest azimuth half-window (buckets) the thread-per-feature kernel scans itself
 
 struct OdoArgs {
   LaneState* ls;
   int lanes, outer;
-  int fast_h;        // widest azimuth half-window (buckets) the thread-per-feature kernel scans itself (16; LVO_FAST_H overrides)
-  int lane0;         // first lane of an association launch (chunked outer loop, see lvo_launch_odometry)
   int distortion;    // 0 | 1 | 2, see the header comment
   const int* lane_flags;   // [lanes] LVO_LANE_* of the step: an idle lane's pose, "last" clouds, status and stats are left alone
   // current features (stride caps)
@@ -298,7 +297,7 @@ __device__ __forceinline__ void scan_range4(const float4* __restrict__ pts, unsi
 
 __global__ void __launch_bounds__(128) k_odo_assoc_fast(OdoArgs a) {
   __shared__ GridView gv[4];
-  const int lane = a.lane0 + blockIdx.y;
+  const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
   if (!s.odo_inited || s.odo_done) return;   // first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   if (threadIdx.x < 4) gv[threadIdx.x] = grid_view(a.grid, LVO_ODO_GRIDS * lane + threadIdx.x);
@@ -461,7 +460,7 @@ __global__ void __launch_bounds__(128) k_odo_assoc_fast(OdoArgs a) {
           // with LVO_OPT_ODO_REUSE the windows reach LVO_ODO_SLACK beyond the best distances: room for the next iterations' certificates
           hA = corner ? 0 : (bA.j >= 0 ? (a.reuse ? az_halfwidth_slack(bA.d, rho) : az_halfwidth(bA.d, rho)) : LVO_AZ_BUCKETS);
           hB = bB.j >= 0 ? (a.reuse ? az_halfwidth_slack(bB.d, rho) : az_halfwidth(bB.d, rho)) : LVO_AZ_BUCKETS;
-          if (hA > a.fast_h || hB > a.fast_h) {   // a target has no candidate nearby or its window is wide: leave it to the cooperative kernel
+          if (hA > LVO_ODO_FAST_AZ_HALF || hB > LVO_ODO_FAST_AZ_HALF) {   // a target has no candidate nearby or its window is wide: leave it to the cooperative kernel
             fast = false; why = ((!corner && bA.j < 0) || bB.j < 0) ? 4 : 3; break;
           }
           skipA = corner ? hA : sA; skipB = sB;
@@ -537,7 +536,7 @@ __device__ __forceinline__ float tile_min_f(float v) {
 template <int TW>
 __global__ void __launch_bounds__(256, 4) k_odo_assoc(OdoArgs a) {
   __shared__ GridView gv[LVO_ODO_GRIDS];
-  const int lane = a.lane0 + blockIdx.y;
+  const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
   if (!s.odo_inited || s.odo_done) return;   // first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   if (threadIdx.x < LVO_ODO_GRIDS) gv[threadIdx.x] = grid_view(a.grid, LVO_ODO_GRIDS * lane + threadIdx.x);
@@ -776,43 +775,27 @@ __global__ void k_odo_swap(OdoArgs a) {
   }
 }
 
-// lanes per chunk of the scan-to-scan outer loop; LVO_ODO_CHUNK overrides (tuning aid)
-static inline int lvo_odo_chunk(int lanes) {
-  static int env = -1;
-  if (env < 0) { const char* e = getenv("LVO_ODO_CHUNK"); env = e ? atoi(e) : 0; }
-  if (env > 0) return env;
-  return lanes;
-}
 static inline void lvo_launch_odometry(cudaStream_t st, OdoArgs a, const SolveArgs& solve_proto, int outer_iters, int lanes, long long* launches, LvoStageTimer* tm = nullptr) {
   LVO_MARK(tm, LVO_ST_ODO_REST, st);
   k_odo_begin<<<lvo_div_up(lanes, 64), 64, 0, st>>>(a);
   if (launches) *launches += 1;
   const int nfeat_cap = a.cap_sharp + a.cap_flat;
-  // The outer loop runs chunk by chunk of lanes: the ten association passes of a lane read the same two grids of its previous
-  // sweep (~1.4 MB per lane), so a chunk whose grids fit the 126 MB L2 pays DRAM for them once instead of ten times.
-  const int chunk = lvo_odo_chunk(lanes);
-  { static int fh = -1; if (fh < 0) { const char* e = getenv("LVO_FAST_H"); fh = e ? atoi(e) : 16; } a.fast_h = fh; }
-  for (int l0 = 0; l0 < lanes; l0 += chunk) {
-    const int nl = min(chunk, lanes - l0);
-    a.lane0 = l0;
-    dim3 ga(max(1, lvo_div_up(nfeat_cap * 8, 256)), nl);          // 8-lane tiles, every feature (outer iteration 0)
-    dim3 gs(max(1, lvo_div_up(nfeat_cap * 32 / 8, 256)), nl);     // full-warp tiles for the slow list (an eighth of the features per pass, grid-strided)
-    dim3 gf(max(1, lvo_div_up(nfeat_cap, 128)), nl);
-    for (int o = 0; o < outer_iters; ++o) {
-      a.outer = o;
-      LVO_MARK(tm, LVO_ST_ODO_ASSOC, st);
-      k_odo_assoc_fast<<<gf, 128, 0, st>>>(a);   // (slow_cnt is zero here: k_odo_begin before the loop, k_lm_solve after every iteration)
-      if (launches) *launches += 1;
-      if (o == 0) k_odo_assoc<8><<<ga, 256, 0, st>>>(a);   // first iteration: more features lack a nearby candidate
-      else k_odo_assoc<32><<<gs, 256, 0, st>>>(a);
-      SolveArgs sa = solve_proto;
-      sa.which = 0; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = a.distortion != 0; sa.lane0 = l0; sa.reset_cnt = a.slow_cnt;
-      LVO_MARK(tm, LVO_ST_ODO_SOLVER, st);
-      lvo_launch_lm(st, sa, nl, nfeat_cap);
-      if (launches) *launches += 2;
-    }
+  dim3 ga(max(1, lvo_div_up(nfeat_cap * 8, 256)), lanes);          // 8-lane tiles, every feature (outer iteration 0)
+  dim3 gs(max(1, lvo_div_up(nfeat_cap * 32 / 8, 256)), lanes);     // full-warp tiles for the slow list (an eighth of the features per pass, grid-strided)
+  dim3 gf(max(1, lvo_div_up(nfeat_cap, 128)), lanes);
+  for (int o = 0; o < outer_iters; ++o) {
+    a.outer = o;
+    LVO_MARK(tm, LVO_ST_ODO_ASSOC, st);
+    k_odo_assoc_fast<<<gf, 128, 0, st>>>(a);   // (slow_cnt is zero here: k_odo_begin before the loop, k_lm_solve after every iteration)
+    if (launches) *launches += 1;
+    if (o == 0) k_odo_assoc<8><<<ga, 256, 0, st>>>(a);   // first iteration: more features lack a nearby candidate
+    else k_odo_assoc<32><<<gs, 256, 0, st>>>(a);
+    SolveArgs sa = solve_proto;
+    sa.which = 0; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = a.distortion != 0; sa.reset_cnt = a.slow_cnt;
+    LVO_MARK(tm, LVO_ST_ODO_SOLVER, st);
+    lvo_launch_lm(st, sa, lanes, nfeat_cap);
+    if (launches) *launches += 2;
   }
-  a.lane0 = 0;
   LVO_MARK(tm, LVO_ST_ODO_REST, st);
   k_odo_integrate<<<lvo_div_up(lanes, 64), 64, 0, st>>>(a, outer_iters);
   if (a.distortion == 2) { k_odo_to_end<<<dim3(64, lanes), 256, 0, st>>>(a); if (launches) *launches += 1; }

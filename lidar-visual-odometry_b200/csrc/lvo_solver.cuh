@@ -287,7 +287,6 @@ struct SolveArgs {
   int max_iters;
   double huber;
   double* trace;              // [lanes][LVO_MAX_OUTER][LVO_MAX_LM + 1][LVO_TRACE_W] or null
-  int lane0;                  // first lane of this launch (lanes are processed in chunks, see lvo_launch_odometry)
   int distort;                // != 0: factors may carry an interpolation ratio s != 1 (scan-to-scan with DISTORTION 1)
   int n_outer;                // outer iterations of the frame (stats slots to fill when the loop is cut short)
   int fixpoint_skip;          // LVO_OPT_FIXPOINT_SKIP
@@ -415,7 +414,7 @@ __global__ void __launch_bounds__(LVO_LM_THREADS, LVO_LM_MINB) k_lm_solve(SolveA
   __shared__ LmShared sh;
   __shared__ LmCtl ctl;  // only thread 0 touches it; shared to keep it out of its registers
   const bool lead = threadIdx.x == 0;
-  const int lane = a.lane0 + blockIdx.x;
+  const int lane = blockIdx.x;
   LaneState& s = a.ls[lane];
   if (a.reset_cnt && threadIdx.x == 0) a.reset_cnt[lane] = 0;   // the association kernels of this iteration are through with it
   if (a.which == 0 ? (s.odo_inited == 0 || s.odo_done != 0) : (s.map_too_small != 0 || s.map_done != 0)) return;

@@ -77,25 +77,11 @@ def test_two_gpus_give_bitwise_identical_poses(lvo_mod, synth):
     a.close(); b.close()
 
 
-def test_tiled_knn_option_gives_identical_index_sets(lvo_mod, synth):
-    """LVO_OPT_KNN_TILE: the shared-memory tiled 5-NN (cell-sorted queries, cp.async.bulk staging) against the thread-per-query search:
-    index sets of every outer iteration, accept flags, poses and maps bit for bit."""
+def test_retired_option_value_is_rejected(lvo_mod):
+    """Option 4 selected a removed 5-NN search: it is not reused and is refused like any unknown option."""
     L = lvo_mod
-    a = L.Lvo(lanes=2, **CAPS)
-    b = L.Lvo(lanes=2, **CAPS)
-    b.set_option(L.LVO_OPT_KNN_TILE, 1)
-    for c in (a, b):
-        c.set_option(L.LVO_OPT_GRAPHS, 0)
-    for k in range(6):
-        sw = [synth.sweep(64, 0, k)[0], synth.sweep(64, 7, k)[0]]
-        sa, oa, ma = a.step_batch(sw)
-        sb, ob, mb = b.step_batch(sw)
-        assert sa == sb and np.array_equal(oa, ob) and np.array_equal(ma, mb), k
-        for lane in range(2):
-            for what in (L.P_MAP_CORNER_KNN, L.P_MAP_SURF_KNN, L.P_MAP_CORNER_VALID, L.P_MAP_SURF_VALID):
-                assert np.array_equal(a.probe(what, lane), b.probe(what, lane)), (k, lane, what)
-    for which in (0, 1):
-        pa, ca = a.map_export(1, which)
-        pb, cb = b.map_export(1, which)
-        assert np.array_equal(ca, cb) and np.array_equal(pa.view(np.uint32), pb.view(np.uint32))
-    a.close(); b.close()
+    lvo = L.Lvo(lanes=1, **CAPS)
+    assert lvo.lib.lvo_set_option(lvo.h, 4, 1) == L.LVO_E_BADARG
+    for opt in (L.LVO_OPT_GRAPHS, L.LVO_OPT_FIXPOINT_SKIP, L.LVO_OPT_STAGE_TIMING, L.LVO_OPT_KNN_REUSE, L.LVO_OPT_ODO_REUSE):
+        assert lvo.lib.lvo_set_option(lvo.h, opt, 1) == L.LVO_OK, opt
+    lvo.close()
