@@ -187,11 +187,36 @@ int lvo_set_lane_active(lvo_ctx* ctx, int lane, int active);
 /* Return `lane` to the state of a freshly created context: next active step is its first frame (LVO_W_FIRST_FRAME), empty map,
  * identity poses and map correction, cen = (10, 10, 5), zero lvo_stats, status LVO_OK, skip_frame phase 0.  Other lanes are
  * untouched, and so is the lane's activity.  Stream-ordered (returns when done); LVO_E_STATE while an *_async step is in flight,
- * LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid.  To start a sequence from a pre-built map, follow it with
- * lvo_map_import / lvo_set_odometry_state. */
+ * LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid.  To resume a saved sequence exactly, use lvo_lane_load instead; to
+ * start a new sequence from a pre-built map, follow the reset with lvo_map_import / lvo_set_odometry_state. */
 int lvo_lane_reset(lvo_ctx* ctx, int lane);
 
-/* ---- state export / import (SURVEY §5 "Checkpoint / resume"; needed to start from a pre-filled map) ------- */
+/* ---- lane snapshots: checkpoint / resume, and moving a running lane to another lane, context or GPU -------- */
+
+/* Snapshot of everything `lane` carries into its next frame: its device state (poses, map correction, cube window, lvo_stats, ...),
+ * the odometry "last" clouds, the current map with its cube offset tables, its skip_frame phase and lvo_lane_status.  Per-frame
+ * intermediates (probes, the registered cloud) are not included.  The format is versioned and documented in DESIGN.md §3; it holds
+ * no lane index, device or pointer, so two lanes that ran the same sequence give the same bytes.  `dst` may be host memory
+ * (pageable or pinned) or device memory of any device.  dst == NULL or cap too small: LVO_E_CAPACITY with *n_bytes = the size
+ * needed (n_bytes may be NULL).  Changes nothing; synchronous on return.  LVO_E_STATE while an *_async step is in flight,
+ * LVO_E_BADARG for a bad lane. */
+int lvo_lane_save(lvo_ctx* ctx, int lane, void* dst, size_t cap, size_t* n_bytes);
+/* Replace the state of `lane` with a snapshot (host or device memory, any device): its next active step continues the saved
+ * sequence exactly as the source lane would have.  The destination may be any lane of any context whose n_scans, minimum_range,
+ * line_res, plane_res, skip_frame, outer_iters, lm_max_iters, huber and distortion equal the source's (else LVO_E_BADARG, and
+ * lvo_last_error names the field); its capacities may differ as long as the saved clouds and map, and the point counts of the
+ * lane's last frame, fit (else LVO_E_CAPACITY).  The snapshot is checked in full before anything is written: a malformed one
+ * returns LVO_E_BADARG and leaves the lane as it was.
+ * lvo_get_stats, lvo_lane_status, lvo_map_export, lvo_map_cloud and lvo_get_map_correction report the snapshot at once;
+ * lvo_probe_fetch of the lane returns LVO_E_STATE for a probe until the stage that writes it has run for the lane: extraction and
+ * odometry probes until its next active frame (or lvo_extract_features / lvo_scan_to_scan), LVO_P_MAP_* and LVO_P_REGISTERED until
+ * its next mapping frame (or lvo_scan_to_map).  The
+ * lane's activity is unchanged.  The next lvo_step_batch* / lvo_scan_to_scan call first rebuilds the odometry search grids of the
+ * context once, however many lanes were loaded.  Synchronous on return; LVO_E_STATE while an *_async step is in flight, LVO_E_BADARG
+ * for a bad lane.  Captured CUDA graphs stay valid. */
+int lvo_lane_load(lvo_ctx* ctx, int lane, const void* src, size_t n_bytes);
+
+/* ---- state export / import (start from a pre-filled map; exact checkpoint / resume: lvo_lane_save / lvo_lane_load) */
 
 /* Replace the map of `lane` with the given cubes.  cube_ind[i] is the reference's array index
  * i + 21*j + 441*k (laserMapping.cpp:522) of point i; points of one cube keep their relative order. */

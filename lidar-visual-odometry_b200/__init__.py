@@ -87,7 +87,7 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_get_map_correction", "lvo_set_map_correction", "lvo_set_odometry_state", "lvo_probe_fetch", "lvo_voxel_downsample", "lvo_knn",
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
            "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
-           "lvo_lane_reset"]
+           "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load"]
 
 
 def load_library():
@@ -114,6 +114,8 @@ def load_library():
     L.lvo_wait.argtypes = [vp, C.POINTER(Pose), C.POINTER(Pose)]
     L.lvo_set_lane_active.argtypes = [vp, ip, ip]
     L.lvo_lane_reset.argtypes = [vp, ip]
+    L.lvo_lane_save.argtypes = [vp, ip, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.lvo_lane_load.argtypes = [vp, ip, vp, C.c_size_t]
     L.lvo_map_import.argtypes = [vp, ip, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
     L.lvo_map_export.argtypes = [vp, ip, ip, C.POINTER(CloudOut), vp]
     L.lvo_map_cloud.argtypes = [vp, ip, ip, C.POINTER(CloudOut)]
@@ -311,6 +313,32 @@ class Lvo:
     def lane_reset(self, lane):
         """Return `lane` to the first-frame state of a new context (empty map, identity poses, skip_frame phase 0)."""
         self._check(self.lib.lvo_lane_reset(self.h, lane))
+
+    def lane_save(self, lane):
+        """Snapshot of `lane` (lvo_lane_save) as a uint8 array: write it to disk, or lane_load it into any lane of a context with the
+        same settings."""
+        n = C.c_size_t(0)
+        r = self.lib.lvo_lane_save(self.h, lane, None, 0, C.byref(n))
+        if r != LVO_E_CAPACITY:
+            self._check(r)
+        buf = np.empty(n.value, np.uint8)
+        self._check(self.lib.lvo_lane_save(self.h, lane, buf.ctypes.data, buf.nbytes, C.byref(n)))
+        return buf
+
+    def lane_load(self, lane, data):
+        """Continue the sequence of a lane_save snapshot (bytes or a uint8 array) in `lane`."""
+        a = np.frombuffer(data, np.uint8) if isinstance(data, (bytes, bytearray)) else np.ascontiguousarray(data, np.uint8)
+        self._check(self.lib.lvo_lane_load(self.h, lane, a.ctypes.data, a.nbytes))
+
+    def lane_save_dev(self, lane, ptr, cap):
+        """lane_save into device memory (any device) at `ptr` with `cap` bytes; returns the snapshot's size."""
+        n = C.c_size_t(0)
+        self._check(self.lib.lvo_lane_save(self.h, lane, C.c_void_p(ptr), cap, C.byref(n)))
+        return n.value
+
+    def lane_load_dev(self, lane, ptr, n):
+        """lane_load from device memory (any device): the snapshot's `n` bytes at `ptr`."""
+        self._check(self.lib.lvo_lane_load(self.h, lane, C.c_void_p(ptr), n))
 
     # ---- state
     def map_import(self, lane, corner, corner_cube, surf, surf_cube):

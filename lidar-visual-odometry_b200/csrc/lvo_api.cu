@@ -13,9 +13,15 @@
 #include "lvo_depth.cuh"
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <nvtx3/nvToolsExt.h>   // header-only; ranges under the reference's stage names show up in Nsight timelines
+
+// lvo_lane_load: lvo_probe_fetch of the lane returns LVO_E_STATE for a probe until the stage that writes it has run for the lane
+#define LVO_PROBE_GATE_EXTRACT 1  // LVO_P_FULL .. LVO_P_LESS_FLAT: its next active frame, or lvo_extract_features
+#define LVO_PROBE_GATE_ODO 2      // LVO_P_ODO_*: its next active frame, or lvo_scan_to_scan
+#define LVO_PROBE_GATE_MAP 4      // LVO_P_MAP_*, LVO_P_REGISTERED: its next mapping frame, or lvo_scan_to_map
 
 struct lvo_ctx {
   lvo_config cfg;
@@ -53,6 +59,10 @@ struct lvo_ctx {
   std::vector<char> lane_active;      // lvo_set_lane_active
   std::vector<char> prefetched_active;  // the active set the prefetched sweeps were staged for
   std::vector<int> lane_status;
+  // lvo_lane_load: a loaded lane's probe arrays belong to this context's earlier frames, its counts to the snapshot; LVO_PROBE_GATE_*
+  // bits stay set until the stage that writes the probe has run for the lane
+  std::vector<char> probe_gate;
+  bool odo_grids_stale = false;     // lvo_lane_load: the odometry grids no longer match the "last" clouds (rebuilt by the next reader)
   cudaEvent_t ev[8];
   LvoStageTimer stage_tm;           // sub-stage CUDA events of plain-launch calls (reference TicToc names)
   lvo_timings tim;
@@ -248,12 +258,22 @@ int sync_state(lvo_ctx* c) {
   LVO_CUDA_OK(c, cudaGetLastError());
   return LVO_OK;
 }
+// The odometry grids of frame k + 1 are built at the end of frame k for all lanes at once (the problems share one table).  After
+// lvo_lane_load the loaded lane's grids are stale; the next call that searches them rebuilds every lane's grids once, however many
+// lanes were loaded.  The other lanes' grids come out the same: they are built from the same clouds.
+void rebuild_stale_grids(lvo_ctx* c) {
+  if (!c->odo_grids_stale) return;
+  lvo_grid_build(c->st, c->odo.grid, &c->launches);
+  c->odo_grids_stale = false;
+}
 void pose_out(lvo_pose* p, const double* q, const double* t) {
   if (!p) return;
   for (int k = 0; k < 4; ++k) p->q[k] = q[k];
   for (int k = 0; k < 3; ++k) p->t[k] = t[k];
 }
 int* lane_flags(lvo_ctx* c) { return c->h_in_n + c->lanes; }
+// the stand-alone stage calls run their stage for every lane: its probes are this context's own again
+void stage_ran_on_all_lanes(lvo_ctx* c, int gate) { for (char& g : c->probe_gate) g &= ~gate; }
 // sweep pointers, counts and lane flags of the step
 int set_inputs(lvo_ctx* c) {
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->d_in_ptr, c->h_in_ptr, sizeof(void*) * c->lanes, cudaMemcpyHostToDevice, c->st));
@@ -424,6 +444,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   c->lane_status.assign(L, 0);
   c->lane_frame.assign(L, 0);
   c->lane_active.assign(L, 1);
+  c->probe_gate.assign(L, 0);
 
   LVO_TRY(dalloc(c, &c->d_ls, (size_t)L));
   LVO_TRY(halloc(c, &c->h_ls, (size_t)L));
@@ -616,6 +637,7 @@ int lvo_extract_features(lvo_ctx* c, lvo_cloud_view sweep, lvo_cloud_out* full, 
   LVO_TRY(set_inputs(c));
   LvoStageTimer* tm = stage_timer_begin(c, true);
   enqueue_extract(c, sweep.n ? (int)sweep.stride : 16, sweep.n ? (int)sweep.off_xyz : 0, (int)sweep.n, tm);
+  stage_ran_on_all_lanes(c, LVO_PROBE_GATE_EXTRACT);
   c->stage_tm.stop(c->st);
   cudaEventRecord(c->ev[1], c->st);
   LVO_TRY(sync_state(c));
@@ -641,6 +663,7 @@ int lvo_scan_to_scan(lvo_ctx* c, lvo_cloud_view sharp, lvo_cloud_view less_sharp
   LVO_TRY(check_view(c, sharp, (size_t)c->cap_sharp)); LVO_TRY(check_view(c, less_sharp, (size_t)c->cap_lsharp));
   LVO_TRY(check_view(c, flat, (size_t)c->cap_flat)); LVO_TRY(check_view(c, less_flat, (size_t)c->P));
   c->launches = 0;
+  rebuild_stale_grids(c);
   cudaEventRecord(c->ev[2], c->st);
   LVO_TRY(upload_cloud(c, sharp, c->ex.sharp)); LVO_TRY(upload_cloud(c, less_sharp, c->ex.less_sharp));
   LVO_TRY(upload_cloud(c, flat, c->ex.flat)); LVO_TRY(upload_cloud(c, less_flat, c->ex.less_flat));
@@ -651,6 +674,7 @@ int lvo_scan_to_scan(lvo_ctx* c, lvo_cloud_view sharp, lvo_cloud_view less_sharp
   c->solve.trace = c->d_trace[0];
   LvoStageTimer* tm = stage_timer_begin(c, true);
   enqueue_odometry(c, tm);
+  stage_ran_on_all_lanes(c, LVO_PROBE_GATE_ODO);
   c->stage_tm.stop(c->st);
   cudaEventRecord(c->ev[3], c->st);
   LVO_TRY(sync_state(c));
@@ -684,6 +708,7 @@ int lvo_scan_to_map(lvo_ctx* c, lvo_cloud_view corner_last, lvo_cloud_view surf_
   c->solve.trace = c->d_trace[1];
   LvoStageTimer* tm = stage_timer_begin(c, true);
   enqueue_mapping(c, 0, want_reg, tm);
+  stage_ran_on_all_lanes(c, LVO_PROBE_GATE_MAP);
   c->stage_tm.stop(c->st);
   cudaEventRecord(c->ev[5], c->st);
   LVO_TRY(sync_state(c));
@@ -731,6 +756,8 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
   if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
   c->launches = 0;
   LVO_TRY(enqueue_prefetch(c));
+  rebuild_stale_grids(c);             // outside the graph: a step without a preceding lvo_lane_load launches nothing more
+  const long long pre_launches = c->launches;
   // a lane maps on its own frames 0, skip_frame, 2 skip_frame, ... (laserOdometry.cpp:643); the mapping stage is enqueued when any
   // lane maps, and the kernels pass the others through (LVO_LANE_MAPS)
   bool do_map = false;
@@ -762,11 +789,11 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
       e = cudaGraphInstantiate(&c->graph_exec[do_map][gen], graph, 0);
       cudaGraphDestroy(graph);
       if (e != cudaSuccess) { nvtxRangePop(); lvo_set_error(c, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e)); return LVO_E_CUDA; }
-      c->graph_launches[do_map][gen] = c->launches;
+      c->graph_launches[do_map][gen] = c->launches - pre_launches;
     }
     cudaError_t ge = cudaGraphLaunch(c->graph_exec[do_map][gen], c->st);
     if (ge != cudaSuccess) { nvtxRangePop(); lvo_set_error(c, std::string("cudaGraphLaunch: ") + cudaGetErrorString(ge)); return LVO_E_CUDA; }
-    c->launches = c->graph_launches[do_map][gen];
+    c->launches = pre_launches + c->graph_launches[do_map][gen];
     if (do_map) c->map.gen = gen ^ 1;
     cudaEventRecord(c->ev[3], c->st);
   } else {
@@ -782,7 +809,11 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
     cudaEventRecord(c->ev[3], c->st);
   }
   nvtxRangePop();
-  for (int l = 0; l < c->lanes; ++l) if (c->lane_active[l]) c->lane_frame[l]++;
+  for (int l = 0; l < c->lanes; ++l) {
+    const int f = lane_flags(c)[l];
+    if (f & LVO_LANE_ACTIVE) { c->lane_frame[l]++; c->probe_gate[l] &= ~(LVO_PROBE_GATE_EXTRACT | LVO_PROBE_GATE_ODO); }
+    if (f & LVO_LANE_MAPS) c->probe_gate[l] = 0;
+  }
   // the lane states come back on the same stream; lvo_wait only has to synchronise
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->h_ls, c->d_ls, sizeof(LaneState) * c->lanes, cudaMemcpyDeviceToHost, c->st));
   c->pending = true; c->pending_do_map = do_map; c->pending_graph = use_graph;
@@ -952,6 +983,207 @@ int lvo_lane_reset(lvo_ctx* c, int lane) {
   LVO_CUDA_OK(c, cudaGetLastError());
   c->lane_status[lane] = LVO_OK;
   c->lane_frame[lane] = 0;
+  c->probe_gate[lane] = 0;   // zero counts: every probe is empty, and in bounds
+  return LVO_OK;
+}
+
+// ---- lane snapshots (DESIGN §3 "Lane snapshot"): header | LaneState | cube_start corner | cube_start surf | corner_last | surf_last |
+// map corner | map surf.  Everything before the point sections has a fixed size, so that a load can check it on the host first.
+}  // extern "C"
+namespace {
+#define LVO_SNAP_VERSION 1u
+static const char kSnapMagic[8] = {'L', 'V', 'O', 'L', 'A', 'N', 'E', '\0'};
+struct LvoSnapHeader {
+  char magic[8];
+  uint32_t version, header_bytes, state_bytes, cube_entries;   // LVO_SNAP_VERSION, 128, sizeof(LaneState), LVO_NCUBES + 1
+  uint64_t total_bytes;
+  // every lvo_config field that changes results
+  int32_t n_scans, skip_frame, outer_iters, lm_max_iters, distortion, reserved0;
+  double minimum_range, line_res, plane_res, huber;
+  // host-side lane data
+  int64_t lane_frame;   // frames since the sequence started (its skip_frame phase)
+  int32_t lane_status;
+  uint32_t n_corner_last, n_surf_last, n_map[2];   // points in the four point sections
+  uint8_t reserved1[12];
+};
+static_assert(sizeof(LvoSnapHeader) == 128, "lane snapshot header layout");
+const size_t kSnapCubeBytes = sizeof(unsigned) * (LVO_NCUBES + 1);
+const size_t kSnapPrefix = sizeof(LvoSnapHeader) + sizeof(LaneState) + 2 * kSnapCubeBytes;   // a multiple of 16: the points stay aligned
+static_assert(kSnapPrefix % 16 == 0, "lane snapshot sections");
+// LaneState::cen: cube_coord adds it to int((v + 25) / 50), and k_map_begin walks the centre cube back into the window one step at a
+// time; a running lane keeps it near the cube of the world origin (50 m cubes: 2^20 of them span 52 000 km).  The poses bound v:
+// every translation within 1e7 m and every quaternion component within [-2, 2] keep the map position that k_map_begin composes
+// below 3e8 m, so the cube coordinate plus cen stays far from int overflow and the walk is finite.
+#define LVO_SNAP_CEN_LIMIT (1 << 20)
+#define LVO_SNAP_T_LIMIT 1.0e7
+#define LVO_SNAP_Q_LIMIT 2.0
+
+uint64_t snap_total(const LvoSnapHeader& h) {
+  return kSnapPrefix + 16ull * ((uint64_t)h.n_corner_last + h.n_surf_last + h.n_map[0] + h.n_map[1]);
+}
+int snap_bad(lvo_ctx* c, const std::string& what) { lvo_set_error(c, "lane snapshot rejected: " + what); return LVO_E_BADARG; }
+int snap_cap(lvo_ctx* c, const std::string& what) { lvo_set_error(c, "lane snapshot does not fit this context: " + what); return LVO_E_CAPACITY; }
+// a (q, t) pair of doubles in LaneState: finite and inside the limits above
+bool pose_ok(const double* q, const double* t) {
+  for (int k = 0; k < 4; ++k) if (!std::isfinite(q[k]) || std::fabs(q[k]) > LVO_SNAP_Q_LIMIT) return false;
+  for (int k = 0; k < 3; ++k) if (!std::isfinite(t[k]) || std::fabs(t[k]) > LVO_SNAP_T_LIMIT) return false;
+  return true;
+}
+bool monotone(const int* v, int n, int lo, int hi) {   // lo <= v[0] <= ... <= v[n - 1] <= hi
+  int prev = lo;
+  for (int i = 0; i < n; ++i) { if (v[i] < prev || v[i] > hi) return false; prev = v[i]; }
+  return true;
+}
+void snap_fingerprint(const lvo_config& cfg, LvoSnapHeader& h) {
+  h.n_scans = cfg.n_scans; h.skip_frame = cfg.skip_frame; h.outer_iters = cfg.outer_iters; h.lm_max_iters = cfg.lm_max_iters;
+  h.distortion = cfg.distortion; h.minimum_range = cfg.minimum_range; h.line_res = cfg.line_res; h.plane_res = cfg.plane_res; h.huber = cfg.huber;
+}
+// Every field of the fixed part that a kernel or an entry point later uses as an index, a loop bound or a size, checked against this
+// context before anything is written.  `cs` = the two cube_start tables.
+int snap_check(lvo_ctx* c, const LvoSnapHeader& h, const LaneState& s, const unsigned* const cs[2], size_t n_bytes) {
+  if (memcmp(h.magic, kSnapMagic, sizeof(kSnapMagic)) != 0) return snap_bad(c, "not a lane snapshot (magic)");
+  if (h.version != LVO_SNAP_VERSION) return snap_bad(c, "format version " + std::to_string(h.version) + ", this library reads " + std::to_string(LVO_SNAP_VERSION));
+  if (h.header_bytes != sizeof(LvoSnapHeader) || h.state_bytes != sizeof(LaneState) || h.cube_entries != LVO_NCUBES + 1)
+    return snap_bad(c, "header / LaneState / cube table size differs from this library's");
+  if (h.total_bytes != snap_total(h) || n_bytes != h.total_bytes)
+    return snap_bad(c, "byte length " + std::to_string(n_bytes) + ", the header describes " + std::to_string(snap_total(h)));
+  LvoSnapHeader mine; memset(&mine, 0, sizeof(mine));
+  snap_fingerprint(c->cfg, mine);
+#define LVO_SNAP_FIELD(f) if (!(h.f == mine.f)) return snap_bad(c, "lvo_config::" #f " differs from this context's");
+  LVO_SNAP_FIELD(n_scans) LVO_SNAP_FIELD(minimum_range) LVO_SNAP_FIELD(line_res) LVO_SNAP_FIELD(plane_res) LVO_SNAP_FIELD(skip_frame)
+  LVO_SNAP_FIELD(outer_iters) LVO_SNAP_FIELD(lm_max_iters) LVO_SNAP_FIELD(huber) LVO_SNAP_FIELD(distortion)
+#undef LVO_SNAP_FIELD
+  if (h.lane_frame < 0) return snap_bad(c, "lane_frame < 0");
+  // odometry: the "last" clouds and their ring-offset tables
+  if ((int64_t)s.n_corner_last != h.n_corner_last || (int64_t)s.n_surf_last != h.n_surf_last) return snap_bad(c, "n_corner_last / n_surf_last disagree with the header");
+  if (s.n_corner_last > c->cap_lsharp) return snap_bad(c, "n_corner_last exceeds the less-sharp capacity of n_scans");
+  if (!monotone(s.corner_ring_first, LVO_MAX_RINGS + 2, 0, s.n_corner_last)) return snap_bad(c, "corner_ring_first");
+  if (!monotone(s.surf_ring_first, LVO_MAX_RINGS + 2, 0, s.n_surf_last)) return snap_bad(c, "surf_ring_first");
+  // poses: the odometry pose and its increment, the mapping pose, the map correction, the odometry pose the mapping stage last read
+  if (!pose_ok(s.para_q, s.para_t) || !pose_ok(s.q_w, s.t_w) || !pose_ok(s.map_x, s.map_x + 4) || !pose_ok(s.q_wmap_wodom, s.t_wmap_wodom) ||
+      !pose_ok(s.q_wodom, s.t_wodom))
+    return snap_bad(c, "a pose is not finite or out of range (|t| <= 1e7 m, |q_i| <= 2)");
+  // the counts of the source lane's last frame.  A batched step rewrites them before reading them, but lvo_scan_to_scan /
+  // lvo_scan_to_map run their stage for every lane of the context from its stored counts: n_sharp, n_flat, n_less_sharp, n_less_flat
+  // and n_kept bound the odometry kernels (association, k_odo_to_end, the swap into the "last" clouds), n_less_* and n_kept the stack
+  // gather and the registered cloud of the mapping stage, n_stack the mapping association and solve.  Bounds that depend on n_scans
+  // alone cannot be exceeded by a snapshot of a matching context (LVO_E_BADARG); those set by max_points can (LVO_E_CAPACITY).
+  const struct { int n; int cap; bool cap_is_P; const char* name; } counts[] = {
+      {s.n_sharp, c->cap_sharp, false, "n_sharp"}, {s.n_less_sharp, c->cap_lsharp, false, "n_less_sharp"}, {s.n_flat, c->cap_flat, false, "n_flat"},
+      {s.n_stack[0], c->map.in_cap[0], false, "n_stack[0]"}, {s.n_kept, c->P, true, "n_kept"}, {s.n_less_flat, c->P, true, "n_less_flat"},
+      {s.n_stack[1], c->map.in_cap[1], true, "n_stack[1]"}};
+  for (const auto& k : counts) {
+    if (k.n < 0) return snap_bad(c, std::string(k.name) + " < 0");
+    if (k.n > k.cap && !k.cap_is_P) return snap_bad(c, std::string(k.name) + " exceeds its capacity for n_scans");
+  }
+  // mapping: cube window, valid list, FromMap offsets
+  const int dims[3] = {LVO_CUBE_W, LVO_CUBE_H, LVO_CUBE_D};
+  for (int k = 0; k < 3; ++k) {
+    if (s.cen[k] < -LVO_SNAP_CEN_LIMIT || s.cen[k] > LVO_SNAP_CEN_LIMIT) return snap_bad(c, "cen out of range");
+    if (s.center[k] < 0 || s.center[k] >= dims[k]) return snap_bad(c, "center out of range");
+    if (s.shift[k] != 0) return snap_bad(c, "shift != 0 (k_map_end clears it after every mapping stage)");
+  }
+  if (s.n_valid < 0 || s.n_valid > LVO_MAX_VALID) return snap_bad(c, "n_valid out of range");
+  for (int v = 0; v < s.n_valid; ++v) if (s.valid_cube[v] < 0 || s.valid_cube[v] >= LVO_NCUBES) return snap_bad(c, "valid_cube out of range");
+  for (int t = 0; t < 2; ++t) {
+    if (s.from_off[t][0] != 0 || !monotone(s.from_off[t], LVO_MAX_VALID + 1, 0, INT_MAX)) return snap_bad(c, "from_off");
+    if (cs[t][0] != 0) return snap_bad(c, "cube_start does not start at 0");
+    for (int k = 0; k < LVO_NCUBES; ++k) if (cs[t][k + 1] < cs[t][k]) return snap_bad(c, "cube_start decreases");
+    if (cs[t][LVO_NCUBES] != h.n_map[t]) return snap_bad(c, "cube_start ends at a count other than the header's");
+  }
+  // capacities: may differ from the source context's as long as the saved counts fit
+  if (s.n_surf_last > c->P) return snap_cap(c, "n_surf_last " + std::to_string(s.n_surf_last) + " > max_points " + std::to_string(c->P));
+  for (const auto& k : counts)
+    if (k.n > k.cap) return snap_cap(c, std::string(k.name) + " " + std::to_string(k.n) + " > max_points " + std::to_string(c->P));
+  for (int t = 0; t < 2; ++t) {
+    const char* nm = t ? "max_map_surf" : "max_map_corner";
+    if (h.n_map[t] > (uint32_t)c->map.map_cap[t]) return snap_cap(c, std::to_string(h.n_map[t]) + " map points > " + nm + " " + std::to_string(c->map.map_cap[t]));
+    // the mapping grid build of a step in which the lane does not map still reads FromMap up to from_off[t][LVO_MAX_VALID]
+    if (s.from_off[t][LVO_MAX_VALID] > c->map.map_cap[t]) return snap_cap(c, std::string("FromMap count > ") + nm);
+  }
+  return LVO_OK;
+}
+}  // namespace
+extern "C" {
+
+int lvo_lane_save(lvo_ctx* c, int lane, void* dst, size_t cap, size_t* n_bytes) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (lane < 0 || lane >= c->lanes) { lvo_set_error(c, "lane out of range"); return LVO_E_BADARG; }
+  // the fixed part is assembled on the host (the device holds no header); the points go straight from the arenas to dst
+  std::vector<unsigned char> pre(kSnapPrefix, 0);
+  LvoSnapHeader& h = *reinterpret_cast<LvoSnapHeader*>(pre.data());
+  LaneState& s = *reinterpret_cast<LaneState*>(pre.data() + sizeof(LvoSnapHeader));
+  unsigned* cs[2] = {reinterpret_cast<unsigned*>(pre.data() + sizeof(LvoSnapHeader) + sizeof(LaneState)), nullptr};
+  cs[1] = cs[0] + (LVO_NCUBES + 1);
+  const int gen = c->map.gen;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(&s, c->d_ls + lane, sizeof(LaneState), cudaMemcpyDeviceToHost, c->st));
+  for (int t = 0; t < 2; ++t)
+    LVO_CUDA_OK(c, cudaMemcpyAsync(cs[t], c->map.cube_start[gen][t] + (size_t)lane * (LVO_NCUBES + 1), kSnapCubeBytes, cudaMemcpyDeviceToHost, c->st));
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  memcpy(h.magic, kSnapMagic, sizeof(kSnapMagic));
+  h.version = LVO_SNAP_VERSION; h.header_bytes = sizeof(LvoSnapHeader); h.state_bytes = sizeof(LaneState); h.cube_entries = LVO_NCUBES + 1;
+  snap_fingerprint(c->cfg, h);
+  h.lane_frame = c->lane_frame[lane]; h.lane_status = c->lane_status[lane];
+  h.n_corner_last = (uint32_t)s.n_corner_last; h.n_surf_last = (uint32_t)s.n_surf_last;
+  h.n_map[0] = cs[0][LVO_NCUBES]; h.n_map[1] = cs[1][LVO_NCUBES];
+  h.total_bytes = snap_total(h);
+  if (n_bytes) *n_bytes = (size_t)h.total_bytes;
+  if (!dst || cap < h.total_bytes) { lvo_set_error(c, "snapshot buffer too small"); return LVO_E_CAPACITY; }
+  // host or device memory of any device: UVA resolves the direction
+  unsigned char* out = (unsigned char*)dst;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(out, pre.data(), kSnapPrefix, cudaMemcpyDefault, c->st));
+  size_t off = kSnapPrefix;
+  const float4* src[4] = {c->odo.corner_last + (size_t)lane * c->cap_lsharp, c->odo.surf_last + (size_t)lane * c->P,
+                          c->map.map_pts[gen][0] + (size_t)lane * c->map.map_cap[0], c->map.map_pts[gen][1] + (size_t)lane * c->map.map_cap[1]};
+  const size_t cnt[4] = {h.n_corner_last, h.n_surf_last, h.n_map[0], h.n_map[1]};
+  for (int k = 0; k < 4; ++k) {
+    if (cnt[k]) LVO_CUDA_OK(c, cudaMemcpyAsync(out + off, src[k], cnt[k] * sizeof(float4), cudaMemcpyDefault, c->st));
+    off += cnt[k] * sizeof(float4);
+  }
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));   // `pre` dies on return
+  LVO_CUDA_OK(c, cudaGetLastError());
+  return LVO_OK;
+}
+
+int lvo_lane_load(lvo_ctx* c, int lane, const void* src, size_t n_bytes) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (lane < 0 || lane >= c->lanes) { lvo_set_error(c, "lane out of range"); return LVO_E_BADARG; }
+  if (!src) return snap_bad(c, "null buffer");
+  if (n_bytes < kSnapPrefix) return snap_bad(c, "truncated: " + std::to_string(n_bytes) + " bytes");
+  // the fixed part comes to the host to be checked (from device memory too); nothing is written before every check has passed
+  std::vector<unsigned char> pre(kSnapPrefix);
+  LVO_CUDA_OK(c, cudaMemcpyAsync(pre.data(), src, kSnapPrefix, cudaMemcpyDefault, c->st));
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LvoSnapHeader h; LaneState s;
+  memcpy(&h, pre.data(), sizeof(h));
+  memcpy(&s, pre.data() + sizeof(h), sizeof(s));
+  const unsigned* cs[2] = {reinterpret_cast<const unsigned*>(pre.data() + sizeof(h) + sizeof(s)), nullptr};
+  cs[1] = cs[0] + (LVO_NCUBES + 1);
+  LVO_TRY(snap_check(c, h, s, cs, n_bytes));
+  // into the current map generation; the other one is rewritten by the next mapping stage before anything reads it
+  const int gen = c->map.gen;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(c->d_ls + lane, &s, sizeof(LaneState), cudaMemcpyHostToDevice, c->st));
+  for (int t = 0; t < 2; ++t)
+    LVO_CUDA_OK(c, cudaMemcpyAsync(c->map.cube_start[gen][t] + (size_t)lane * (LVO_NCUBES + 1), cs[t], kSnapCubeBytes, cudaMemcpyHostToDevice, c->st));
+  float4* dst[4] = {c->odo.corner_last + (size_t)lane * c->cap_lsharp, c->odo.surf_last + (size_t)lane * c->P,
+                    c->map.map_pts[gen][0] + (size_t)lane * c->map.map_cap[0], c->map.map_pts[gen][1] + (size_t)lane * c->map.map_cap[1]};
+  const size_t cnt[4] = {h.n_corner_last, h.n_surf_last, h.n_map[0], h.n_map[1]};
+  size_t off = kSnapPrefix;
+  for (int k = 0; k < 4; ++k) {
+    if (cnt[k]) LVO_CUDA_OK(c, cudaMemcpyAsync(dst[k], (const unsigned char*)src + off, cnt[k] * sizeof(float4), cudaMemcpyDefault, c->st));
+    off += cnt[k] * sizeof(float4);
+  }
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LVO_CUDA_OK(c, cudaGetLastError());
+  c->h_ls[lane] = s;   // lvo_get_stats / lvo_get_map_correction / lvo_map_* see the snapshot at once
+  c->lane_frame[lane] = h.lane_frame;
+  c->lane_status[lane] = h.lane_status;
+  c->probe_gate[lane] = LVO_PROBE_GATE_EXTRACT | LVO_PROBE_GATE_ODO | LVO_PROBE_GATE_MAP;
+  c->odo_grids_stale = true;
   return LVO_OK;
 }
 
@@ -1111,6 +1343,11 @@ int lvo_probe_fetch(lvo_ctx* c, int lane, int what, void* out, size_t cap_bytes,
     default: return LVO_E_BADARG;
   }
   if (per_outer && !c->cfg.debug_probes) { lvo_set_error(c, "per-outer-iteration probes need lvo_config::debug_probes = 1"); return LVO_E_STATE; }
+  const int gate = what <= LVO_P_LESS_FLAT ? LVO_PROBE_GATE_EXTRACT : (what <= LVO_P_ODO_LM_TRACE ? LVO_PROBE_GATE_ODO : LVO_PROBE_GATE_MAP);
+  if (c->probe_gate[lane] & gate) {
+    lvo_set_error(c, "the lane was loaded from a snapshot and the stage that writes this probe has not run for it since");
+    return LVO_E_STATE;
+  }
   if (rows > 1 || row_bytes) bytes = row_bytes * rows;
   if (n_bytes) *n_bytes = bytes;
   if (!out) return LVO_OK;  // size query
