@@ -284,6 +284,28 @@ typedef struct lvo_camera { float fx, fy, cx, cy; int width, height; float extri
 int lvo_depth_associate(lvo_ctx* ctx, lvo_cloud_view sweep, const lvo_camera* cam, const float* keypoints_uv, size_t n_kp, float* depth_out,
                         int* valid_out, int* nn_out, lvo_cloud_out* depth_cloud_or_null);
 
+/* Depth association for every active lane of the context in one call (a fleet of lidar-visual front ends).  Lane l gets, bit for
+ * bit, what lvo_depth_associate(sweeps[l], &cams[l], keypoints_uv[l], n_kp[l], ...) returns: depth_out[l] / valid_out[l] are
+ * [n_kp[l]], nn_out_or_null[l] is [n_kp[l]][3] indices into that lane's depth cloud.  Only cams[l].extrinsic is read, and no
+ * lane's result depends on another lane's inputs.  Idle lanes (lvo_set_lane_active) are skipped: none of their entries is read or
+ * written, and they may be NULL / 0.
+ *   - Sweep views follow lvo_step_batch: one layout for all active lanes, stride <= 32, packed 12-byte x, y, z records allowed.
+ *   - Limits of the single call: n <= max_points and 2 n_kp <= max_points (LVO_E_CAPACITY).  NULL arrays, or a NULL keypoint /
+ *     output pointer of an active lane with n_kp > 0: LVO_E_BADARG.  nn_out_or_null may be NULL as a whole.  LVO_E_STATE while an
+ *     *_async step is in flight.  All of this is checked before anything is enqueued; on an error no output is written.
+ *   - Synchronous on return, on the context's stream (lvo_set_stream).  One launch sequence for all lanes; its length does not
+ *     depend on the number of lanes or keypoints.
+ *   - The calls use their own device arena, allocated on the first call and grown when a call brings more points, keypoints or
+ *     lanes (freed by lvo_destroy).  They read and write no state of the step: lane states, maps, probes, staging buffers, the
+ *     prefetch of lvo_step_batch_pipelined and captured CUDA graphs are left as they were.
+ * No depth cloud is returned; lvo_depth_associate remains the way to get one. */
+int lvo_depth_associate_batch(lvo_ctx* ctx, const lvo_camera* cams, const lvo_cloud_view* sweeps, const float* const* keypoints_uv,
+                              const size_t* n_kp, float* const* depth_out, int* const* valid_out, int* const* nn_out_or_null);
+/* Same, with sweeps (packed lvo_point, n[l] points), keypoints and outputs in device memory of the context's device. */
+int lvo_depth_associate_batch_dev(lvo_ctx* ctx, const lvo_camera* cams, const lvo_point* const* d_sweeps, const size_t* n,
+                                  const float* const* d_keypoints_uv, const size_t* n_kp, float* const* d_depth_out, int* const* d_valid_out,
+                                  int* const* d_nn_out_or_null);
+
 /* Throughput-mode 5-NN benchmark entry (SURVEY §8d): S independent (map, query) problems in ONE launch.
  * d_maps / d_queries are device pointers to packed points, problems laid out back to back with the given
  * per-problem counts.  Builds the cell grids (untimed part) on first call with build != 0, then runs the search

@@ -87,7 +87,7 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_get_map_correction", "lvo_set_map_correction", "lvo_set_odometry_state", "lvo_probe_fetch", "lvo_voxel_downsample", "lvo_knn",
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
            "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
-           "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load"]
+           "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load", "lvo_depth_associate_batch", "lvo_depth_associate_batch_dev"]
 
 
 def load_library():
@@ -133,6 +133,10 @@ def load_library():
     L.lvo_set_option.argtypes = [vp, ip, ip]
     L.lvo_state_bytes.restype = C.c_size_t
     L.lvo_depth_associate.argtypes = [vp, CloudView, C.POINTER(Camera), vp, C.c_size_t, vp, vp, vp, C.POINTER(CloudOut)]
+    L.lvo_depth_associate_batch.argtypes = [vp, C.POINTER(Camera), C.POINTER(CloudView), C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(vp),
+                                            C.POINTER(vp), C.POINTER(vp)]
+    L.lvo_depth_associate_batch_dev.argtypes = [vp, C.POINTER(Camera), C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(vp), C.POINTER(C.c_size_t),
+                                                C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
     return L
 
 
@@ -158,6 +162,16 @@ def to_pcl_layout(a):
     o[:, 3] = 1.0
     o[:, 4] = a[:, 3]
     return o
+
+
+def camera_of(d=None):
+    """lvo_camera from a dict like KITTI00_CAMERA (None: KITTI00_CAMERA)."""
+    cd = dict(KITTI00_CAMERA if d is None else d)
+    cam = Camera()
+    cam.fx, cam.fy, cam.cx, cam.cy, cam.width, cam.height = cd["fx"], cd["fy"], cd["cx"], cd["cy"], cd["width"], cd["height"]
+    for k in range(12):
+        cam.extrinsic[k] = cd["extrinsic"][k]
+    return cam
 
 
 def pose_to_np(p):
@@ -202,6 +216,7 @@ class Lvo:
             raise LvoError(f"lvo_create failed ({r}): {msg}")
         self.P = max_points or 262144
         self.lanes = lanes
+        self._active = [True] * lanes
 
     def close(self):
         if getattr(self, "h", None):
@@ -309,6 +324,7 @@ class Lvo:
     def set_lane_active(self, lane, active):
         """An idle lane is skipped by every step (its sweep may be None) and resumes its sequence bit for bit."""
         self._check(self.lib.lvo_set_lane_active(self.h, lane, int(bool(active))))
+        self._active[lane] = bool(active)
 
     def lane_reset(self, lane):
         """Return `lane` to the first-frame state of a new context (empty map, identity poses, skip_frame phase 0)."""
@@ -456,6 +472,39 @@ class Lvo:
         out, buf = self._out(max(v.n, 1))
         self._check(self.lib.lvo_depth_associate(self.h, v, C.byref(cam), uv.ctypes.data, n, depth.ctypes.data, valid.ctypes.data, nn.ctypes.data, C.byref(out)))
         return buf[:out.n].copy(), depth[:n], valid[:n], nn[:n]
+
+    def _cameras(self, cameras):
+        """cameras: None (KITTI00_CAMERA for every lane), one dict for every lane, or a per-lane list of dicts / None."""
+        if cameras is None or isinstance(cameras, dict):
+            cameras = [cameras] * self.lanes
+        return (Camera * self.lanes)(*[camera_of(c) for c in cameras])
+
+    def depth_associate_batch(self, sweeps, keypoints, cameras=None):
+        """Depth association for every active lane in one call (lvo_depth_associate_batch).  sweeps[l]: (n,3), (n,4) or (n,8) float32, one
+        layout for all active lanes; keypoints[l]: (k,2) normalised coordinates.  Returns a per-lane list of (depth[k], valid[k], nn[k,3]),
+        None for idle lanes (whose entries may be None)."""
+        views = [view_of(s if a else None) for s, a in zip(sweeps, self._active)]
+        uvs = [np.ascontiguousarray(k, np.float32).reshape(-1, 2) if (a and k is not None) else np.zeros((0, 2), np.float32)
+               for k, a in zip(keypoints, self._active)]
+        outs = [(np.zeros(len(u), np.float32), np.zeros(len(u), np.int32), np.full((len(u), 3), -1, np.int32)) if a else None
+                for u, a in zip(uvs, self._active)]
+        ptr = lambda i, o: o[i].ctypes.data if (o is not None and len(o[i])) else None
+        VP = C.c_void_p * self.lanes
+        r = self.lib.lvo_depth_associate_batch(self.h, self._cameras(cameras), (CloudView * self.lanes)(*[v[0] for v in views]),
+                                               VP(*[u.ctypes.data if len(u) else None for u in uvs]), (C.c_size_t * self.lanes)(*[len(u) for u in uvs]),
+                                               VP(*[ptr(0, o) for o in outs]), VP(*[ptr(1, o) for o in outs]), VP(*[ptr(2, o) for o in outs]))
+        self._check(r)
+        return outs
+
+    def depth_associate_batch_dev(self, d_sweeps, counts, d_keypoints, kp_counts, d_depth, d_valid, d_nn=None, cameras=None):
+        """Device form (lvo_depth_associate_batch_dev): per-lane device pointers (packed lvo_point sweeps, float2 keypoints, float /
+        int / int[3] outputs) and counts, None for idle lanes; d_nn may be None as a whole."""
+        VP = C.c_void_p * self.lanes
+        NS = C.c_size_t * self.lanes
+        p = lambda xs: VP(*[int(x or 0) for x in xs])
+        self._check(self.lib.lvo_depth_associate_batch_dev(self.h, self._cameras(cameras), p(d_sweeps), NS(*[int(n or 0) for n in counts]), p(d_keypoints),
+                                                           NS(*[int(n or 0) for n in kp_counts]), p(d_depth), p(d_valid),
+                                                           p(d_nn) if d_nn is not None else None))
 
     # ---- stand-alone operators
     def voxel_downsample(self, pts, leaf):

@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <nvtx3/nvToolsExt.h>   // header-only; ranges under the reference's stage names show up in Nsight timelines
 
 // lvo_lane_load: lvo_probe_fetch of the lane returns LVO_E_STATE for a probe until the stage that writes it has run for the lane
@@ -77,6 +78,22 @@ struct lvo_ctx {
   long long graph_launches[2][2] = {{0, 0}, {0, 0}};
   int graph_stride = -1, graph_off = -1;
   int opt_graphs = -1;
+  // lvo_depth_associate_batch*: the calls' own arena (DESIGN §3), allocated on the first call and grown, never shrunk, when a call
+  // brings more points, keypoints or lanes; the step's buffers are not touched
+  struct DepthArena {
+    size_t cap_pts = 0, cap_raw = 0, cap_kp = 0; int cap_slots = 0;
+    std::vector<void*> dev, pin;
+    unsigned char* raw = nullptr;      // [cap_raw] host-form sweep records, back to back in slot order
+    unsigned* flag = nullptr;          // [cap_pts]
+    float4* dc = nullptr;              // [cap_pts] depth clouds
+    unsigned char* d_in = nullptr;     // slots, then the host form's keypoints (one upload)
+    unsigned char* h_in = nullptr;     // its pinned staging
+    unsigned* d_res = nullptr;         // host form: depth [K], valid [K], nn [3 K] (one download)
+    unsigned* h_res = nullptr;
+    unsigned* dc_off = nullptr; int* ndc = nullptr;   // [cap_slots]
+    int* cnt = nullptr;                // scan length, depth-cloud total
+    GridSet grid;                      // one problem per slot, LVO_DEPTH_CELLS cells each
+  } depth;
 };
 
 void lvo_set_error(lvo_ctx* ctx, const std::string& msg) { if (ctx) ctx->err = msg; }
@@ -175,8 +192,8 @@ __global__ void k_setup_grid_problems(GridProblem* prob, int nprob, const float4
   prob[p].clamp_xy = 0.f;
   prob[p].bbox_from = (which == 0 && k >= 4) ? p - k + (k & 1) : -1;   // middle / coarse grids reuse the fine grid's box
 }
-__global__ void k_setup_one_problem(GridProblem* prob, const float4* pts, const int* d_n, float cell, float clamp = 0.f) {
-  prob[0].pts = pts; prob[0].d_n = d_n; prob[0].want_cell = cell; prob[0].want_cell_z = 0.f; prob[0].mode = 0; prob[0].cells_cap = 0; prob[0].clamp_xy = clamp; prob[0].bbox_from = -1;
+__global__ void k_setup_one_problem(GridProblem* prob, const float4* pts, const int* d_n, float cell) {
+  prob[0].pts = pts; prob[0].d_n = d_n; prob[0].want_cell = cell; prob[0].want_cell_z = 0.f; prob[0].mode = 0; prob[0].cells_cap = 0; prob[0].clamp_xy = 0.f; prob[0].bbox_from = -1;
 }
 __global__ void k_vx_single_setup(VoxelEngine e, int n, float leaf) {
   if (blockIdx.x == 0 && threadIdx.x == 0) { *e.d_n = n; *e.d_nsegs = 1; e.seg_leaf[0] = leaf; }
@@ -571,6 +588,8 @@ int lvo_destroy(lvo_ctx* c) {
   if (c->st) cudaStreamSynchronize(c->st);
   for (void* p : c->allocs) cudaFree(p);
   for (void* p : c->pinned) cudaFreeHost(p);
+  for (void* p : c->depth.dev) cudaFree(p);
+  for (void* p : c->depth.pin) cudaFreeHost(p);
   destroy_graphs(c);
   if (c->copy_st) { cudaStreamSynchronize(c->copy_st); cudaStreamDestroy(c->copy_st); cudaEventDestroy(c->copy_ev); cudaEventDestroy(c->compute_ev); }
   if (c->own_st) { for (int i = 0; i < 8; ++i) cudaEventDestroy(c->ev[i]); c->stage_tm.destroy(); cudaStreamDestroy(c->own_st); }
@@ -1462,32 +1481,31 @@ int lvo_depth_associate(lvo_ctx* c, lvo_cloud_view sweep, const lvo_camera* cam,
   unsigned* d_flag = (unsigned*)c->ex.sort_ind;    // [P]
   float* d_uv = (float*)c->ex.curv;                // [P] floats >= 2 * n_kp?  (checked below)
   if (2 * n_kp > (size_t)c->P) { lvo_set_error(c, "too many keypoints"); return LVO_E_CAPACITY; }
+  // the one slot descriptor goes to the strided-upload scratch once k_unpack has consumed it (stream order); that scratch holds
+  // 64 * max(max_points, max_map_corner, max_map_surf) bytes
+  if ((size_t)std::max(c->P, std::max(c->map.map_cap[0], c->map.map_cap[1])) * 64 < sizeof(DepthSlot)) { lvo_set_error(c, "context too small for lvo_depth_associate"); return LVO_E_CAPACITY; }
   LVO_TRY(upload_cloud(c, sweep, d_sweep));
   if (n_kp) LVO_CUDA_OK(c, cudaMemcpyAsync(d_uv, keypoints_uv, 2 * n_kp * sizeof(float), cudaMemcpyHostToDevice, c->st));
+  DepthSlot slot;
+  memset(&slot, 0, sizeof(slot));
+  slot.pts = (const unsigned char*)d_sweep; slot.n = (int)sweep.n;
+  slot.uv = d_uv; slot.nkp = (int)n_kp;
+  slot.depth = c->d_knn_sq; slot.valid = c->d_knn_ind; slot.nn = c->d_knn_ind + c->P;
+  for (int k = 0; k < 12; ++k) slot.extr[k] = cam->extrinsic[k];
+  DepthSlot* d_slot = (DepthSlot*)c->d_upload;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(d_slot, &slot, sizeof(slot), cudaMemcpyHostToDevice, c->st));
   DepthArgs a;
   memset(&a, 0, sizeof(a));
-  a.sweep = d_sweep; a.n = (int)sweep.n;
-  for (int k = 0; k < 12; ++k) a.extr[k] = cam->extrinsic[k];
-  a.flag = d_flag; a.d_n = c->d_knn_n; a.d_ndc = c->d_knn_n + 1; a.dc = d_dc;
-  a.uv = d_uv; a.nkp = (int)n_kp;
-  a.depth = c->d_knn_sq; a.valid = c->d_knn_ind; a.nn = c->d_knn_ind + c->P;
+  a.slot = d_slot; a.nslot = 1; a.stride = 16; a.off_xyz = 0; a.n_total = (int)sweep.n; a.kp_total = (int)n_kp;
+  a.flag = d_flag; a.d_n = c->d_knn_n; a.d_total = c->map.vx.d_n_out; a.dc_off = (unsigned*)(c->d_knn_n + 2); a.ndc = c->d_knn_n + 1; a.dc = d_dc;
   a.grid = c->gknn;
-  const int gb = std::max(1, std::min(lvo_div_up((long long)sweep.n, 256), 592));
-  unsigned* d_total = c->map.vx.d_n_out;
-  k_depth_flag<<<gb, 256, 0, c->st>>>(a);
-  lvo_scan_exclusive(c->st, d_flag, a.d_n, (int)std::max<size_t>(sweep.n, 1), d_total, c->map.vx.scan, &c->launches);
-  k_depth_write<<<gb, 256, 0, c->st>>>(a, d_total);
-  // 2-D grid over the image plane: 0.125-unit cells (the cloud is in 10 x normalised coordinates), clamped to +-16
-  k_setup_one_problem<<<1, 1, 0, c->st>>>(c->d_knn_prob, d_dc, a.d_ndc, 0.125f, 16.0f);
-  lvo_grid_build(c->st, c->gknn, &c->launches);
-  if (n_kp) k_depth_assoc<<<std::max(1, std::min(lvo_div_up((long long)n_kp, 8), 592)), 256, 0, c->st>>>(a);
-  c->launches += 4;
+  lvo_launch_depth(c->st, a, (int)sweep.n, c->map.vx.scan, &c->launches);
   int ndc = 0;
-  LVO_CUDA_OK(c, cudaMemcpyAsync(&ndc, a.d_ndc, 4, cudaMemcpyDeviceToHost, c->st));
+  LVO_CUDA_OK(c, cudaMemcpyAsync(&ndc, a.ndc, 4, cudaMemcpyDeviceToHost, c->st));
   if (n_kp) {
-    LVO_CUDA_OK(c, cudaMemcpyAsync(depth_out, a.depth, n_kp * 4, cudaMemcpyDeviceToHost, c->st));
-    LVO_CUDA_OK(c, cudaMemcpyAsync(valid_out, a.valid, n_kp * 4, cudaMemcpyDeviceToHost, c->st));
-    if (nn_out) LVO_CUDA_OK(c, cudaMemcpyAsync(nn_out, a.nn, n_kp * 12, cudaMemcpyDeviceToHost, c->st));
+    LVO_CUDA_OK(c, cudaMemcpyAsync(depth_out, slot.depth, n_kp * 4, cudaMemcpyDeviceToHost, c->st));
+    LVO_CUDA_OK(c, cudaMemcpyAsync(valid_out, slot.valid, n_kp * 4, cudaMemcpyDeviceToHost, c->st));
+    if (nn_out) LVO_CUDA_OK(c, cudaMemcpyAsync(nn_out, slot.nn, n_kp * 12, cudaMemcpyDeviceToHost, c->st));
   }
   LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
   LVO_CUDA_OK(c, cudaGetLastError());
@@ -1495,6 +1513,183 @@ int lvo_depth_associate(lvo_ctx* c, lvo_cloud_view sweep, const lvo_camera* cam,
   int r = download_cloud(c, d_dc, (size_t)ndc, depth_cloud_or_null);
   LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
   return r;
+}
+
+// ---- batched depth association: one problem per active lane, one launch sequence (lvo_launch_depth)
+static size_t depth_slot_bytes(int slots) { return ((size_t)slots * sizeof(DepthSlot) + 15) & ~(size_t)15; }
+
+// Grows the depth arena to hold `pts` points (`raw` bytes of host-form records), `kp` host-form keypoints and `slots` lanes.  The
+// stream is idle here (every call ends synchronised), so the old buffers can be freed at once.
+static int depth_reserve(lvo_ctx* c, size_t pts, size_t raw, size_t kp, int slots) {
+  lvo_ctx::DepthArena& d = c->depth;
+  if (d.cnt && pts <= d.cap_pts && raw <= d.cap_raw && kp <= d.cap_kp && slots <= d.cap_slots) return LVO_OK;
+  pts = std::max(pts, d.cap_pts); raw = std::max(raw, d.cap_raw); kp = std::max(kp, d.cap_kp); slots = std::max(slots, d.cap_slots);
+  for (void* p : d.dev) cudaFree(p);
+  for (void* p : d.pin) cudaFreeHost(p);
+  d.dev.clear(); d.pin.clear(); d.cnt = nullptr;
+  d.cap_pts = d.cap_raw = d.cap_kp = 0; d.cap_slots = 0;
+  bool ok = true;
+  auto dev = [&](auto** p, size_t bytes) {
+    void* q = nullptr;
+    if (ok && cudaMalloc(&q, std::max<size_t>(bytes, 16)) == cudaSuccess) d.dev.push_back(q);
+    else ok = false;
+    *p = (std::remove_reference_t<decltype(**p)>*)q;
+  };
+  auto pin = [&](auto** p, size_t bytes) {
+    void* q = nullptr;
+    if (ok && cudaMallocHost(&q, std::max<size_t>(bytes, 16)) == cudaSuccess) d.pin.push_back(q);
+    else ok = false;
+    *p = (std::remove_reference_t<decltype(**p)>*)q;
+  };
+  const size_t cells = (size_t)slots * LVO_DEPTH_CELLS + 1;
+  dev(&d.raw, raw); dev(&d.flag, 4 * pts); dev(&d.dc, 16 * pts);
+  dev(&d.d_in, depth_slot_bytes(slots) + 8 * kp); pin(&d.h_in, depth_slot_bytes(slots) + 8 * kp);
+  dev(&d.d_res, 20 * kp); pin(&d.h_res, 20 * kp);
+  dev(&d.dc_off, 4 * (size_t)slots); dev(&d.ndc, 4 * (size_t)slots);
+  GridSet& g = d.grid;
+  memset(&g, 0, sizeof(g));
+  g.cells_cap_per_problem = LVO_DEPTH_CELLS;
+  dev(&g.prob, sizeof(GridProblem) * slots); dev(&g.table, 4 * cells); dev(&g.d_table_len, 4);
+  dev(&g.rank, 4 * pts); dev(&g.pt_off, 4 * ((size_t)slots + 1)); dev(&g.sorted_pts, 16 * pts);   // sorted_id: no search reads it
+  g.scan.cap_tiles = lvo_div_up((long long)std::max(pts, cells), LVO_SCAN_TILE) + 2;
+  dev(&g.scan.partial, 4 * (size_t)g.scan.cap_tiles);
+  int* cnt = nullptr;
+  dev(&cnt, 8);
+  if (!ok) {
+    for (void* p : d.dev) cudaFree(p);
+    for (void* p : d.pin) cudaFreeHost(p);
+    d.dev.clear(); d.pin.clear();
+    lvo_set_error(c, "lvo_depth_associate_batch: out of memory");
+    return LVO_E_CUDA;
+  }
+  d.cnt = cnt;
+  d.cap_pts = pts; d.cap_raw = raw; d.cap_kp = kp; d.cap_slots = slots;
+  return LVO_OK;
+}
+
+// Per active lane: keypoint counts within the single call's limit, and the pointers a lane with keypoints needs.
+static int depth_check_keypoints(lvo_ctx* c, const void* const* kp, const size_t* n_kp, const void* const* depth, const void* const* valid, const void* const* nn) {
+  for (int l = 0; l < c->lanes; ++l) {
+    if (!c->lane_active[l] || n_kp[l] == 0) continue;
+    if (2 * n_kp[l] > (size_t)c->P) { lvo_set_error(c, "too many keypoints"); return LVO_E_CAPACITY; }
+    if (!kp[l] || !depth[l] || !valid[l] || (nn && !nn[l])) { lvo_set_error(c, "NULL keypoint or output pointer of an active lane"); return LVO_E_BADARG; }
+  }
+  return LVO_OK;
+}
+
+// Uploads the slots (and the host form's keypoints behind them) staged in h_in, then enqueues the kernels.
+static int depth_enqueue(lvo_ctx* c, int nslot, size_t n_total, size_t kp_total, int max_n, int stride, int off_xyz, size_t in_bytes) {
+  lvo_ctx::DepthArena& d = c->depth;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(d.d_in, d.h_in, in_bytes, cudaMemcpyHostToDevice, c->st));
+  DepthArgs a;
+  memset(&a, 0, sizeof(a));
+  a.slot = (const DepthSlot*)d.d_in; a.nslot = nslot; a.stride = stride; a.off_xyz = off_xyz;
+  a.n_total = (int)n_total; a.kp_total = (int)kp_total;
+  a.flag = d.flag; a.d_n = d.cnt; a.d_total = (unsigned*)(d.cnt + 1); a.dc_off = d.dc_off; a.ndc = d.ndc; a.dc = d.dc;
+  a.grid = d.grid;
+  a.grid.nprob = nslot; a.grid.table_cap_total = (long long)nslot * LVO_DEPTH_CELLS; a.grid.pts_cap_per_problem = std::max(max_n, 1);
+  lvo_launch_depth(c->st, a, max_n, d.grid.scan, &c->launches);
+  return LVO_OK;
+}
+
+static void depth_slot_camera(DepthSlot& s, const lvo_camera& cam) { for (int k = 0; k < 12; ++k) s.extr[k] = cam.extrinsic[k]; }
+
+int lvo_depth_associate_batch(lvo_ctx* c, const lvo_camera* cams, const lvo_cloud_view* sweeps, const float* const* keypoints_uv, const size_t* n_kp,
+                              float* const* depth_out, int* const* valid_out, int* const* nn_out_or_null) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (!cams || !sweeps || !keypoints_uv || !n_kp || !depth_out || !valid_out) { lvo_set_error(c, "NULL array"); return LVO_E_BADARG; }
+  int max_n = 0, stride = 16, off_xyz = 0;
+  LVO_TRY(check_sweeps(c, sweeps, &max_n, &stride, &off_xyz));
+  LVO_TRY(depth_check_keypoints(c, (const void* const*)keypoints_uv, n_kp, (const void* const*)depth_out, (const void* const*)valid_out,
+                                (const void* const*)nn_out_or_null));
+  int A = 0; size_t N = 0, K = 0;
+  for (int l = 0; l < c->lanes; ++l) if (c->lane_active[l]) { A++; N += sweeps[l].n; K += n_kp[l]; }
+  if (N > INT_MAX || K > INT_MAX) { lvo_set_error(c, "too many points or keypoints in one call"); return LVO_E_CAPACITY; }
+  c->launches = 0;
+  if (A == 0) return LVO_OK;
+  LVO_TRY(depth_reserve(c, N, N * stride, K, A));
+  lvo_ctx::DepthArena& d = c->depth;
+  DepthSlot* hs = (DepthSlot*)d.h_in;
+  float* huv = (float*)(d.h_in + depth_slot_bytes(A));
+  const float* d_uv = (const float*)(d.d_in + depth_slot_bytes(A));
+  float* r_depth = (float*)d.d_res; int* r_valid = (int*)d.d_res + K; int* r_nn = (int*)d.d_res + 2 * K;
+  // sweeps back to back in lane order: exactly the bytes of each view, one copy per run of views that are contiguous in host memory
+  struct Run { const unsigned char* host; size_t bytes; size_t dev_off; };
+  std::vector<Run> runs;
+  int s = 0; size_t po = 0, ko = 0;
+  for (int l = 0; l < c->lanes; ++l) {
+    if (!c->lane_active[l]) continue;
+    const lvo_cloud_view& v = sweeps[l];
+    DepthSlot& t = hs[s++];
+    memset(&t, 0, sizeof(t));
+    t.pts = d.raw + po * stride; t.n = (int)v.n; t.pt_off = (unsigned)po;
+    t.uv = d_uv + 2 * ko; t.nkp = (int)n_kp[l]; t.kp_off = (unsigned)ko;
+    t.depth = r_depth + ko; t.valid = r_valid + ko; t.nn = nn_out_or_null ? r_nn + 3 * ko : nullptr;
+    depth_slot_camera(t, cams[l]);
+    if (n_kp[l]) memcpy(huv + 2 * ko, keypoints_uv[l], 8 * n_kp[l]);
+    if (v.n) {
+      const unsigned char* h = (const unsigned char*)v.data;
+      const size_t bytes = v.n * stride;
+      if (!runs.empty() && runs.back().host + runs.back().bytes == h) runs.back().bytes += bytes;
+      else runs.push_back(Run{h, bytes, po * stride});
+    }
+    po += v.n; ko += n_kp[l];
+  }
+  for (const Run& r : runs) LVO_CUDA_OK(c, cudaMemcpyAsync(d.raw + r.dev_off, r.host, r.bytes, cudaMemcpyHostToDevice, c->st));
+  LVO_TRY(depth_enqueue(c, A, N, K, max_n, stride, off_xyz, depth_slot_bytes(A) + 8 * K));
+  const size_t res_words = (nn_out_or_null ? 5 : 2) * K;
+  if (res_words) LVO_CUDA_OK(c, cudaMemcpyAsync(d.h_res, d.d_res, 4 * res_words, cudaMemcpyDeviceToHost, c->st));
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LVO_CUDA_OK(c, cudaGetLastError());
+  const float* h_depth = (const float*)d.h_res; const int* h_valid = (const int*)d.h_res + K; const int* h_nn = (const int*)d.h_res + 2 * K;
+  ko = 0;
+  for (int l = 0; l < c->lanes; ++l) {
+    if (!c->lane_active[l] || n_kp[l] == 0) continue;
+    memcpy(depth_out[l], h_depth + ko, 4 * n_kp[l]);
+    memcpy(valid_out[l], h_valid + ko, 4 * n_kp[l]);
+    if (nn_out_or_null) memcpy(nn_out_or_null[l], h_nn + 3 * ko, 12 * n_kp[l]);
+    ko += n_kp[l];
+  }
+  return LVO_OK;
+}
+
+int lvo_depth_associate_batch_dev(lvo_ctx* c, const lvo_camera* cams, const lvo_point* const* d_sweeps, const size_t* n, const float* const* d_keypoints_uv,
+                                  const size_t* n_kp, float* const* d_depth_out, int* const* d_valid_out, int* const* d_nn_out_or_null) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (!cams || !d_sweeps || !n || !d_keypoints_uv || !n_kp || !d_depth_out || !d_valid_out) { lvo_set_error(c, "NULL array"); return LVO_E_BADARG; }
+  int A = 0, max_n = 0; size_t N = 0, K = 0;
+  for (int l = 0; l < c->lanes; ++l) {
+    if (!c->lane_active[l]) continue;
+    if (n[l] > (size_t)c->P) { lvo_set_error(c, "input cloud exceeds context capacity"); return LVO_E_CAPACITY; }
+    if (n[l] && !d_sweeps[l]) { lvo_set_error(c, "NULL sweep of an active lane"); return LVO_E_BADARG; }
+    A++; N += n[l]; K += n_kp[l]; max_n = std::max(max_n, (int)n[l]);
+  }
+  LVO_TRY(depth_check_keypoints(c, (const void* const*)d_keypoints_uv, n_kp, (const void* const*)d_depth_out, (const void* const*)d_valid_out,
+                                (const void* const*)d_nn_out_or_null));
+  if (N > INT_MAX || K > INT_MAX) { lvo_set_error(c, "too many points or keypoints in one call"); return LVO_E_CAPACITY; }
+  c->launches = 0;
+  if (A == 0) return LVO_OK;
+  LVO_TRY(depth_reserve(c, N, 0, 0, A));
+  DepthSlot* hs = (DepthSlot*)c->depth.h_in;
+  int s = 0; size_t po = 0, ko = 0;
+  for (int l = 0; l < c->lanes; ++l) {
+    if (!c->lane_active[l]) continue;
+    DepthSlot& t = hs[s++];
+    memset(&t, 0, sizeof(t));
+    t.pts = (const unsigned char*)d_sweeps[l]; t.n = (int)n[l]; t.pt_off = (unsigned)po;
+    t.uv = d_keypoints_uv[l]; t.nkp = (int)n_kp[l]; t.kp_off = (unsigned)ko;
+    t.depth = d_depth_out[l]; t.valid = d_valid_out[l]; t.nn = d_nn_out_or_null ? d_nn_out_or_null[l] : nullptr;
+    depth_slot_camera(t, cams[l]);
+    po += n[l]; ko += n_kp[l];
+  }
+  LVO_TRY(depth_enqueue(c, A, N, K, max_n, 16, 0, depth_slot_bytes(A)));
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LVO_CUDA_OK(c, cudaGetLastError());
+  return LVO_OK;
 }
 
 int lvo_knn5_throughput(lvo_ctx* c, const lvo_point* d_maps, const int* map_counts, const lvo_point* d_queries, const int* query_counts, int S, int reps,
