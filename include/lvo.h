@@ -226,8 +226,43 @@ int lvo_map_import(lvo_ctx* ctx, int lane, const lvo_point* corner, const int* c
 int lvo_map_export(lvo_ctx* ctx, int lane, int which, lvo_cloud_out* pts, int* cube_out);
 /* Map outputs of laserMapping.cpp:806-836.  which: 0 = "surround" cloud (:806-815: the cubes of the last frame's valid list in
  * i,j,k loop order, corner points then surf points of each cube), 1 = whole map (:823-836: all 4851 cubes in array order, corner
- * then surf).  The reference publishes them every 5th / 20th mapping frame; the schedule is the caller's (host/lvo_handlers.hpp). */
+ * then surf).  The reference publishes them every 5th / 20th mapping frame; the schedule is the caller's (host/lvo_handlers.hpp).
+ * Synchronous; runs the kernels of lvo_map_cloud_batch for one lane, in the arena of those calls, and leaves
+ * lvo_timings::kernel_launches as it was.  n > cap, or data == NULL with n > 0: LVO_E_CAPACITY with pts->n = n. */
 int lvo_map_cloud(lvo_ctx* ctx, int lane, int which, lvo_cloud_out* pts);
+
+/* Map outputs of every lane of the context in one call: what the reference's mapping node publishes besides the pose. */
+#define LVO_MAP_SURROUND 0   /* as lvo_map_cloud which = 0: /laser_cloud_surround, laserMapping.cpp:806-815              */
+#define LVO_MAP_WHOLE 1      /* as lvo_map_cloud which = 1: /laser_cloud_map, :823-836                                   */
+#define LVO_MAP_REGISTERED 2 /* registered full-resolution cloud of the last step: /velodyne_cloud_registered, :838-842    */
+/* outs[l] is lane l's output, for every lane of the context.
+ *   - Lane selection.  outs[l].n is written for every lane.  Points are copied only for lanes whose outs[l].data is non-NULL; a call
+ *     whose destinations are all NULL is a size query (which = 0 / 1: one launch; which = 2: none).  So a caller can keep the
+ *     reference's 5th / 20th-frame schedule for each lane.
+ *   - LVO_MAP_SURROUND / LVO_MAP_WHOLE: every lane, active or idle, gets exactly the points, in the same order, that
+ *     lvo_map_cloud(ctx, l, which, ...) returns, from the current map.  A freshly created or reset lane has an empty map (n = 0); a
+ *     lane loaded with lvo_lane_load gets its snapshot's map at once.
+ *   - LVO_MAP_REGISTERED reports the lanes that mapped in the last lvo_step_batch* call: each gets the n_kept points of that frame
+ *     moved into the map frame, bit for bit what lvo_probe_fetch(LVO_P_REGISTERED) returns right after that step.  Every other lane
+ *     gets n = 0 and its destination is not written: lanes that did not map (off their skip_frame phase or idle), and lanes reset or
+ *     loaded since the step.  The counts are recorded on the host when the step completes.  lvo_scan_to_map, lvo_knn and
+ *     lvo_depth_associate overwrite the registered clouds; after any of them which = 2 returns LVO_E_STATE (lvo_last_error says
+ *     why) until the next lvo_step_batch* call completes.
+ *   - Errors, each checked before any destination is written: LVO_E_BADARG for a NULL array or a bad `which`; LVO_E_STATE while an
+ *     *_async step is in flight, or after the invalidation above; LVO_E_CAPACITY when a selected lane's cap is below its n (every n
+ *     is still written, and no point is copied for any lane).
+ *   - Synchronous on return, on the context's stream (lvo_set_stream).  which = 0 / 1 count the lanes' clouds in one launch and copy
+ *     them in a second one; one small device-to-host copy of the per-lane totals between the two is the only synchronisation inside
+ *     the call.  which = 2 is one launch.  These launch counts do not depend on the number of lanes (lvo_timings::kernel_launches
+ *     reports them).  The host form gathers the selected clouds back to back on the device and copies each to its buffer once.
+ *   - The calls use their own device arena: per-lane descriptors, offset tables and totals, allocated on the first call, and a point
+ *     buffer on the device that grows, never shrinks, when a host-form call brings more points; lvo_destroy frees it.
+ *     They read and write no state of the step: lane states, maps, probes, staging buffers, the prefetch of
+ *     lvo_step_batch_pipelined and captured CUDA graphs are left as they were. */
+int lvo_map_cloud_batch(lvo_ctx* ctx, int which, lvo_cloud_out* outs);
+/* Same, into device memory of the context's device: d_out[l] (NULL = lane not copied) holds cap[l] points; n_out[l] gets every
+ * lane's count.  The arena's point buffer is neither allocated nor used by this form. */
+int lvo_map_cloud_batch_dev(lvo_ctx* ctx, int which, lvo_point* const* d_out, const size_t* cap, size_t* n_out);
 /* (q_wmap_wodom, t_wmap_wodom), laserMapping.cpp:116-117 */
 int lvo_get_map_correction(lvo_ctx* ctx, int lane, lvo_pose* T_wmap_wodom);
 int lvo_set_map_correction(lvo_ctx* ctx, int lane, const lvo_pose* T_wmap_wodom);

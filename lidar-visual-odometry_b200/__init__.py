@@ -21,6 +21,7 @@ LVO_OPT_FIXPOINT_SKIP = 2
 LVO_OPT_STAGE_TIMING = 3
 LVO_OPT_KNN_REUSE = 5
 LVO_OPT_ODO_REUSE = 6
+LVO_MAP_SURROUND, LVO_MAP_WHOLE, LVO_MAP_REGISTERED = 0, 1, 2
 
 # enum lvo_probe
 (P_FULL, P_CURVATURE, P_SORT_IND, P_LABEL, P_PICKED, P_SCAN_START, P_SCAN_END, P_SHARP, P_LESS_SHARP, P_FLAT, P_LESS_FLAT,
@@ -87,7 +88,8 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_get_map_correction", "lvo_set_map_correction", "lvo_set_odometry_state", "lvo_probe_fetch", "lvo_voxel_downsample", "lvo_knn",
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
            "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
-           "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load", "lvo_depth_associate_batch", "lvo_depth_associate_batch_dev"]
+           "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load", "lvo_depth_associate_batch", "lvo_depth_associate_batch_dev",
+           "lvo_map_cloud_batch", "lvo_map_cloud_batch_dev"]
 
 
 def load_library():
@@ -119,6 +121,8 @@ def load_library():
     L.lvo_map_import.argtypes = [vp, ip, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
     L.lvo_map_export.argtypes = [vp, ip, ip, C.POINTER(CloudOut), vp]
     L.lvo_map_cloud.argtypes = [vp, ip, ip, C.POINTER(CloudOut)]
+    L.lvo_map_cloud_batch.argtypes = [vp, ip, C.POINTER(CloudOut)]
+    L.lvo_map_cloud_batch_dev.argtypes = [vp, ip, C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
     L.lvo_transform_cloud.argtypes = [vp, CloudView, C.POINTER(Pose), ip, C.POINTER(CloudOut)]
     L.lvo_get_map_correction.argtypes = [vp, ip, C.POINTER(Pose)]
     L.lvo_set_map_correction.argtypes = [vp, ip, C.POINTER(Pose)]
@@ -378,6 +382,26 @@ class Lvo:
         out, buf = self._out(cap)
         self._check(self.lib.lvo_map_cloud(self.h, lane, which, C.byref(out)))
         return buf[:out.n].copy()
+
+    def map_cloud_batch(self, which, lanes=None):
+        """Map outputs of every lane in one call (lvo_map_cloud_batch).  which: LVO_MAP_SURROUND, LVO_MAP_WHOLE or LVO_MAP_REGISTERED;
+        lanes: the lanes to fetch (None: all).  Returns one (n,4) float32 array per lane, None for a lane that was not requested."""
+        want = set(range(self.lanes)) if lanes is None else set(lanes)
+        outs = (CloudOut * self.lanes)()
+        self._check(self.lib.lvo_map_cloud_batch(self.h, which, outs))   # size query: every destination NULL
+        bufs = [np.empty((max(outs[l].n, 1), 4), np.float32) if l in want else None for l in range(self.lanes)]
+        for l, b in enumerate(bufs):
+            outs[l] = CloudOut(b.ctypes.data, len(b), 0) if b is not None else CloudOut(None, 0, 0)
+        self._check(self.lib.lvo_map_cloud_batch(self.h, which, outs))
+        return [b[:outs[l].n].copy() if b is not None else None for l, b in enumerate(bufs)]
+
+    def map_cloud_batch_dev(self, which, d_out, caps):
+        """Device form (lvo_map_cloud_batch_dev): d_out[l] is a device pointer (None: lane not copied) with room for caps[l] points.
+        Returns every lane's point count."""
+        n = (C.c_size_t * self.lanes)()
+        self._check(self.lib.lvo_map_cloud_batch_dev(self.h, which, (C.c_void_p * self.lanes)(*[int(p or 0) for p in d_out]),
+                                                     (C.c_size_t * self.lanes)(*[int(c or 0) for c in caps]), n))
+        return list(n)
 
     def transform_cloud(self, pts, T_last_curr=None, to_end=False):
         """TransformToStart / TransformToEnd (laserOdometry.cpp:154-191) with the context's distortion mode."""

@@ -11,6 +11,7 @@
 #include "lvo_odometry.cuh"
 #include "lvo_mapping.cuh"
 #include "lvo_depth.cuh"
+#include "lvo_outputs.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -94,6 +95,21 @@ struct lvo_ctx {
     int* cnt = nullptr;                // scan length, depth-cloud total
     GridSet grid;                      // one problem per slot, LVO_DEPTH_CELLS cells each
   } depth;
+  // lvo_map_cloud / lvo_map_cloud_batch*: the calls' own arena (DESIGN §3), allocated on the first call; the point buffer grows, never
+  // shrinks, when a call brings more points; the step's buffers are not touched
+  struct MapOutArena {
+    std::vector<void*> dev, pin;       // the per-slot part, sized for every lane of the context
+    MapOutDesc* d_desc = nullptr; MapOutDesc* h_desc = nullptr;   // [lanes] copy descriptors and their pinned staging
+    unsigned* off = nullptr;           // [lanes][LVO_NCUBES + 1] cube offsets of each slot's cloud
+    unsigned* d_tot = nullptr; unsigned* h_tot = nullptr;         // [lanes] points of each slot's cloud
+    size_t cap_pts = 0;
+    float4* d_pts = nullptr;           // [cap_pts] host form: the selected lanes' clouds back to back
+  } mapout;
+  // lvo_map_cloud_batch* LVO_MAP_REGISTERED: points of each lane's registered cloud in the last lvo_step_batch* call (n_kept of that
+  // frame for a lane that mapped, 0 otherwise), recorded by step_finish; reg_valid is false once lvo_scan_to_map, lvo_knn or
+  // lvo_depth_associate has overwritten map.registered, until the next step completes
+  std::vector<size_t> reg_n;
+  bool reg_valid = true;
 };
 
 void lvo_set_error(lvo_ctx* ctx, const std::string& msg) { if (ctx) ctx->err = msg; }
@@ -208,40 +224,6 @@ __global__ void k_transform_cloud(const LaneState* ls, PoseArg pa, const float4*
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
     out[i] = to_end ? transform_to_end(q, t, in[i]) : transform_to_start(q, t, in[i], distortion);
 }
-// lvo_map_cloud: slot k = rank in the valid list (surround) or cube index (whole map); off[k] = exclusive prefix of the
-// corner + surf counts of the slots before it
-__global__ void __launch_bounds__(256) k_mapcloud_offsets(MapArgs a, int lane, int surround, unsigned* off) {
-  __shared__ unsigned sm[33];
-  const LaneState& s = a.ls[lane];
-  const int n = surround ? s.n_valid : LVO_NCUBES;
-  const unsigned* cs0 = a.cube_start[a.gen][0] + (size_t)lane * (LVO_NCUBES + 1);
-  const unsigned* cs1 = a.cube_start[a.gen][1] + (size_t)lane * (LVO_NCUBES + 1);
-  unsigned carry = 0;
-  for (int base = 0; base < n; base += blockDim.x) {
-    const int k = base + threadIdx.x;
-    unsigned cnt = 0;
-    if (k < n) { const int c = surround ? s.valid_cube[k] : k; cnt = (cs0[c + 1] - cs0[c]) + (cs1[c + 1] - cs1[c]); }
-    unsigned tot;
-    const unsigned ex = block_excl_scan(cnt, sm, &tot);
-    if (k < n) off[k] = carry + ex;
-    carry += tot;
-  }
-  if (threadIdx.x == 0) off[LVO_NCUBES] = carry;
-}
-__global__ void k_mapcloud_copy(MapArgs a, int lane, int surround, const unsigned* off, float4* out) {
-  const LaneState& s = a.ls[lane];
-  const int n = surround ? s.n_valid : LVO_NCUBES;
-  const unsigned* cs0 = a.cube_start[a.gen][0] + (size_t)lane * (LVO_NCUBES + 1);
-  const unsigned* cs1 = a.cube_start[a.gen][1] + (size_t)lane * (LVO_NCUBES + 1);
-  const float4* M0 = a.map_pts[a.gen][0] + (size_t)lane * a.map_cap[0];
-  const float4* M1 = a.map_pts[a.gen][1] + (size_t)lane * a.map_cap[1];
-  for (int k = blockIdx.x; k < n; k += gridDim.x) {
-    const int c = surround ? s.valid_cube[k] : k;
-    const unsigned b0 = cs0[c], n0 = cs0[c + 1] - b0, b1 = cs1[c], n1 = cs1[c + 1] - b1, o = off[k];
-    for (unsigned i = threadIdx.x; i < n0 + n1; i += blockDim.x) out[o + i] = i < n0 ? M0[b0 + i] : M1[b1 + (i - n0)];
-  }
-}
-
 // xyz_only: the cloud is a raw sweep, whose intensity the path never reads (scanRegistration.cpp:132-133 converts to pcl::PointXYZ):
 // records of 12 bytes (packed x, y, z) are accepted and off_intensity is ignored.
 int check_view(lvo_ctx* c, const lvo_cloud_view& v, size_t cap, bool xyz_only = false) {
@@ -462,6 +444,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   c->lane_frame.assign(L, 0);
   c->lane_active.assign(L, 1);
   c->probe_gate.assign(L, 0);
+  c->reg_n.assign(L, 0);
 
   LVO_TRY(dalloc(c, &c->d_ls, (size_t)L));
   LVO_TRY(halloc(c, &c->h_ls, (size_t)L));
@@ -590,6 +573,9 @@ int lvo_destroy(lvo_ctx* c) {
   for (void* p : c->pinned) cudaFreeHost(p);
   for (void* p : c->depth.dev) cudaFree(p);
   for (void* p : c->depth.pin) cudaFreeHost(p);
+  for (void* p : c->mapout.dev) cudaFree(p);
+  for (void* p : c->mapout.pin) cudaFreeHost(p);
+  if (c->mapout.d_pts) cudaFree(c->mapout.d_pts);
   destroy_graphs(c);
   if (c->copy_st) { cudaStreamSynchronize(c->copy_st); cudaStreamDestroy(c->copy_st); cudaEventDestroy(c->copy_ev); cudaEventDestroy(c->compute_ev); }
   if (c->own_st) { for (int i = 0; i < 8; ++i) cudaEventDestroy(c->ev[i]); c->stage_tm.destroy(); cudaStreamDestroy(c->own_st); }
@@ -714,6 +700,7 @@ int lvo_scan_to_map(lvo_ctx* c, lvo_cloud_view corner_last, lvo_cloud_view surf_
   LVO_TRY(check_view(c, corner_last, (size_t)c->cap_lsharp)); LVO_TRY(check_view(c, surf_last, (size_t)c->P));
   LVO_TRY(check_view(c, full_or_null, (size_t)c->P));
   c->launches = 0;
+  c->reg_valid = false;   // its k_register rewrites map.registered
   cudaEventRecord(c->ev[4], c->st);
   LVO_TRY(upload_cloud(c, corner_last, c->ex.less_sharp)); LVO_TRY(upload_cloud(c, surf_last, c->ex.less_flat));
   const bool want_reg = registered_or_null && full_or_null.n > 0;
@@ -846,6 +833,10 @@ static int step_finish(lvo_ctx* c, lvo_pose* T_wodom, lvo_pose* T_wmap) {
   const bool do_map = c->pending_do_map;
   LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
   LVO_CUDA_OK(c, cudaGetLastError());
+  // the registered clouds of this step (k_register ran for the lanes that mapped): their sizes are n_kept of this frame, read here
+  // because a later extraction rewrites n_kept
+  for (int l = 0; l < c->lanes; ++l) c->reg_n[l] = (lane_flags(c)[l] & LVO_LANE_MAPS) ? (size_t)c->h_ls[l].n_kept : 0;
+  c->reg_valid = true;
   if (c->pending_graph) {
     c->tim.extract_ms = c->tim.odometry_ms = 0.f;     // per-stage times are only available with plain launches
     cudaEventElapsedTime(&c->tim.mapping_ms, c->ev[0], c->ev[3]);
@@ -1003,6 +994,7 @@ int lvo_lane_reset(lvo_ctx* c, int lane) {
   c->lane_status[lane] = LVO_OK;
   c->lane_frame[lane] = 0;
   c->probe_gate[lane] = 0;   // zero counts: every probe is empty, and in bounds
+  c->reg_n[lane] = 0;
   return LVO_OK;
 }
 
@@ -1203,6 +1195,7 @@ int lvo_lane_load(lvo_ctx* c, int lane, const void* src, size_t n_bytes) {
   c->lane_status[lane] = h.lane_status;
   c->probe_gate[lane] = LVO_PROBE_GATE_EXTRACT | LVO_PROBE_GATE_ODO | LVO_PROBE_GATE_MAP;
   c->odo_grids_stale = true;
+  c->reg_n[lane] = 0;
   return LVO_OK;
 }
 
@@ -1251,20 +1244,174 @@ int lvo_map_export(lvo_ctx* c, int lane, int which, lvo_cloud_out* pts, int* cub
   return LVO_OK;
 }
 
+// ---- map outputs (DESIGN §3 "Map-output arena"): one launch sequence for any number of lanes, slot s = lane first_lane + s
+static int mapout_fail(lvo_ctx* c, cudaError_t e) { lvo_set_error(c, std::string("map outputs: ") + cudaGetErrorString(e)); return LVO_E_CUDA; }
+// The per-slot part, allocated on the first call for every lane of the context.
+static int mapout_reserve_slots(lvo_ctx* c) {
+  lvo_ctx::MapOutArena& m = c->mapout;
+  auto fail = [&](cudaError_t e) { return mapout_fail(c, e); };
+  if (!m.d_desc) {
+    const size_t L = (size_t)c->lanes;
+    void* q[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    const size_t dev_bytes[3] = {L * sizeof(MapOutDesc), L * LVO_MAPOUT_STRIDE * sizeof(unsigned), L * sizeof(unsigned)};
+    for (int k = 0; k < 3; ++k) { cudaError_t e = cudaMalloc(&q[k], dev_bytes[k]); if (e != cudaSuccess) return fail(e); m.dev.push_back(q[k]); }
+    for (int k = 3; k < 5; ++k) {
+      cudaError_t e = cudaMallocHost(&q[k], k == 3 ? L * sizeof(MapOutDesc) : L * sizeof(unsigned));
+      if (e != cudaSuccess) return fail(e);
+      m.pin.push_back(q[k]);
+    }
+    m.d_desc = (MapOutDesc*)q[0]; m.off = (unsigned*)q[1]; m.d_tot = (unsigned*)q[2]; m.h_desc = (MapOutDesc*)q[3]; m.h_tot = (unsigned*)q[4];
+  }
+  return LVO_OK;
+}
+// The host form's point buffer, grown to `pts`.  Every call ends synchronised, so the old buffer can be freed at once.
+static int mapout_reserve_points(lvo_ctx* c, size_t pts) {
+  lvo_ctx::MapOutArena& m = c->mapout;
+  LVO_TRY(mapout_reserve_slots(c));
+  if (m.d_pts && pts <= m.cap_pts) return LVO_OK;
+  pts = std::max<size_t>({pts, m.cap_pts + m.cap_pts / 2, 1024});   // a growing map does not reallocate on every call
+  if (m.d_pts) { cudaFree(m.d_pts); m.d_pts = nullptr; }
+  m.cap_pts = 0;
+  cudaError_t e = cudaMalloc(&m.d_pts, pts * sizeof(float4));
+  if (e != cudaSuccess) { m.d_pts = nullptr; return mapout_fail(c, e); }
+  m.cap_pts = pts;
+  return LVO_OK;
+}
+
+static MapOutArgs mapout_args(const lvo_ctx* c, int which, int first_lane) {
+  MapOutArgs a;
+  memset(&a, 0, sizeof(a));
+  a.ls = c->d_ls;
+  for (int t = 0; t < 2; ++t) { a.cube_start[t] = c->map.cube_start[c->map.gen][t]; a.map_pts[t] = c->map.map_pts[c->map.gen][t]; a.map_cap[t] = c->map.map_cap[t]; }
+  a.first_lane = first_lane;
+  a.surround = which == LVO_MAP_SURROUND;
+  return a;
+}
+
+// which 0 / 1: the cloud sizes of S slots (one launch and the call's only synchronisation)
+static int mapout_count(lvo_ctx* c, const MapOutArgs& a, int S, size_t* n) {
+  lvo_ctx::MapOutArena& m = c->mapout;
+  k_mapout_offsets<<<S, 256, 0, c->st>>>(a, m.off, m.d_tot);
+  c->launches++;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(m.h_tot, m.d_tot, sizeof(unsigned) * S, cudaMemcpyDeviceToHost, c->st));
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LVO_CUDA_OK(c, cudaGetLastError());
+  for (int s = 0; s < S; ++s) n[s] = m.h_tot[s];
+  return LVO_OK;
+}
+
+// Uploads the descriptors staged in h_desc[0, S) and enqueues the copy kernel (not synchronised).
+static int mapout_copy(lvo_ctx* c, int which, const MapOutArgs& a, int S) {
+  lvo_ctx::MapOutArena& m = c->mapout;
+  LVO_CUDA_OK(c, cudaMemcpyAsync(m.d_desc, m.h_desc, sizeof(MapOutDesc) * S, cudaMemcpyHostToDevice, c->st));
+  if (which == LVO_MAP_REGISTERED) k_mapout_registered<<<dim3(64, S), 256, 0, c->st>>>(c->map.registered, c->P, m.d_desc);
+  else k_mapout_copy<<<dim3(which == LVO_MAP_SURROUND ? LVO_MAX_VALID : 296, S), 256, 0, c->st>>>(a, m.d_desc, m.off);
+  c->launches++;
+  return LVO_OK;
+}
+
+// Host form: the selected slots' clouds (dst[s] != NULL) are gathered back to back into the arena, and each goes to the caller's
+// buffer in one cudaMemcpyAsync.  profiles/map_outputs.md compares this with one packed download into pinned memory followed by a
+// host scatter.
+static int mapout_host(lvo_ctx* c, int which, const MapOutArgs& a, int S, const size_t* n, lvo_point* const* dst) {
+  lvo_ctx::MapOutArena& m = c->mapout;
+  size_t total = 0; bool any = false;
+  for (int s = 0; s < S; ++s) if (dst[s]) { total += n[s]; any = true; }
+  if (!any) return LVO_OK;
+  LVO_TRY(mapout_reserve_points(c, total));
+  size_t o = 0;
+  for (int s = 0; s < S; ++s) {
+    m.h_desc[s] = MapOutDesc{dst[s] ? m.d_pts + o : nullptr, (unsigned)n[s], 0u};
+    if (dst[s]) o += n[s];
+  }
+  LVO_TRY(mapout_copy(c, which, a, S));
+  o = 0;
+  for (int s = 0; s < S; ++s) {
+    if (!dst[s]) continue;
+    if (n[s]) LVO_CUDA_OK(c, cudaMemcpyAsync(dst[s], m.d_pts + o, n[s] * sizeof(float4), cudaMemcpyDeviceToHost, c->st));
+    o += n[s];
+  }
+  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+  LVO_CUDA_OK(c, cudaGetLastError());
+  return LVO_OK;
+}
+
+// Checks shared by the batch forms; n[l] gets every lane's count.  Nothing is written to a destination before it returns.
+static int mapout_batch_begin(lvo_ctx* c, int which, size_t* n, MapOutArgs* a) {
+  if (which < LVO_MAP_SURROUND || which > LVO_MAP_REGISTERED) { lvo_set_error(c, "bad `which`: LVO_MAP_SURROUND, LVO_MAP_WHOLE or LVO_MAP_REGISTERED"); return LVO_E_BADARG; }
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (which == LVO_MAP_REGISTERED && !c->reg_valid) {
+    lvo_set_error(c, "the registered clouds were overwritten by lvo_scan_to_map, lvo_knn or lvo_depth_associate; the next lvo_step_batch* call makes them available again");
+    return LVO_E_STATE;
+  }
+  c->launches = 0;
+  *a = mapout_args(c, which, 0);
+  if (which == LVO_MAP_REGISTERED) { for (int l = 0; l < c->lanes; ++l) n[l] = c->reg_n[l]; return LVO_OK; }
+  LVO_TRY(mapout_reserve_slots(c));
+  return mapout_count(c, *a, c->lanes, n);
+}
+
+static int map_cloud_one(lvo_ctx* c, int lane, int which, lvo_cloud_out* pts) {
+  LVO_TRY(mapout_reserve_slots(c));
+  const MapOutArgs a = mapout_args(c, which, lane);
+  size_t n = 0;
+  LVO_TRY(mapout_count(c, a, 1, &n));
+  pts->n = n;
+  if (n > pts->cap || (n && !pts->data)) { lvo_set_error(c, "output cloud buffer too small"); return LVO_E_CAPACITY; }
+  lvo_point* dst = pts->data;
+  return mapout_host(c, which, a, 1, &n, &dst);
+}
 int lvo_map_cloud(lvo_ctx* c, int lane, int which, lvo_cloud_out* pts) {
   LvoDeviceGuard _dev(c);
   if (!c || lane < 0 || lane >= c->lanes || which < 0 || which > 1 || !pts) return LVO_E_BADARG;
-  unsigned* off = c->map.new_cnt;              // [LVO_NCUBES + 1] scratch (rewritten by every mapping frame)
-  float4* out = (float4*)c->d_upload;          // >= 4 * max(map_cap) points
-  k_mapcloud_offsets<<<1, 256, 0, c->st>>>(c->map, lane, which == 0, off);
-  k_mapcloud_copy<<<which == 0 ? LVO_MAX_VALID : 296, 256, 0, c->st>>>(c->map, lane, which == 0, off, out);
-  unsigned n = 0;
-  LVO_CUDA_OK(c, cudaMemcpyAsync(&n, off + LVO_NCUBES, 4, cudaMemcpyDeviceToHost, c->st));
+  const long long launches = c->launches;   // lvo_timings::kernel_launches keeps reporting the last step / stage call
+  const int r = map_cloud_one(c, lane, which, pts);
+  c->launches = launches;
+  return r;
+}
+
+int lvo_map_cloud_batch(lvo_ctx* c, int which, lvo_cloud_out* outs) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (!outs) { lvo_set_error(c, "NULL array"); return LVO_E_BADARG; }
+  const int L = c->lanes;
+  std::vector<size_t> n(L);
+  MapOutArgs a;
+  LVO_TRY(mapout_batch_begin(c, which, n.data(), &a));
+  std::vector<lvo_point*> dst(L);
+  int short_lane = -1;
+  for (int l = 0; l < L; ++l) {
+    outs[l].n = n[l];
+    dst[l] = outs[l].data;
+    if (dst[l] && outs[l].cap < n[l] && short_lane < 0) short_lane = l;
+  }
+  if (short_lane >= 0) { lvo_set_error(c, "output buffer of lane " + std::to_string(short_lane) + " too small"); return LVO_E_CAPACITY; }
+  return mapout_host(c, which, a, L, n.data(), dst.data());
+}
+
+int lvo_map_cloud_batch_dev(lvo_ctx* c, int which, lvo_point* const* d_out, const size_t* cap, size_t* n_out) {
+  LvoDeviceGuard _dev(c);
+  if (!c) return LVO_E_BADARG;
+  if (!d_out || !cap || !n_out) { lvo_set_error(c, "NULL array"); return LVO_E_BADARG; }
+  const int L = c->lanes;
+  std::vector<size_t> n(L);
+  MapOutArgs a;
+  LVO_TRY(mapout_batch_begin(c, which, n.data(), &a));
+  int short_lane = -1;
+  bool any = false;
+  for (int l = 0; l < L; ++l) {
+    n_out[l] = n[l];
+    any = any || d_out[l];
+    if (d_out[l] && cap[l] < n[l] && short_lane < 0) short_lane = l;
+  }
+  if (short_lane >= 0) { lvo_set_error(c, "output buffer of lane " + std::to_string(short_lane) + " too small"); return LVO_E_CAPACITY; }
+  if (!any) return LVO_OK;
+  LVO_TRY(mapout_reserve_slots(c));
+  for (int l = 0; l < L; ++l) c->mapout.h_desc[l] = MapOutDesc{(float4*)d_out[l], (unsigned)n[l], 0u};
+  LVO_TRY(mapout_copy(c, which, a, L));
   LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
   LVO_CUDA_OK(c, cudaGetLastError());
-  const int r = download_cloud(c, out, n, pts);
-  LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
-  return r;
+  return LVO_OK;
 }
 
 int lvo_transform_cloud(lvo_ctx* c, lvo_cloud_view in, const lvo_pose* T, int to_end, lvo_cloud_out* out) {
@@ -1439,6 +1586,7 @@ int lvo_knn(lvo_ctx* c, lvo_cloud_view cloud, lvo_cloud_view queries, int K, flo
   c->launches = 0;
   float4* d_cloud = c->map.from_map[1];
   float4* d_q = c->map.registered;
+  c->reg_valid = false;   // the queries are staged in map.registered
   LVO_TRY(upload_cloud(c, cloud, d_cloud)); LVO_TRY(upload_cloud(c, queries, d_q));
   const int n = (int)cloud.n;
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->d_knn_n, &n, 4, cudaMemcpyHostToDevice, c->st));
@@ -1484,6 +1632,7 @@ int lvo_depth_associate(lvo_ctx* c, lvo_cloud_view sweep, const lvo_camera* cam,
   // the one slot descriptor goes to the strided-upload scratch once k_unpack has consumed it (stream order); that scratch holds
   // 64 * max(max_points, max_map_corner, max_map_surf) bytes
   if ((size_t)std::max(c->P, std::max(c->map.map_cap[0], c->map.map_cap[1])) * 64 < sizeof(DepthSlot)) { lvo_set_error(c, "context too small for lvo_depth_associate"); return LVO_E_CAPACITY; }
+  c->reg_valid = false;   // the depth cloud is built in map.registered
   LVO_TRY(upload_cloud(c, sweep, d_sweep));
   if (n_kp) LVO_CUDA_OK(c, cudaMemcpyAsync(d_uv, keypoints_uv, 2 * n_kp * sizeof(float), cudaMemcpyHostToDevice, c->st));
   DepthSlot slot;
