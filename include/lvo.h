@@ -124,7 +124,7 @@ int lvo_destroy(lvo_ctx* ctx);
 const char* lvo_last_error(const lvo_ctx* ctx);
 int lvo_get_stats(const lvo_ctx* ctx, int lane, lvo_stats* out, size_t bytes);
 
-/* ---- the three drop-in entry points (lane 0; synchronous on return) --------------------------------------- */
+/* ---- the three drop-in entry points (lane 0 with lane 0's lvo_lane_config; synchronous on return) ----------- */
 
 /* scanRegistration.cpp:127-411.  `sweep` = /velodyne_points; outputs = /velodyne_cloud_2, /laser_cloud_sharp,
  * /laser_cloud_less_sharp, /laser_cloud_flat, /laser_cloud_less_flat (:413-441).  Any output may be NULL. */
@@ -186,15 +186,44 @@ int lvo_lane_status(const lvo_ctx* ctx, int lane);
 int lvo_set_lane_active(lvo_ctx* ctx, int lane, int active);
 /* Return `lane` to the state of a freshly created context: next active step is its first frame (LVO_W_FIRST_FRAME), empty map,
  * identity poses and map correction, cen = (10, 10, 5), zero lvo_stats, status LVO_OK, skip_frame phase 0.  Other lanes are
- * untouched, and so is the lane's activity.  Stream-ordered (returns when done); LVO_E_STATE while an *_async step is in flight,
+ * untouched, and so are the lane's activity and its settings (lvo_lane_configure).  Stream-ordered (returns when done); LVO_E_STATE while an *_async step is in flight,
  * LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid.  To resume a saved sequence exactly, use lvo_lane_load instead; to
  * start a new sequence from a pre-built map, follow the reset with lvo_map_import / lvo_set_odometry_state. */
 int lvo_lane_reset(lvo_ctx* ctx, int lane);
 
+/* ---- per-lane sensor settings: sequences of VLP-16, HDL-32 and HDL-64 sensors side by side in one context ---------------- */
+
+/* The values the reference's launch files set per sensor model (launch/aloam_velodyne_VLP_16.launch: 16, 0.3, 0.2, 0.4;
+ * aloam_velodyne_HDL_64.launch: 64, 5.0, 0.4, 0.8; both with mapping_skip_frame 1).  Same meaning and units as in lvo_config. */
+typedef struct lvo_lane_config {
+  int n_scans;           /* 16 | 32 | 64, and <= the context's lvo_config::n_scans   scan_line               */
+  double minimum_range;  /* m, finite and >= 0                                        minimum_range           */
+  double line_res;       /* corner voxel leaf, m, finite and > 0                      mapping_line_resolution  */
+  double plane_res;      /* surf voxel leaf, m, finite and > 0                        mapping_plane_resolution */
+  int skip_frame;        /* >= 1                                                      mapping_skip_frame       */
+} lvo_lane_config;
+/* Start a new sequence in `lane` with the settings `cfg` (NULL: the context's own values): everything lvo_lane_reset does (the next
+ * active step is the lane's first frame, its skip_frame phase 0), then the lane takes the settings.  They change only here, at the
+ * start of a sequence, as the reference reads them once at start-up.  Every other lane and the lane's activity are untouched.
+ *   - A lane that was never configured has the context's lvo_config values; lvo_lane_reset and lvo_lane_load keep a lane's settings.
+ *   - A lane computes bit for bit what lane 0 of a context created with its settings computes; the context's n_scans, the largest a
+ *     lane may take, only sizes the buffers: a 16-beam lane of a 64-beam context holds 64-beam feature buffers (DESIGN.md §1).
+ *   - outer_iters, lm_max_iters, huber and distortion are solver settings and stay per context.
+ *   - Errors, all checked before anything is written (the lane's state and settings are left as they were; lvo_last_error names the
+ *     field): LVO_E_BADARG for n_scans not 16, 32 or 64, a minimum_range that is not finite or is negative, a resolution that is not
+ *     finite or is <= 0 (each as the float the kernels use), skip_frame < 1, or a bad lane; LVO_E_CAPACITY for n_scans above the
+ *     context's; LVO_E_STATE while an *_async step is in flight.
+ *   - Stream-ordered, returns when done.  Captured CUDA graphs stay valid, and a step launches the same kernels whatever the lanes'
+ *     settings. */
+int lvo_lane_configure(lvo_ctx* ctx, int lane, const lvo_lane_config* cfg_or_null);
+/* The settings of `lane`.  LVO_E_BADARG for a bad lane or a NULL `out`. */
+int lvo_lane_get_config(const lvo_ctx* ctx, int lane, lvo_lane_config* out);
+
 /* ---- lane snapshots: checkpoint / resume, and moving a running lane to another lane, context or GPU -------- */
 
 /* Snapshot of everything `lane` carries into its next frame: its device state (poses, map correction, cube window, lvo_stats, ...),
- * the odometry "last" clouds, the current map with its cube offset tables, its skip_frame phase and lvo_lane_status.  Per-frame
+ * the odometry "last" clouds, the current map with its cube offset tables, its skip_frame phase and lvo_lane_status, and as a
+ * fingerprint the settings it ran with (the lane's lvo_lane_config, the context's solver settings).  Per-frame
  * intermediates (probes, the registered cloud) are not included.  The format is versioned and documented in DESIGN.md §3; it holds
  * no lane index, device or pointer, so two lanes that ran the same sequence give the same bytes.  `dst` may be host memory
  * (pageable or pinned) or device memory of any device.  dst == NULL or cap too small: LVO_E_CAPACITY with *n_bytes = the size
@@ -202,9 +231,10 @@ int lvo_lane_reset(lvo_ctx* ctx, int lane);
  * LVO_E_BADARG for a bad lane. */
 int lvo_lane_save(lvo_ctx* ctx, int lane, void* dst, size_t cap, size_t* n_bytes);
 /* Replace the state of `lane` with a snapshot (host or device memory, any device): its next active step continues the saved
- * sequence exactly as the source lane would have.  The destination may be any lane of any context whose n_scans, minimum_range,
- * line_res, plane_res, skip_frame, outer_iters, lm_max_iters, huber and distortion equal the source's (else LVO_E_BADARG, and
- * lvo_last_error names the field); its capacities may differ as long as the saved clouds and map, and the point counts of the
+ * sequence exactly as the source lane would have.  The destination may be any lane of any context whose lane settings (n_scans,
+ * minimum_range, line_res, plane_res, skip_frame: lvo_lane_get_config) and context settings (outer_iters, lm_max_iters, huber,
+ * distortion) equal the source's (else LVO_E_BADARG, and lvo_last_error names the field).  The load does not change the lane's
+ * settings: to move a 16-beam lane into a lane of a 64-beam context, lvo_lane_configure that lane first.  Its capacities may differ as long as the saved clouds and map, and the point counts of the
  * lane's last frame, fit (else LVO_E_CAPACITY).  The snapshot is checked in full before anything is written: a malformed one
  * returns LVO_E_BADARG and leaves the lane as it was.
  * lvo_get_stats, lvo_lane_status, lvo_map_export, lvo_map_cloud and lvo_get_map_correction report the snapshot at once;
@@ -276,8 +306,8 @@ enum lvo_probe {
   LVO_P_SORT_IND = 2,      /* int[n_kept]        cloudSortInd after all sector sorts      :288                        */
   LVO_P_LABEL = 3,         /* int[n_kept]        cloudLabel                               :303,309,355                */
   LVO_P_PICKED = 4,        /* int[n_kept]        cloudNeighborPicked                      :317-342                    */
-  LVO_P_SCAN_START = 5,    /* int[n_scans]       scanStartInd                             :249                        */
-  LVO_P_SCAN_END = 6,      /* int[n_scans]       scanEndInd                               :251                        */
+  LVO_P_SCAN_START = 5,    /* int[n_scans]       scanStartInd (the lane's n_scans)        :249                        */
+  LVO_P_SCAN_END = 6,      /* int[n_scans]       scanEndInd (the lane's n_scans)          :251                        */
   LVO_P_SHARP = 7, LVO_P_LESS_SHARP = 8, LVO_P_FLAT = 9, LVO_P_LESS_FLAT = 10, /* lvo_point[]                          */
   LVO_P_ODO_CORNER_CORR = 11, /* int[outer][n_sharp][2]  (closestPointInd, minPointInd2) or -1  laserOdometry.cpp:388-442 */
   LVO_P_ODO_PLANE_CORR = 12,  /* int[outer][n_flat][3]   (closest, minPointInd2, minPointInd3)   :472-534             */

@@ -47,6 +47,11 @@ class Config(C.Structure):
                 ("lanes", C.c_int), ("max_points", C.c_int), ("max_map_corner", C.c_int), ("max_map_surf", C.c_int), ("distortion", C.c_int), ("debug_probes", C.c_int)]
 
 
+class LaneConfig(C.Structure):
+    """lvo_lane_config: the per-sensor launch parameters of one lane."""
+    _fields_ = [("n_scans", C.c_int), ("minimum_range", C.c_double), ("line_res", C.c_double), ("plane_res", C.c_double), ("skip_frame", C.c_int)]
+
+
 class Stats(C.Structure):
     _fields_ = [("n_in", C.c_int), ("n_kept", C.c_int), ("n_sharp", C.c_int), ("n_less_sharp", C.c_int), ("n_flat", C.c_int), ("n_less_flat", C.c_int),
                 ("odo_corner_corr", C.c_int * 16), ("odo_plane_corr", C.c_int * 16), ("odo_lm_iters", C.c_int * 16), ("odo_final_cost", C.c_double * 16),
@@ -89,7 +94,7 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
            "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
            "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load", "lvo_depth_associate_batch", "lvo_depth_associate_batch_dev",
-           "lvo_map_cloud_batch", "lvo_map_cloud_batch_dev"]
+           "lvo_map_cloud_batch", "lvo_map_cloud_batch_dev", "lvo_lane_configure", "lvo_lane_get_config"]
 
 
 def load_library():
@@ -116,6 +121,8 @@ def load_library():
     L.lvo_wait.argtypes = [vp, C.POINTER(Pose), C.POINTER(Pose)]
     L.lvo_set_lane_active.argtypes = [vp, ip, ip]
     L.lvo_lane_reset.argtypes = [vp, ip]
+    L.lvo_lane_configure.argtypes = [vp, ip, C.POINTER(LaneConfig)]
+    L.lvo_lane_get_config.argtypes = [vp, ip, C.POINTER(LaneConfig)]
     L.lvo_lane_save.argtypes = [vp, ip, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     L.lvo_lane_load.argtypes = [vp, ip, vp, C.c_size_t]
     L.lvo_map_import.argtypes = [vp, ip, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
@@ -333,6 +340,23 @@ class Lvo:
     def lane_reset(self, lane):
         """Return `lane` to the first-frame state of a new context (empty map, identity poses, skip_frame phase 0)."""
         self._check(self.lib.lvo_lane_reset(self.h, lane))
+
+    LANE_FIELDS = ("n_scans", "minimum_range", "line_res", "plane_res", "skip_frame")
+
+    def lane_configure(self, lane, n_scans=None, minimum_range=None, line_res=None, plane_res=None, skip_frame=None):
+        """Start a new sequence in `lane` with these sensor settings (lvo_lane_configure); None means the context's value."""
+        given = dict(n_scans=n_scans, minimum_range=minimum_range, line_res=line_res, plane_res=plane_res, skip_frame=skip_frame)
+        if all(v is None for v in given.values()):
+            self._check(self.lib.lvo_lane_configure(self.h, lane, None))
+            return
+        cfg = LaneConfig(**{f: getattr(self.cfg, f) if v is None else v for f, v in given.items()})
+        self._check(self.lib.lvo_lane_configure(self.h, lane, C.byref(cfg)))
+
+    def lane_config(self, lane):
+        """The sensor settings of `lane` as a dict (lvo_lane_get_config)."""
+        cfg = LaneConfig()
+        self._check(self.lib.lvo_lane_get_config(self.h, lane, C.byref(cfg)))
+        return {f: getattr(cfg, f) for f in self.LANE_FIELDS}
 
     def lane_save(self, lane):
         """Snapshot of `lane` (lvo_lane_save) as a uint8 array: write it to disk, or lane_load it into any lane of a context with the

@@ -31,8 +31,8 @@ struct ExtractArgs {
   const int* in_n;                     // [lanes] (0 for an idle lane)
   const int* lane_flags;               // [lanes] LVO_LANE_* of the step: the kernels below leave an idle lane's state alone
   int in_stride, in_off_xyz;
-  int n_scans;
-  float thres;                         // (float)MINIMUM_RANGE
+  const LaneConfig* lcfg;              // [lanes] n_scans and (float)MINIMUM_RANGE of each lane
+  int max_scans;                       // lvo_config::n_scans: sizes the per-ring grids only; rings at or above a lane's n_scans are empty
   int P;                               // capacity per lane
   int nblk_cap;                        // ceil(P / LVO_EX_THREADS)
   LaneState* ls;
@@ -93,15 +93,16 @@ __global__ void k_extract_reset(ExtractArgs a) {
 __global__ void __launch_bounds__(LVO_EX_THREADS) k_classify(ExtractArgs a) {
   const int lane = blockIdx.y;
   const int n = a.in_n[lane];
+  const LaneConfig lc = a.lcfg[lane];
   const int i = blockIdx.x * LVO_EX_THREADS + threadIdx.x;
   bool kept = false;
   if (i < n) {
     float3 p = load_xyz(a.in_ptr[lane], a.in_stride, a.in_off_xyz, i);
-    kept = isfinite(p.x) && isfinite(p.y) && isfinite(p.z) && !(p.x * p.x + p.y * p.y + p.z * p.z < a.thres * a.thres);
+    kept = isfinite(p.x) && isfinite(p.y) && isfinite(p.z) && !(p.x * p.x + p.y * p.y + p.z * p.z < lc.thres * lc.thres);
     int ring = -2;
     float ori = 0.f;
     if (kept) {
-      ring = ring_of_dev(p.x, p.y, p.z, a.n_scans);
+      ring = ring_of_dev(p.x, p.y, p.z, lc.n_scans);
       ori = -lvo_atan2f(p.y, p.x);
     }
     a.ring[(size_t)lane * a.P + i] = (signed char)ring;
@@ -180,12 +181,13 @@ __global__ void k_ring_offsets(ExtractArgs a) {
   s.ring_count[r] = run;
   __syncthreads();
   if (r == 0) {
+    const int ns = a.lcfg[lane].n_scans;
     int acc = 0;
     for (int k = 0; k < LVO_MAX_RINGS; ++k) {
       s.ring_start[k] = acc;
-      if (k < a.n_scans) s.scan_start[k] = acc + 5;   // :249
+      if (k < ns) s.scan_start[k] = acc + 5;   // :249
       acc += s.ring_count[k];
-      if (k < a.n_scans) s.scan_end[k] = acc - 6;     // :251
+      if (k < ns) s.scan_end[k] = acc - 6;     // :251
     }
     s.ring_start[LVO_MAX_RINGS] = acc;
     s.n_kept = acc;
@@ -405,7 +407,10 @@ __global__ void __launch_bounds__(LVO_SECSORT_THREADS, 4) k_sector_sort(ExtractA
   const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int S = s.scan_start[ring], E = s.scan_end[ring];
-  if (!lane_active(a.lane_flags, lane)) return;
+  const int ns = a.lcfg[lane].n_scans;
+  // a ring at or above the lane's n_scans holds no point and the lane's steps never write its scan_start / scan_end: no kernel of the
+  // ring runs (k_sector_pick_warp, k_lessflat_voxel and k_sector_pick return for it too)
+  if (!lane_active(a.lane_flags, lane) || ring >= ns) return;
   if (threadIdx.x == 0) a.lf_cnt[lane * LVO_MAX_RINGS + ring] = 0;
   if (threadIdx.x < LVO_SECTORS * 3) a.slot_cnt[sbase * 3 + threadIdx.x] = 0;
   const int RL = (E + 6) - (S - 5) + 1;          // the ring occupies [S - 5, E + 6]
@@ -450,11 +455,10 @@ __global__ void __launch_bounds__(LVO_PICKW_THREADS) k_sector_pick_warp(ExtractA
   const int lane = blockIdx.y;
   const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int ring = blockIdx.x * (LVO_PICKW_THREADS / 32) + (int)w;
-  if (ring >= a.n_scans) return;
   const LaneState& s = a.ls[lane];
-  const int S = s.scan_start[ring], E = s.scan_end[ring];
+  const int S = s.scan_start[ring], E = s.scan_end[ring];   // ring < LVO_MAX_RINGS: the grid covers at most the context's n_scans
   const bool active = lane_active(a.lane_flags, lane);
-  if (!active || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
+  if (!active || ring >= a.lcfg[lane].n_scans || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
   const size_t lo = (size_t)lane * a.P;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int R0 = S - 5, RL = (E + 6) - R0 + 1;
@@ -563,7 +567,8 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 5 : 3) k_lessflat_voxel(Extrac
   const LaneState& s = a.ls[lane];
   const int S = s.scan_start[ring], E = s.scan_end[ring];
   const bool active = lane_active(a.lane_flags, lane);
-  if (!active || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
+  const int ns = a.lcfg[lane].n_scans;
+  if (!active || ring >= ns || E - S < 6 || !a.ring_done[lane * LVO_MAX_RINGS + ring]) return;
   if (NT == 256 && E - S <= 2048) return;       // candidates come from [S, E - 1]: at most 2048 of them, the other instantiation's ring
   const size_t lo = (size_t)lane * a.P;
   const float4* P = a.full + lo;
@@ -717,7 +722,8 @@ __global__ void __launch_bounds__(LVO_PICK_THREADS) k_sector_pick(ExtractArgs a)
   const unsigned ln = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int sbase = (lane * LVO_MAX_RINGS + ring) * LVO_SECTORS;
   const int S = s.scan_start[ring], E = s.scan_end[ring];
-  if (!active || a.ring_done[lane * LVO_MAX_RINGS + ring]) return;   // idle lane / handled by k_sector_pick_fast
+  const int ns = a.lcfg[lane].n_scans;
+  if (!active || ring >= ns || a.ring_done[lane * LVO_MAX_RINGS + ring]) return;   // idle lane / empty ring / handled by k_sector_pick_fast
   if (threadIdx.x == 0) a.lf_cnt[lane * LVO_MAX_RINGS + ring] = 0;
   if (threadIdx.x < LVO_SECTORS * 3) a.slot_cnt[sbase * 3 + threadIdx.x] = 0;
   if (E - S < 6) return;  // :279-280
@@ -929,7 +935,8 @@ __global__ void __launch_bounds__(512) k_feature_compact(ExtractArgs a) {
   __shared__ int lfo[LVO_MAX_RINGS + 1];
   const int lane = blockIdx.x;
   LaneState& s = a.ls[lane];
-  const int nsec = a.n_scans * LVO_SECTORS;
+  const int ns = a.lcfg[lane].n_scans;
+  const int nsec = ns * LVO_SECTORS;
   const int k = threadIdx.x;
   const int r = k / LVO_SECTORS, j = k % LVO_SECTORS;
   const size_t sb = (size_t)(lane * LVO_MAX_RINGS + r) * LVO_SECTORS;
@@ -940,11 +947,11 @@ __global__ void __launch_bounds__(512) k_feature_compact(ExtractArgs a) {
   const unsigned o0 = block_excl_scan((unsigned)c0, sm, &t0);
   const unsigned o1 = block_excl_scan((unsigned)c1, sm, &t1);
   const unsigned o2 = block_excl_scan((unsigned)c2, sm, &t2);
-  const int lc = k < a.n_scans ? a.lf_cnt[lane * LVO_MAX_RINGS + k] : 0;
+  const int lc = k < ns ? a.lf_cnt[lane * LVO_MAX_RINGS + k] : 0;
   const unsigned ol = block_excl_scan((unsigned)lc, sm, &tl);
-  if (k < a.n_scans) { lfo[k] = (int)ol; s.lf_ring_off[k] = (int)ol; }
+  if (k < ns) { lfo[k] = (int)ol; s.lf_ring_off[k] = (int)ol; }
   if (k == 0) {
-    lfo[a.n_scans] = (int)tl; s.lf_ring_off[a.n_scans] = (int)tl;
+    lfo[ns] = (int)tl; s.lf_ring_off[ns] = (int)tl;
     s.n_sharp = (int)t0; s.n_less_sharp = (int)t1; s.n_flat = (int)t2; s.n_less_flat = (int)tl;
     s.stats.n_sharp = (int)t0; s.stats.n_less_sharp = (int)t1; s.stats.n_flat = (int)t2; s.stats.n_less_flat = (int)tl;
   }
@@ -957,7 +964,7 @@ __global__ void __launch_bounds__(512) k_feature_compact(ExtractArgs a) {
   }
   // less-flat: warp w copies rings w, w + 16, ...
   const int w = threadIdx.x >> 5, ln = threadIdx.x & 31;
-  for (int rr = w; rr < a.n_scans; rr += 16) {
+  for (int rr = w; rr < ns; rr += 16) {
     const int c = lfo[rr + 1] - lfo[rr];
     const float4* src = a.lf_ring + (size_t)lane * a.P + s.ring_start[rr];
     for (int t = ln; t < c; t += 32) a.less_flat[(size_t)lane * a.P + lfo[rr] + t] = src[t];
@@ -981,12 +988,12 @@ static inline void lvo_launch_extract(cudaStream_t st, const ExtractArgs& a, int
   k_ring_scatter<<<gpts, LVO_EX_THREADS, 0, st>>>(a);
   k_curvature<<<gpts, LVO_EX_THREADS, 0, st>>>(a);
   LVO_MARK(tm, LVO_ST_REG_SORT, st);
-  k_sector_sort<<<dim3(a.n_scans, lanes), LVO_SECSORT_THREADS, 0, st>>>(a);
+  k_sector_sort<<<dim3(a.max_scans, lanes), LVO_SECSORT_THREADS, 0, st>>>(a);
   LVO_MARK(tm, LVO_ST_REG_SEPARATE, st);
-  k_sector_pick_warp<<<dim3(lvo_div_up(a.n_scans, LVO_PICKW_THREADS / 32), lanes), LVO_PICKW_THREADS, 0, st>>>(a);
-  k_lessflat_voxel<128><<<dim3(a.n_scans, lanes), 128, LVO_LFV_SMEM(128), st>>>(a);
-  k_lessflat_voxel<256><<<dim3(a.n_scans, lanes), 256, LVO_LFV_SMEM(256), st>>>(a);
-  k_sector_pick<<<dim3(a.n_scans, lanes), LVO_PICK_THREADS, LVO_PICK_SMEM_KEYS * sizeof(unsigned long long), st>>>(a);
+  k_sector_pick_warp<<<dim3(lvo_div_up(a.max_scans, LVO_PICKW_THREADS / 32), lanes), LVO_PICKW_THREADS, 0, st>>>(a);
+  k_lessflat_voxel<128><<<dim3(a.max_scans, lanes), 128, LVO_LFV_SMEM(128), st>>>(a);
+  k_lessflat_voxel<256><<<dim3(a.max_scans, lanes), 256, LVO_LFV_SMEM(256), st>>>(a);
+  k_sector_pick<<<dim3(a.max_scans, lanes), LVO_PICK_THREADS, LVO_PICK_SMEM_KEYS * sizeof(unsigned long long), st>>>(a);
   k_feature_compact<<<lanes, 512, 0, st>>>(a);
   if (launches) *launches += 12;
 }

@@ -87,6 +87,14 @@ struct LaneState {
   int status;
 };
 
+// The sensor settings of one lane (lvo_lane_configure; lvo_create gives every lane the context's), one record per lane in device
+// memory.  Not part of LaneState: a lane snapshot saves that struct verbatim, and its bytes must not change.
+struct LaneConfig {
+  int n_scans;   // 16 | 32 | 64, <= lvo_config::n_scans
+  float thres;   // (float)minimum_range
+  float leaf[2]; // (float)line_res, (float)plane_res (setLeafSize takes floats)
+};
+
 // Per-lane flags of a batched step, [lanes] ints uploaded right after the sweep counts (set_inputs in lvo_api.cu).  A lane without
 // LVO_LANE_ACTIVE is idle (lvo_set_lane_active): every per-lane kernel leaves its state alone.  LVO_LANE_MAPS: the lane runs the
 // mapping stage in this step (active and on its own skip_frame phase); the other lanes keep their map, poses and map correction.

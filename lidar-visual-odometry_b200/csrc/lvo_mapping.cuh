@@ -34,7 +34,7 @@ struct MapArgs {
   LaneState* ls;
   int lanes, outer, from_odo;
   const int* lane_flags;             // [lanes] LVO_LANE_* of the step: a lane without LVO_LANE_MAPS keeps its map, poses and counters
-  float leaf[2];                     // lineRes, planeRes as float (setLeafSize takes floats)
+  const LaneConfig* lcfg;            // [lanes] leaf[0], leaf[1]: each lane's lineRes, planeRes as float (setLeafSize takes floats)
   // inputs: corner_last / surf_last / full-res of this frame
   const float4* in_pts[2]; int in_cap[2];   // less_sharp [cap_lsharp], less_flat [P]; counts n_less_sharp / n_less_flat
   const float4* full; int P;
@@ -145,7 +145,7 @@ __global__ void __launch_bounds__(256) k_stack_offsets(MapArgs a) {
     if (lt < L2) {
       const LaneState& s = a.ls[lt >> 1];
       if (lane_maps(a.lane_flags, lt >> 1)) v = (unsigned)((lt & 1) ? s.n_less_flat : s.n_less_sharp);
-      a.vx.seg_leaf[lt] = a.leaf[lt & 1];
+      a.vx.seg_leaf[lt] = a.lcfg[lt >> 1].leaf[lt & 1];
     }
     unsigned tot;
     const unsigned ex = block_excl_scan(v, sm, &tot);
@@ -631,7 +631,19 @@ __global__ void k_map_finish(MapArgs a) {
 __global__ void __launch_bounds__(256) k_refilter_offsets(MapArgs a) {
   __shared__ unsigned sm[33];
   const int L2 = 2 * a.lanes;
-  for (int k = threadIdx.x; k < L2 * LVO_MSEGS; k += blockDim.x) a.vx.seg_leaf[k] = (k % LVO_MSEGS) < LVO_MAX_VALID ? a.leaf[(k / LVO_MSEGS) & 1] : 0.f;
+  // one (lane, type) row of segments per warp: the lane's leaf for its valid cubes, 0 (pseudo segment) for the rest.  Each lane of the
+  // warp loads the leaf of one of the warp's next 32 rows, so that the rows wait for one load, not for one each.
+  const int nw = blockDim.x >> 5, ln = threadIdx.x & 31;
+  for (int r0 = threadIdx.x >> 5; r0 < L2; r0 += 32 * nw) {
+    const int mine = r0 + ln * nw;
+    const float my_leaf = mine < L2 ? a.lcfg[mine >> 1].leaf[mine & 1] : 0.f;
+    for (int j = 0; j < 32; ++j) {
+      const float leaf = __shfl_sync(0xffffffffu, my_leaf, j);
+      const int lt = r0 + j * nw;
+      if (lt >= L2) break;   // the same for the whole warp
+      for (int k = ln; k < LVO_MSEGS; k += 32) a.vx.seg_leaf[lt * LVO_MSEGS + k] = k < LVO_MAX_VALID ? leaf : 0.f;
+    }
+  }
   unsigned acc = 0;
   for (int base = 0; base < L2; base += blockDim.x) {
     const int lt = base + threadIdx.x;
