@@ -184,6 +184,25 @@ int lvo_lane_status(const lvo_ctx* ctx, int lane);
  * (profiles/lane_lifecycle.md); the cost of an idle lane by itself is not measured.
  * LVO_E_STATE while an *_async step is in flight, LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid. */
 int lvo_set_lane_active(lvo_ctx* ctx, int lane, int active);
+/* Map updates of `lane` (default: on).  update != 0: every mapping frame inserts the frame's stack into the cubes and re-filters the
+ * valid cubes (laserMapping.cpp:737-801), as the reference does.  update == 0, localisation in a fixed prior map: the lane runs
+ * process() (:307-848) with the insertion (:737-783) and the per-cube re-filter (:788-801) skipped; everything else runs unchanged:
+ * transformAssociateToMap, the cube-window shift (:312-507), the valid list, the FromMap gather, the stack downsample, the 5-NN
+ * search and the fits, the LM solve over every outer iteration, transformUpdate (the map correction keeps being refined) and the
+ * registered cloud.  The reference has no such mode.  Consequences:
+ *   - The map does not change while updates are off, except by the cube-window shift: cubes that leave the 21 x 21 x 11 window are
+ *     dropped, as always, so a fixed map is bounded by the window (about 1050 x 1050 x 550 m around where it sits).
+ *     lvo_stats::map_corner_total / map_surf_total report the stored map after any such drop.
+ *   - An empty or too-small map gives LVO_W_MAP_TOO_SMALL on every mapping frame, with the initial guess as the pose.
+ *   - A lane with updates off never returns LVO_E_CAPACITY from the map.
+ *   - skip_frame, the high-frequency pose of non-mapping frames, statuses, probes and lvo_map_cloud[_batch] behave as for a lane
+ *     with updates on.
+ * Takes effect from the next call that runs the mapping stage (the lvo_step_batch* calls, and lvo_scan_to_map for lane 0) and may
+ * change between any two steps.  It is host state, like activity: not part of lvo_config, lvo_lane_config or a snapshot (the bytes
+ * of lvo_lane_save do not depend on it), and lvo_lane_reset, lvo_lane_configure, lvo_lane_load and lvo_set_lane_active leave it as
+ * it is.  LVO_E_STATE while an *_async step is in flight, LVO_E_BADARG for a bad lane.  Captured CUDA graphs stay valid, and a step
+ * launches the same kernels whatever the lanes' settings.  INTEGRATION.md, "Localisation in a prior map", gives the recipe. */
+int lvo_set_lane_map_update(lvo_ctx* ctx, int lane, int update);
 /* Return `lane` to the state of a freshly created context: next active step is its first frame (LVO_W_FIRST_FRAME), empty map,
  * identity poses and map correction, cen = (10, 10, 5), zero lvo_stats, status LVO_OK, skip_frame phase 0.  Other lanes are
  * untouched, and so are the lane's activity and its settings (lvo_lane_configure).  Stream-ordered (returns when done); LVO_E_STATE while an *_async step is in flight,

@@ -94,7 +94,7 @@ EXPORTS = ["lvo_default_config", "lvo_create", "lvo_destroy", "lvo_last_error", 
            "lvo_knn5_throughput", "lvo_get_timings", "lvo_set_stream", "lvo_state_bytes", "lvo_depth_associate", "lvo_step_batch_pipelined", "lvo_set_option", "lvo_voxel_downsample_dev",
            "lvo_map_cloud", "lvo_transform_cloud", "lvo_step_batch_async", "lvo_step_batch_dev_async", "lvo_wait", "lvo_set_lane_active",
            "lvo_lane_reset", "lvo_lane_save", "lvo_lane_load", "lvo_depth_associate_batch", "lvo_depth_associate_batch_dev",
-           "lvo_map_cloud_batch", "lvo_map_cloud_batch_dev", "lvo_lane_configure", "lvo_lane_get_config"]
+           "lvo_map_cloud_batch", "lvo_map_cloud_batch_dev", "lvo_lane_configure", "lvo_lane_get_config", "lvo_set_lane_map_update"]
 
 
 def load_library():
@@ -120,6 +120,7 @@ def load_library():
     L.lvo_step_batch_dev_async.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.lvo_wait.argtypes = [vp, C.POINTER(Pose), C.POINTER(Pose)]
     L.lvo_set_lane_active.argtypes = [vp, ip, ip]
+    L.lvo_set_lane_map_update.argtypes = [vp, ip, ip]
     L.lvo_lane_reset.argtypes = [vp, ip]
     L.lvo_lane_configure.argtypes = [vp, ip, C.POINTER(LaneConfig)]
     L.lvo_lane_get_config.argtypes = [vp, ip, C.POINTER(LaneConfig)]
@@ -336,6 +337,11 @@ class Lvo:
         """An idle lane is skipped by every step (its sweep may be None) and resumes its sequence bit for bit."""
         self._check(self.lib.lvo_set_lane_active(self.h, lane, int(bool(active))))
         self._active[lane] = bool(active)
+
+    def set_lane_map_update(self, lane, update):
+        """update=False: the lane localises in its map (insertion and re-filter skipped, only the cube-window shift changes it);
+        True (the default) maps as the reference does.  Takes effect from the next mapping frame."""
+        self._check(self.lib.lvo_set_lane_map_update(self.h, lane, int(bool(update))))
 
     def lane_reset(self, lane):
         """Return `lane` to the first-frame state of a new context (empty map, identity poses, skip_frame phase 0)."""

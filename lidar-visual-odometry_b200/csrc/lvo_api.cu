@@ -63,6 +63,7 @@ struct lvo_ctx {
   std::vector<lvo_lane_config> lane_cfg;
   LaneConfig* d_lcfg = nullptr; LaneConfig* h_lcfg = nullptr;
   std::vector<char> lane_active;      // lvo_set_lane_active
+  std::vector<char> lane_map_update;  // lvo_set_lane_map_update (host state like activity: not in LaneState or a snapshot)
   std::vector<char> prefetched_active;  // the active set the prefetched sweeps were staged for
   std::vector<int> lane_status;
   // lvo_lane_load: a loaded lane's probe arrays belong to this context's earlier frames, its counts to the snapshot; LVO_PROBE_GATE_*
@@ -296,9 +297,9 @@ int set_inputs(lvo_ctx* c) {
   return LVO_OK;
 }
 // lvo_extract_features / lvo_scan_to_scan / lvo_scan_to_map enqueue the batched kernels for every lane: all lanes active and mapping,
-// whatever the last batched step left in the flags.  upload = false: set_inputs follows.
+// whatever the last batched step left in the flags, each with its own map-update setting.  upload = false: set_inputs follows.
 int flags_all_lanes(lvo_ctx* c, bool upload) {
-  for (int l = 0; l < c->lanes; ++l) lane_flags(c)[l] = LVO_LANE_ACTIVE | LVO_LANE_MAPS;
+  for (int l = 0; l < c->lanes; ++l) lane_flags(c)[l] = LVO_LANE_ACTIVE | LVO_LANE_MAPS | (c->lane_map_update[l] ? 0 : LVO_LANE_MAP_FIXED);
   if (upload) LVO_CUDA_OK(c, cudaMemcpyAsync(c->d_in_n + c->lanes, lane_flags(c), sizeof(int) * c->lanes, cudaMemcpyHostToDevice, c->st));
   return LVO_OK;
 }
@@ -458,6 +459,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   c->lane_status.assign(L, 0);
   c->lane_frame.assign(L, 0);
   c->lane_active.assign(L, 1);
+  c->lane_map_update.assign(L, 1);
   c->probe_gate.assign(L, 0);
   c->reg_n.assign(L, 0);
   c->lane_cfg.assign(L, lvo_lane_config{c->cfg.n_scans, c->cfg.minimum_range, c->cfg.line_res, c->cfg.plane_res, c->cfg.skip_frame});
@@ -788,7 +790,7 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
   bool do_map = false;
   for (int l = 0; l < c->lanes; ++l) {
     const bool maps = c->lane_active[l] && (c->lane_frame[l] % c->lane_cfg[l].skip_frame) == 0;
-    lane_flags(c)[l] = (c->lane_active[l] ? LVO_LANE_ACTIVE : 0) | (maps ? LVO_LANE_MAPS : 0);
+    lane_flags(c)[l] = (c->lane_active[l] ? LVO_LANE_ACTIVE : 0) | (maps ? LVO_LANE_MAPS : 0) | (maps && !c->lane_map_update[l] ? LVO_LANE_MAP_FIXED : 0);
     do_map = do_map || maps;
   }
   LVO_TRY(set_inputs(c));
@@ -991,6 +993,13 @@ int lvo_set_lane_active(lvo_ctx* c, int lane, int active) {
   if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
   if (lane < 0 || lane >= c->lanes) { lvo_set_error(c, "lane out of range"); return LVO_E_BADARG; }
   c->lane_active[lane] = active ? 1 : 0;
+  return LVO_OK;
+}
+int lvo_set_lane_map_update(lvo_ctx* c, int lane, int update) {
+  if (!c) return LVO_E_BADARG;
+  if (c->pending) { lvo_set_error(c, "lvo_wait has not been called for the last *_async step"); return LVO_E_STATE; }
+  if (lane < 0 || lane >= c->lanes) { lvo_set_error(c, "lane out of range"); return LVO_E_BADARG; }
+  c->lane_map_update[lane] = update ? 1 : 0;
   return LVO_OK;
 }
 

@@ -98,8 +98,11 @@ struct LaneConfig {
 // Per-lane flags of a batched step, [lanes] ints uploaded right after the sweep counts (set_inputs in lvo_api.cu).  A lane without
 // LVO_LANE_ACTIVE is idle (lvo_set_lane_active): every per-lane kernel leaves its state alone.  LVO_LANE_MAPS: the lane runs the
 // mapping stage in this step (active and on its own skip_frame phase); the other lanes keep their map, poses and map correction.
+// LVO_LANE_MAP_FIXED (set together with LVO_LANE_MAPS, lvo_set_lane_map_update): the lane registers against its map but inserts
+// nothing and re-filters no cube; only the cube-window shift of this step changes its map.
 #define LVO_LANE_ACTIVE 1
 #define LVO_LANE_MAPS 2
+#define LVO_LANE_MAP_FIXED 4
 
 // Launch accounting (bench.py's gpu_launches) and error capture.
 struct LvoLaunchCounter { long long launches; };
@@ -170,9 +173,13 @@ static inline int lvo_div_up(long long a, long long b) { return (int)((a + b - 1
 // ------------------------------------------------------------------------------------------------------------
 #ifdef __CUDACC__
 
-// the two lane predicates of a batched step (flags: ExtractArgs / OdoArgs / MapArgs::lane_flags)
+// the lane predicates of a batched step (flags: ExtractArgs / OdoArgs / MapArgs::lane_flags)
 __device__ __forceinline__ bool lane_active(const int* flags, int lane) { return (__ldg(flags + lane) & LVO_LANE_ACTIVE) != 0; }
 __device__ __forceinline__ bool lane_maps(const int* flags, int lane) { return (__ldg(flags + lane) & LVO_LANE_MAPS) != 0; }
+// maps in this step and inserts into its map (lvo_set_lane_map_update on): the lanes that take part in the insertion + re-filter
+__device__ __forceinline__ bool lane_updates_map(const int* flags, int lane) {
+  return (__ldg(flags + lane) & (LVO_LANE_MAPS | LVO_LANE_MAP_FIXED)) == LVO_LANE_MAPS;
+}
 
 struct d3 { double x, y, z; };
 __device__ __forceinline__ d3 d3cross(const d3& a, const d3& b) { return d3{a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x}; }

@@ -17,7 +17,7 @@
 //   k_lm_solve         ceres::Solve :712-720
 //   k_map_finish       transformUpdate :148-152
 //   refilter           insert the transformed stack points into their cubes :737-783 and VoxelGrid every valid cube
-//                      :788-801: one lvo_voxel_run over 77 segments per lane and type
+//                      :788-801: one lvo_voxel_run over 77 segments per lane and type (none for a lane with a fixed map)
 //   k_rebuild_*        new cube offset table + gather into the other map generation
 //   k_register         registered full-resolution cloud :838-842
 #pragma once
@@ -33,7 +33,8 @@
 struct MapArgs {
   LaneState* ls;
   int lanes, outer, from_odo;
-  const int* lane_flags;             // [lanes] LVO_LANE_* of the step: a lane without LVO_LANE_MAPS keeps its map, poses and counters
+  const int* lane_flags;             // [lanes] LVO_LANE_* of the step: a lane without LVO_LANE_MAPS keeps its map, poses and counters;
+                                     // one with LVO_LANE_MAP_FIXED maps but skips the insertion + re-filter
   const LaneConfig* lcfg;            // [lanes] leaf[0], leaf[1]: each lane's lineRes, planeRes as float (setLeafSize takes floats)
   // inputs: corner_last / surf_last / full-res of this frame
   const float4* in_pts[2]; int in_cap[2];   // less_sharp [cap_lsharp], less_flat [P]; counts n_less_sharp / n_less_flat
@@ -648,7 +649,7 @@ __global__ void __launch_bounds__(256) k_refilter_offsets(MapArgs a) {
   for (int base = 0; base < L2; base += blockDim.x) {
     const int lt = base + threadIdx.x;
     unsigned v = 0;
-    if (lt < L2 && lane_maps(a.lane_flags, lt >> 1)) { const LaneState& s = a.ls[lt >> 1]; v = (unsigned)(s.from_off[lt & 1][LVO_MAX_VALID] + s.n_stack[lt & 1]); }
+    if (lt < L2 && lane_updates_map(a.lane_flags, lt >> 1)) { const LaneState& s = a.ls[lt >> 1]; v = (unsigned)(s.from_off[lt & 1][LVO_MAX_VALID] + s.n_stack[lt & 1]); }
     unsigned tot;
     const unsigned ex = block_excl_scan(v, sm, &tot);
     if (lt < L2) a.item_off[lt] = acc + ex;
@@ -660,7 +661,7 @@ __global__ void k_refilter_gather(MapArgs a) {
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
   const int nfrom = s.from_off[t][LVO_MAX_VALID], nst = s.n_stack[t];
-  if (!lane_maps(a.lane_flags, lane)) return;
+  if (!lane_updates_map(a.lane_flags, lane)) return;
   const unsigned off = a.item_off[lt];
   const float4* FM = a.from_map[t] + (size_t)lane * a.map_cap[t];
   const float4* ST = a.stack[t] + (size_t)lane * a.in_cap[t];
@@ -704,15 +705,17 @@ __global__ void k_rebuild_appended(MapArgs a) {
 }
 // one block per (lane, type): new per-cube counts and their exclusive scan.  A lane that does not map in this step counts as having
 // no valid cube (its n_valid / valid_cube stay for lvo_map_cloud) and no shift (k_map_end left it 0): its map passes through unchanged.
+// A lane with a fixed map (LVO_LANE_MAP_FIXED) also counts as having no valid cube, but with the shift k_map_begin computed in this
+// step: its map passes through shifted, cubes that left the window dropped, and its n_map / totals are written.
 __global__ void __launch_bounds__(256) k_rebuild_offsets(MapArgs a) {
   __shared__ unsigned sm[33];
   __shared__ signed char vrank[LVO_NCUBES];
   const int lt = blockIdx.x, lane = lt >> 1, t = lt & 1;
   LaneState& s = a.ls[lane];
-  const bool maps = lane_maps(a.lane_flags, lane);
+  const bool maps = lane_maps(a.lane_flags, lane), updates = lane_updates_map(a.lane_flags, lane);
   for (int c = threadIdx.x; c < LVO_NCUBES; c += blockDim.x) vrank[c] = -1;
   __syncthreads();
-  if (maps && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
+  if (updates && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
   __syncthreads();
   const unsigned* cs = a.cube_start[a.gen][t] + (size_t)lane * (LVO_NCUBES + 1);
   unsigned* ncs = a.cube_start[a.gen ^ 1][t] + (size_t)lane * (LVO_NCUBES + 1);
@@ -750,10 +753,10 @@ __global__ void __launch_bounds__(256) k_rebuild_copy(MapArgs a) {
   __shared__ signed char vrank[LVO_NCUBES];
   const int lt = blockIdx.y, lane = lt >> 1, t = lt & 1;
   const LaneState& s = a.ls[lane];
-  const bool maps = lane_maps(a.lane_flags, lane);   // see k_rebuild_offsets
+  const bool updates = lane_updates_map(a.lane_flags, lane);   // see k_rebuild_offsets
   for (int c = threadIdx.x; c < LVO_NCUBES; c += blockDim.x) vrank[c] = -1;
   __syncthreads();
-  if (maps && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
+  if (updates && threadIdx.x < s.n_valid) vrank[s.valid_cube[threadIdx.x]] = (signed char)threadIdx.x;
   __syncthreads();
   const unsigned* cs = a.cube_start[a.gen][t] + (size_t)lane * (LVO_NCUBES + 1);
   const unsigned* ncs = a.cube_start[a.gen ^ 1][t] + (size_t)lane * (LVO_NCUBES + 1);

@@ -161,6 +161,9 @@ class LaserMapping {
   void laserCloudSurround(Cloud& out) { fetch(0, out); }   // :806-815
   template <class Cloud>
   void laserCloudMap(Cloud& out) { fetch(1, out); }        // :823-836
+  // Localisation in a fixed prior map (lvo_set_lane_map_update): false skips the insertion and re-filter of :737-801 on the
+  // following frames, so an imported map is registered against but not changed; true (the default) maps as the reference does.
+  void setMapUpdate(bool update) { c_.check(lvo_set_lane_map_update(c_.get(), 0, update ? 1 : 0)); }
 
  private:
   template <class Cloud>
