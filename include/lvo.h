@@ -160,7 +160,7 @@ int lvo_step_batch_pipelined(lvo_ctx* ctx, const lvo_cloud_view* sweeps, const l
  * processes overlap): lvo_step_batch_async copies and enqueues one frame for every lane and returns without waiting for the GPU;
  * lvo_wait blocks until that frame is done and delivers its poses / statuses (same return value as lvo_step_batch).  The sweep
  * buffers must stay valid and unchanged until lvo_wait returns; exactly one step may be in flight per context; every other entry
- * point returns LVO_E_STATE while one is.  Lanes whose host buffers are adjacent in memory (one slab) are uploaded in one copy. */
+ * point but lvo_destroy and lvo_last_error returns LVO_E_STATE while one is, and writes none of its outputs.  Lanes whose host buffers are adjacent in memory (one slab) are uploaded in one copy. */
 int lvo_step_batch_async(lvo_ctx* ctx, const lvo_cloud_view* sweeps);
 int lvo_step_batch_dev_async(lvo_ctx* ctx, const lvo_point* const* d_sweeps, const size_t* n);
 int lvo_wait(lvo_ctx* ctx, lvo_pose* T_wodom_curr, lvo_pose* T_wmap_curr);
@@ -294,9 +294,9 @@ int lvo_map_cloud(lvo_ctx* ctx, int lane, int which, lvo_cloud_out* pts);
  *   - LVO_MAP_REGISTERED reports the lanes that mapped in the last lvo_step_batch* call: each gets the n_kept points of that frame
  *     moved into the map frame, bit for bit what lvo_probe_fetch(LVO_P_REGISTERED) returns right after that step.  Every other lane
  *     gets n = 0 and its destination is not written: lanes that did not map (off their skip_frame phase or idle), and lanes reset or
- *     loaded since the step.  The counts are recorded on the host when the step completes.  lvo_scan_to_map, lvo_knn and
- *     lvo_depth_associate overwrite the registered clouds; after any of them which = 2 returns LVO_E_STATE (lvo_last_error says
- *     why) until the next lvo_step_batch* call completes.
+ *     loaded since the step.  The counts are recorded on the host when the step completes.  lvo_scan_to_map and lvo_knn
+ *     overwrite the registered clouds; after either of them which = 2 returns LVO_E_STATE (lvo_last_error says why) until the
+ *     next lvo_step_batch* call completes.
  *   - Errors, each checked before any destination is written: LVO_E_BADARG for a NULL array or a bad `which`; LVO_E_STATE while an
  *     *_async step is in flight, or after the invalidation above; LVO_E_CAPACITY when a selected lane's cap is below its n (every n
  *     is still written, and no point is copied for any lane).
@@ -363,7 +363,10 @@ int lvo_knn(lvo_ctx* ctx, lvo_cloud_view cloud, lvo_cloud_view queries, int K, f
  * The sweep is moved into the camera frame by the 3x4 extrinsic, every point with z > 0 becomes a depth-cloud point
  * (10 x/z, 10 y/z, 10, intensity = z); each keypoint (normalised coordinates u = (px - cx)/fx, v = (py - cy)/fy) gets the
  * depth of the plane through its 3 nearest depth-cloud points when the nearest lies within d^2 < 0.5, with the reference's
- * clamps.  depth_out / valid_out are [n_kp]; nn_out (optional) is [n_kp][3] indices into the depth cloud (-1 if rejected). */
+ * clamps.  depth_out / valid_out are [n_kp]; nn_out (optional) is [n_kp][3] indices into the depth cloud (-1 if rejected).
+ * Runs as one slot of lvo_depth_associate_batch, in the arena of those calls (reserved on first use for max_points points of the
+ * view's stride and max_points / 2 keypoints), and reads and writes no state of the step: probes, maps and the registered clouds
+ * of lvo_map_cloud_batch are left as they were. */
 typedef struct lvo_camera { float fx, fy, cx, cy; int width, height; float extrinsic[12]; /* row-major 3x4 lidar -> camera */ } lvo_camera;
 int lvo_depth_associate(lvo_ctx* ctx, lvo_cloud_view sweep, const lvo_camera* cam, const float* keypoints_uv, size_t n_kp, float* depth_out,
                         int* valid_out, int* nn_out, lvo_cloud_out* depth_cloud_or_null);

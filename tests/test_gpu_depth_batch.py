@@ -235,7 +235,7 @@ def probes(lvo, lane):
 def test_no_effect_on_pipeline(lvo_mod, synth, skip, graphs):
     import torch
     L = lvo_mod
-    ctx = [small_ctx(L, 2, skip_frame=skip) for _ in range(2)]   # ctx[0] runs depth calls between its steps, ctx[1] does not
+    ctx = [small_ctx(L, 2, skip_frame=skip) for _ in range(2)]   # ctx[0] runs all three depth calls between its steps, ctx[1] none
     for c in ctx:
         c.set_option(L.LVO_OPT_GRAPHS, graphs)
     frames = [[synth.sweep(64, lane, f)[0] for lane in range(2)] for f in range(13)]
@@ -260,6 +260,7 @@ def test_no_effect_on_pipeline(lvo_mod, synth, skip, graphs):
             launches = c.timings().kernel_launches
             if i == 0:
                 dev_call(c, frames[(f + 5) % 13], uv, cams)
+                c.depth_associate(frames[(f + 3) % 13][f % 2], uv[f % 2], camera=cams[f % 2])
             outs.append((r, launches, [c.lane_status(l) for l in range(2)], [bytes(c.stats(l)) for l in range(2)]))
         (r0, n0, s0, st0), (r1, n1, s1, st1) = outs
         assert r0[0] == r1[0] and np.array_equal(r0[1], r1[1]) and np.array_equal(r0[2], r1[2]), f"frame {f} poses"

@@ -188,7 +188,7 @@ def untouched(bufs):
     return all(b is None or (b == SENTINEL).all() for b in bufs)
 
 
-def test_errors_leave_buffers_untouched(lvo_mod, sweeps):
+def test_errors_leave_buffers_untouched_and_depth_keeps_registered(lvo_mod, sweeps):
     import torch
     L = lvo_mod
     lvo = make(L, 2)
@@ -236,14 +236,18 @@ def test_errors_leave_buffers_untouched(lvo_mod, sweeps):
         assert raw_dev(which, big[which]) == (L.LVO_E_STATE, [777, 777]) and dev_untouched()
     lvo.wait()
     check_outputs(L, lvo, [True, True])
-    # which 2 after the three calls that overwrite the registered clouds; the next step makes it valid again
+    # the single depth call runs in its own arena: the registered clouds stay available, bit for bit
     pts = sweeps(0, 3)
+    before = lvo.map_cloud_batch(2)
+    lvo.depth_associate(pts, np.zeros((4, 2), np.float32))
+    assert all(len(b) > 1000 and same(a, b) for a, b in zip(lvo.map_cloud_batch(2), before))
+    assert all(same(a, b) for a, b in zip(dev_call(lvo, 2), before))
+    # which 2 after the two calls that overwrite the registered clouds; the next step makes it valid again
     one = L.Lvo(lanes=1, **CAPS)
     ex = one.extract_features(pts)[1]
     one.close()
     overwriters = {
         "knn": lambda: lvo.knn(pts[:5000], pts[:100], 5, 1.0),
-        "depth": lambda: lvo.depth_associate(pts, np.zeros((4, 2), np.float32)),
         "scan_to_map": lambda: lvo.scan_to_map(ex["less_sharp"], ex["less_flat"], ex["full"], np.array([0, 0, 0, 1, 0, 0, 0.0]), want_registered=True),
     }
     for f, (name, call) in enumerate(overwriters.items()):
