@@ -73,9 +73,10 @@ __global__ void k_map_begin(MapArgs a) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
   if (lane >= a.lanes) return;
   LaneState& s = a.ls[lane];
-  // a lane that does not map in this step (idle, or off its skip_frame phase): k-NN, fit and solve return for it, the gather / stack /
-  // refilter / finish / register kernels see no items, and the rebuild carries its map into the other generation unchanged
-  if (!lane_maps(a.lane_flags, lane)) { s.map_done = 1; return; }
+  // a lane that does not map in this step (idle, or off its skip_frame phase): k-NN, fit and solve return for it by its lane flags, the
+  // gather / stack / refilter / finish / register kernels see no items, and the rebuild carries its map into the other generation
+  // unchanged.  Nothing of its state is written, so that its snapshot does not depend on what the other lanes of the context do.
+  if (!lane_maps(a.lane_flags, lane)) return;
   if (a.from_odo) { for (int k = 0; k < 4; ++k) s.q_wodom[k] = s.q_w[k]; for (int k = 0; k < 3; ++k) s.t_wodom[k] = s.t_w[k]; }
   // transformAssociateToMap
   quat_mul(s.q_wmap_wodom, s.q_wodom, s.map_x);
@@ -240,7 +241,7 @@ __device__ __forceinline__ void fit_factor(int t, const float4 ori, const float4
 __global__ void __launch_bounds__(128) k_map_knn(MapArgs a) {
   const int lane = blockIdx.y;
   const LaneState& s = a.ls[lane];
-  if (s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
+  if (!lane_maps(a.lane_flags, lane) || s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   const int n0 = s.n_stack[0], ntot = n0 + s.n_stack[1];
   const GridView g0 = grid_view(a.grid, 2 * lane), g1 = grid_view(a.grid, 2 * lane + 1);
   for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < ntot; f += gridDim.x * blockDim.x) {
@@ -379,7 +380,7 @@ __global__ void __launch_bounds__(128) k_map_knn_reuse(MapArgs a) {
   __shared__ int s_n, s_nfit, s_off;
   const int lane = blockIdx.y;
   const LaneState& s = a.ls[lane];
-  if (s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
+  if (!lane_maps(a.lane_flags, lane) || s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   const int n0 = s.n_stack[0], ntot = n0 + s.n_stack[1];
   int nc = 0, nsf = 0;   // factors kept from the previous iteration (unchanged rows)
   __shared__ GridView gv[2];   // shared, not registers: the certificate phase wants occupancy
@@ -542,7 +543,7 @@ __global__ void __launch_bounds__(128) k_map_knn_reuse(MapArgs a) {
 __global__ void __launch_bounds__(128) k_map_fit_reuse(MapArgs a) {
   const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
-  if (s.map_too_small || s.map_done) return;
+  if (!lane_maps(a.lane_flags, lane) || s.map_too_small || s.map_done) return;
   const int n0 = s.n_stack[0], ntot = n0 + s.n_stack[1];
   const int n = a.outer > 0 ? a.fit_cnt[lane * LVO_MAX_OUTER + a.outer] : ntot;
   const int* fl = a.fit_list + (size_t)lane * (a.in_cap[0] + a.in_cap[1]);
@@ -585,7 +586,7 @@ __global__ void __launch_bounds__(128) k_map_fit_reuse(MapArgs a) {
 __global__ void __launch_bounds__(128) k_map_fit(MapArgs a) {
   const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
-  if (s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
+  if (!lane_maps(a.lane_flags, lane) || s.map_too_small || s.map_done) return;   // :554 / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   const int n0 = s.n_stack[0], ntot = n0 + s.n_stack[1];
   const float4* M0 = a.from_map[0] + (size_t)lane * a.map_cap[0];
   const float4* M1 = a.from_map[1] + (size_t)lane * a.map_cap[1];
@@ -826,6 +827,7 @@ static inline void lvo_launch_mapping(cudaStream_t st, MapArgs a, const SolveArg
     else k_map_fit<<<ga, 128, 0, st>>>(a);
     if (launches) *launches += 1;
     SolveArgs sa = solve_proto;
+    sa.lane_flags = a.lane_flags;
     sa.which = 1; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = 0; sa.reset_cnt = nullptr;  // LidarEdgeFactor(..., 1.0), :610
     LVO_MARK(tm, LVO_ST_MAP_SOLVER, st);
     lvo_launch_lm(st, sa, lanes, 16384);

@@ -101,7 +101,7 @@ __global__ void k_odo_begin(OdoArgs a) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
   if (lane >= a.lanes) return;
   LaneState& s = a.ls[lane];
-  if (!lane_active(a.lane_flags, lane)) { s.odo_done = 1; return; }   // idle: the association and solve kernels return at once
+  if (!lane_active(a.lane_flags, lane)) return;   // idle: the association and solve kernels return for it by its lane flags
   s.odo_status = s.odo_inited ? LVO_OK : LVO_W_FIRST_FRAME;
   s.odo_done = 0; s.stats.odo_outer_executed = 0;
   for (int o = 0; o < LVO_MAX_OUTER; ++o) { s.stats.odo_corner_corr[o] = 0; s.stats.odo_plane_corr[o] = 0; s.stats.odo_lm_iters[o] = 0; s.stats.odo_final_cost[o] = 0; s.stats.odo_slow[o] = 0; s.stats.odo_certified[o] = 0; }
@@ -299,7 +299,7 @@ __global__ void __launch_bounds__(128) k_odo_assoc_fast(OdoArgs a) {
   __shared__ GridView gv[4];
   const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
-  if (!s.odo_inited || s.odo_done) return;   // first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
+  if (!lane_active(a.lane_flags, lane) || !s.odo_inited || s.odo_done) return;   // idle / first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   if (threadIdx.x < 4) gv[threadIdx.x] = grid_view(a.grid, LVO_ODO_GRIDS * lane + threadIdx.x);
   __syncthreads();
   const int ns = s.n_sharp, nf = s.n_flat;
@@ -538,7 +538,7 @@ __global__ void __launch_bounds__(256, 4) k_odo_assoc(OdoArgs a) {
   __shared__ GridView gv[LVO_ODO_GRIDS];
   const int lane = blockIdx.y;
   LaneState& s = a.ls[lane];
-  if (!s.odo_inited || s.odo_done) return;   // first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
+  if (!lane_active(a.lane_flags, lane) || !s.odo_inited || s.odo_done) return;   // idle / first frame / fixed point reached (LVO_OPT_FIXPOINT_SKIP)
   if (threadIdx.x < LVO_ODO_GRIDS) gv[threadIdx.x] = grid_view(a.grid, LVO_ODO_GRIDS * lane + threadIdx.x);
   __syncthreads();
   const int ns = s.n_sharp, nf = s.n_flat;
@@ -791,6 +791,7 @@ static inline void lvo_launch_odometry(cudaStream_t st, OdoArgs a, const SolveAr
     if (o == 0) k_odo_assoc<8><<<ga, 256, 0, st>>>(a);   // first iteration: more features lack a nearby candidate
     else k_odo_assoc<32><<<gs, 256, 0, st>>>(a);
     SolveArgs sa = solve_proto;
+    sa.lane_flags = a.lane_flags;
     sa.which = 0; sa.outer = o; sa.n_outer = outer_iters; sa.factors = a.factors; sa.factor_cap = a.factor_cap; sa.distort = a.distortion != 0; sa.reset_cnt = a.slow_cnt;
     LVO_MARK(tm, LVO_ST_ODO_SOLVER, st);
     lvo_launch_lm(st, sa, lanes, nfeat_cap);

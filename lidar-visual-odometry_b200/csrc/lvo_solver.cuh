@@ -291,6 +291,7 @@ struct SolveArgs {
   int n_outer;                // outer iterations of the frame (stats slots to fill when the loop is cut short)
   int fixpoint_skip;          // LVO_OPT_FIXPOINT_SKIP
   int* reset_cnt;             // [lanes] or null: per-lane counter the solve zeroes for the next outer iteration (the scan-to-scan slow-list length)
+  const int* lane_flags;      // [lanes] LVO_LANE_* of the step: idle lanes (odometry) and lanes that do not map (mapping) return at once
 };
 
 struct LmShared {
@@ -417,7 +418,8 @@ __global__ void __launch_bounds__(LVO_LM_THREADS, LVO_LM_MINB) k_lm_solve(SolveA
   const int lane = blockIdx.x;
   LaneState& s = a.ls[lane];
   if (a.reset_cnt && threadIdx.x == 0) a.reset_cnt[lane] = 0;   // the association kernels of this iteration are through with it
-  if (a.which == 0 ? (s.odo_inited == 0 || s.odo_done != 0) : (s.map_too_small != 0 || s.map_done != 0)) return;
+  if (a.which == 0 ? (!lane_active(a.lane_flags, lane) || s.odo_inited == 0 || s.odo_done != 0)
+                   : (!lane_maps(a.lane_flags, lane) || s.map_too_small != 0 || s.map_done != 0)) return;
   const int nslots = a.which == 0 ? (s.n_sharp + s.n_flat) : (s.n_stack[0] + s.n_stack[1]);
   const LvoFactor* F = a.factors + (size_t)lane * a.factor_cap;
   double* xg = a.which == 0 ? s.para_q : s.map_x;  // para_q[4], para_t[3] are contiguous

@@ -182,10 +182,12 @@ long lvo_synth_rays(int model) { return model == 16 ? 16L * 1800 : 64L * 1875; }
 // Generates sweep `frame` of sequence `seq` into out[cap] (packed x,y,z,intensity=0).  gt_pose7 (optional) gets the
 // ground-truth sensor pose (q xyzw, t) in the frame of sweep 0 of the same sequence.  Returns the number of points,
 // or -1 if cap is too small / the model is unknown.
-static long synth_sweep(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7, bool moving) {
+// naz = azimuth columns per sweep (0: the model's default).
+static long synth_sweep(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7, bool moving, int naz = 0) {
   if (model != 16 && model != 64) return -1;
-  const int beams = model, naz = model == 16 ? 1800 : 1875;
-  if (cap < (long)beams * naz) return -1;
+  const int beams = model;
+  if (naz == 0) naz = model == 16 ? 1800 : 1875;
+  if (naz < 1 || cap < (long)beams * naz) return -1;
   Scene sc;
   sc.seed = 1000ull * (uint64_t)model + 10ull * (uint64_t)seq;
   Pose P, P0;
@@ -237,7 +239,7 @@ static long synth_sweep(int model, int seq, int frame, double speed, float* out_
                       P.R[6] * ds[0] + P.R[7] * ds[1] + P.R[8] * ds[2]};
       double t = sc.cast(P.t, dw);
       if (!(t < max_range) || t < min_keep) continue;
-      uint64_t h = hash3(sc.seed ^ 0xABCDEF, (uint64_t)frame, (uint64_t)(j * 64 + b));
+      uint64_t h = hash3(sc.seed ^ 0xABCDEF, (uint64_t)frame, (uint64_t)j * 64 + (uint64_t)b);
       double u1 = u01(h), u2 = u01(mix64(h));
       double g = std::sqrt(-2.0 * std::log(u1)) * std::cos(2 * M_PI * u2);
       double r = t + sigma * g;
@@ -256,6 +258,11 @@ long lvo_synth_sweep(int model, int seq, int frame, double speed, float* out_xyz
 // frame + j / naz.  gt_pose7 = pose at the end of the sweep relative to the end of sweep 0.
 long lvo_synth_sweep_moving(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7) {
   return synth_sweep(model, seq, frame, speed, out_xyzi, cap, gt_pose7, true);
+}
+// Same scene and trajectory as lvo_synth_sweep with `naz` azimuth columns per ring (0: the model's default): dense rings of sensors
+// that spin slower or fire faster, e.g. a VLP-16 at 5 Hz (~3600 columns).  out[cap] needs model * naz entries.
+long lvo_synth_sweep_res(int model, int seq, int frame, double speed, int naz, float* out_xyzi, long cap, double* gt_pose7) {
+  return synth_sweep(model, seq, frame, speed, out_xyzi, cap, gt_pose7, false, naz);
 }
 
 }  // extern "C"

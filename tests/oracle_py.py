@@ -27,15 +27,21 @@ class Synth:
         self.lib.lvo_synth_sweep.argtypes = [C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_long, C.c_void_p]
         self.lib.lvo_synth_sweep_moving.restype = C.c_long
         self.lib.lvo_synth_sweep_moving.argtypes = self.lib.lvo_synth_sweep.argtypes
+        self.lib.lvo_synth_sweep_res.restype = C.c_long
+        self.lib.lvo_synth_sweep_res.argtypes = [C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_long, C.c_void_p]
 
-    def sweep(self, model, seq, frame, speed=None, moving=False):
-        """moving=True: the sensor keeps moving while it spins (intra-sweep motion distortion, the DISTORTION 1 input)."""
+    def sweep(self, model, seq, frame, speed=None, moving=False, naz=None):
+        """moving=True: the sensor keeps moving while it spins (intra-sweep motion distortion, the DISTORTION 1 input).
+        naz: azimuth columns per ring instead of the model's 1800 / 1875 (dense rings; rigid sweeps only)."""
         if speed is None:
             speed = 1.0 if model == 64 else 0.2
-        cap = self.lib.lvo_synth_rays(model)
-        out = np.empty((cap, 4), np.float32)
+        out = np.empty((model * naz if naz else self.lib.lvo_synth_rays(model), 4), np.float32)
         gt = np.empty(7, np.float64)
-        n = (self.lib.lvo_synth_sweep_moving if moving else self.lib.lvo_synth_sweep)(model, seq, frame, speed, _ptr(out), cap, _ptr(gt))
+        if naz:
+            assert not moving
+            n = self.lib.lvo_synth_sweep_res(model, seq, frame, speed, naz, _ptr(out), len(out), _ptr(gt))
+        else:
+            n = (self.lib.lvo_synth_sweep_moving if moving else self.lib.lvo_synth_sweep)(model, seq, frame, speed, _ptr(out), len(out), _ptr(gt))
         assert n >= 0
         return out[:n].copy(), gt
 

@@ -5,6 +5,7 @@ iteration 0 bit-exact, LM control flow, pose within 1e-4 m / 1e-5 rad, map sizes
 import numpy as np
 import pytest
 
+from conftest import record_metric
 from dense_map import make_dense_map
 from oracle_py import Oracle
 
@@ -57,7 +58,10 @@ def test_scan_to_map_dense_map_parity(lvo_mod, synth):
             if f1 == 0 and f2 == 0:
                 n = len(lg["lm"])
                 assert np.array_equal(tr[o][:n, 9], lg["lm"][:, 9]), (k, o)
-        assert flips <= 0.002 * rows, (flips, rows)
+        # both sides are deterministic on fixed inputs: a B200 run records 0 differing rows on every frame of this test
+        print(f"dense map frame {k}: {flips} of {rows} kNN / accept rows differ")
+        record_metric(f"dense_map_rows_differing_from_oracle/frame{k}", {"differ": flips, "rows": rows})
+        assert flips == 0, (flips, rows)
         assert np.linalg.norm(pose_g[4:] - pose_o[4:]) < 1e-4 and rot_err(pose_g[:4], pose_o[:4]) < 1e-5, (k, pose_g, pose_o)
         lvo.set_map_correction(0, corr_o)
         for which in (0, 1):

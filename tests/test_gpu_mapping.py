@@ -86,7 +86,9 @@ def test_scan_to_map_from_imported_state(lvo_mod, synth, model, cfg, seq):
         assert reg_g.shape == reg_o.shape and np.abs(reg_g - reg_o).max() < 1e-3
     from conftest import record_metric
     record_metric(f"mapping_knn_and_accept_rows_differing_from_oracle/model{model}_seq{seq}", {"differ": int(flips), "rows": int(rows), "frames": len(frames)})
-    assert flips <= 0.002 * max(rows, 1), f"{flips} of {rows} kNN / accept rows differ"
+    # both sides are deterministic on fixed inputs: a B200 run records 0 differing rows on both sequences of this test
+    print(f"mapping model {model} seq {seq}: {flips} of {rows} kNN / accept rows differ")
+    assert flips == 0, f"{flips} of {rows} kNN / accept rows differ"
     lvo.close()
 
 

@@ -53,7 +53,9 @@ def _run(lvo_mod, synth, model, cfg, nframes, seq, distortion=0):
         assert np.linalg.norm(w_g[4:] - w_o[4:]) < POS_TOL and rot_err(w_g[:4], w_o[:4]) < ROT_TOL, (k, w_g, w_o)
     from conftest import record_metric
     record_metric(f"odometry_rows_differing_from_oracle/model{model}_seq{seq}_distortion{distortion}", {"differ": int(flips_total), "rows": int(rows_total), "frames": nframes})
-    assert flips_total <= 0.002 * max(rows_total, 1), f"{flips_total} of {rows_total} correspondence rows differ"
+    # both sides are deterministic on fixed inputs: a B200 run records 0 differing rows on every sequence of this test
+    print(f"odometry model {model} seq {seq} distortion {distortion}: {flips_total} of {rows_total} correspondence rows differ")
+    assert flips_total == 0, f"{flips_total} of {rows_total} correspondence rows differ"
     lvo.close()
 
 
