@@ -338,8 +338,53 @@ enum lvo_probe {
   LVO_P_MAP_CORNER_VALID = 20,/* int[outer][n_corner_stack]  1 if an edge factor was added        :611                 */
   LVO_P_MAP_SURF_VALID = 21,  /* int[outer][n_surf_stack]    1 if a plane factor was added        :681                 */
   LVO_P_MAP_LM_TRACE = 22,    /* as LVO_P_ODO_LM_TRACE                                            ceres::Solve :720    */
-  LVO_P_REGISTERED = 23       /* lvo_point[n_kept]                                                :838-842             */
+  LVO_P_REGISTERED = 23,      /* lvo_point[n_kept]                                                :838-842             */
+  LVO_P_ODO_UNCERTAINTY = 24, /* lvo_pose_uncertainty[1] of the scan-to-scan solve (T_last_curr)  :571-576             */
+  LVO_P_MAP_UNCERTAINTY = 25  /* lvo_pose_uncertainty[1] of the scan-to-map solve (T_wmap_curr)   laserMapping.cpp:720 */
 };
+
+/* Pose uncertainty of a stage's solve: how well the reference's final ceres::Problem constrains the pose (LVO_P_ODO_UNCERTAINTY,
+ * LVO_P_MAP_UNCERTAINTY).  The reference publishes /laser_odom_to_init and /aft_mapped_to_init with a zero covariance.
+ *   - The record describes the lane's LAST EXECUTED outer iteration of the stage's most recent run: scan-to-scan the problem on
+ *     (para_q, para_t) = T_last_curr, scan-to-map the problem on parameters[7] = T_wmap_curr.  (With LVO_OPT_FIXPOINT_SKIP that is
+ *     the fixed-point iteration, whose problem every later iteration would reproduce bit for bit.)
+ *   - Coordinates p = (tx, ty, tz, theta_x, theta_y, theta_z), the order of ROS PoseWithCovariance::covariance: theta is the rotation
+ *     vector of a LEFT perturbation R <- Exp(theta) R about the parent frame's fixed axes (the previous sensor frame for odometry, the
+ *     map frame for mapping), and t <- t + dt.
+ *   - information: the Gauss-Newton information J^T W J at the final pose, built from that iteration's residual blocks with their
+ *     Huber corrector weights, i.e. what ceres::Covariance with default options (apply_loss_function = true) would use on the
+ *     reference's final problem, expressed in p.  Row-major 6 x 6, symmetric.
+ *   - eigenvalues ascending; eigenvectors row-major 6 x 6, eigenvector k in column k, its largest-magnitude entry positive (the first
+ *     one on ties).  eigenvalues[0] and column 0 are the weakest direction: a degenerate lane (a straight corridor, open flat
+ *     ground, a map too sparse to pin an axis) shows a small eigenvalues[0] relative to eigenvalues[5].
+ *   - positive_definite = eigenvalues[0] > 0 && eigenvalues[0] >= 1e-14 eigenvalues[5] (the threshold is Ceres' default
+ *     min_reciprocal_condition_number; Ceres applies it to its own factorisation, this library to the eigenvalues).  Then
+ *     covariance = V diag(1 / eigenvalues) V^T (row-major 6 x 6, symmetric: m^2 and rad^2); otherwise all zeros.
+ *   - frame: the lane's frame index within its sequence (0 = first frame) of the run that wrote the record; -1 when the stage has
+ *     not run since the lane was created, reset, configured or loaded, and -1 when lvo_scan_to_scan / lvo_scan_to_map (which keep no
+ *     frame count) wrote it.
+ *   - solved: the stage's solver ran for the lane on that frame: 0 on the odometry's first frame and on a map-too-small frame, and
+ *     then information, cost and n_factors are zero.  n_factors: residual blocks of the iteration (lvo_stats corner + plane
+ *     correspondences, or corner + surf); cost equals that iteration's lvo_stats::odo_final_cost / map_final_cost bit for bit.
+ * Lifecycle: an idle lane keeps both records; a lane that does not map in a step keeps its mapping record (with its old frame);
+ * lvo_lane_reset and lvo_lane_configure clear both (frame = -1); after lvo_lane_load the probes return LVO_E_STATE until the stage
+ * runs, like the other probes of the stage.  lvo_knn, the depth calls and the map outputs leave them alone.  The records are not
+ * part of a snapshot.  They are results, not per-iteration intermediates: lvo_config::debug_probes does not affect them.
+ * Cost: the first fetch after a call that can change a record derives every lane's records in one launch and one copy into a host
+ * mirror; later fetches read the mirror.  A fetch leaves lvo_timings as it was. */
+typedef struct lvo_pose_uncertainty {
+  int64_t frame;
+  int solved;
+  int positive_definite;
+  int n_factors;
+  int reserved;
+  double cost;
+  double information[36];
+  double covariance[36];
+  double eigenvalues[6];
+  double eigenvectors[36];
+} lvo_pose_uncertainty;
+
 /* Copies up to cap_bytes; *n_bytes gets the full size (so a too-small buffer can be detected). */
 int lvo_probe_fetch(lvo_ctx* ctx, int lane, int what, void* out, size_t cap_bytes, size_t* n_bytes);
 

@@ -27,6 +27,8 @@ LVO_MAP_SURROUND, LVO_MAP_WHOLE, LVO_MAP_REGISTERED = 0, 1, 2
 (P_FULL, P_CURVATURE, P_SORT_IND, P_LABEL, P_PICKED, P_SCAN_START, P_SCAN_END, P_SHARP, P_LESS_SHARP, P_FLAT, P_LESS_FLAT,
  P_ODO_CORNER_CORR, P_ODO_PLANE_CORR, P_ODO_LM_TRACE, P_MAP_CORNER_STACK, P_MAP_SURF_STACK, P_MAP_CORNER_FROM_MAP,
  P_MAP_SURF_FROM_MAP, P_MAP_CORNER_KNN, P_MAP_SURF_KNN, P_MAP_CORNER_VALID, P_MAP_SURF_VALID, P_MAP_LM_TRACE, P_REGISTERED) = range(24)
+P_ODO_UNCERTAINTY, P_MAP_UNCERTAINTY = 24, 25   # one lvo_pose_uncertainty record each (Lvo.pose_uncertainty)
+UNCERTAINTY_PROBES = {"odometry": P_ODO_UNCERTAINTY, "mapping": P_MAP_UNCERTAINTY}
 
 
 class CloudView(C.Structure):
@@ -59,6 +61,21 @@ class Stats(C.Structure):
                 ("map_corner_corr", C.c_int * 16), ("map_surf_corr", C.c_int * 16), ("map_lm_iters", C.c_int * 16), ("map_final_cost", C.c_double * 16),
                 ("map_corner_total", C.c_int), ("map_surf_total", C.c_int), ("center_cube", C.c_int * 3), ("cen", C.c_int * 3),
                 ("odo_outer_executed", C.c_int), ("map_outer_executed", C.c_int), ("map_knn_full", C.c_int * 16), ("odo_slow", C.c_int * 16), ("odo_slow_why", C.c_int * 6), ("odo_certified", C.c_int * 16)]
+
+
+class PoseUncertainty(C.Structure):
+    """lvo_pose_uncertainty: information, covariance and eigen-decomposition of a stage's solve in p = (tx, ty, tz, theta_x, theta_y, theta_z)."""
+    _fields_ = [("frame", C.c_int64), ("solved", C.c_int), ("positive_definite", C.c_int), ("n_factors", C.c_int), ("reserved", C.c_int),
+                ("cost", C.c_double), ("information", C.c_double * 36), ("covariance", C.c_double * 36), ("eigenvalues", C.c_double * 6),
+                ("eigenvectors", C.c_double * 36)]
+
+
+def uncertainty_to_dict(u):
+    """PoseUncertainty -> dict of numpy arrays (6 x 6 matrices row-major, eigenvector k in column k)."""
+    m = lambda a: np.ctypeslib.as_array(a).reshape(6, 6).copy()
+    return dict(frame=int(u.frame), solved=int(u.solved), positive_definite=int(u.positive_definite), n_factors=int(u.n_factors), cost=float(u.cost),
+                information=m(u.information), covariance=m(u.covariance), eigenvalues=np.ctypeslib.as_array(u.eigenvalues).copy(),
+                eigenvectors=m(u.eigenvectors))
 
 
 class Camera(C.Structure):
@@ -499,6 +516,14 @@ class Lvo:
         if what in (P_MAP_CORNER_VALID, P_MAP_SURF_VALID):
             return raw.view(np.int32).reshape(O, -1).copy()
         raise KeyError(what)
+
+    def pose_uncertainty(self, lane=0, stage="odometry"):
+        """The pose-uncertainty record of `lane` for stage "odometry" (T_last_curr) or "mapping" (T_wmap_curr), as a dict of numpy arrays:
+        frame, solved, positive_definite, n_factors, cost, information (6 x 6), covariance (6 x 6), eigenvalues (6, ascending),
+        eigenvectors (6 x 6, column k for eigenvalue k).  Coordinates (tx, ty, tz, theta_x, theta_y, theta_z), include/lvo.h."""
+        u = PoseUncertainty()
+        self._check(self.lib.lvo_probe_fetch(self.h, lane, UNCERTAINTY_PROBES[stage], C.byref(u), C.sizeof(u), None))
+        return uncertainty_to_dict(u)
 
     def knn5_throughput(self, d_maps_ptr, map_counts, d_queries_ptr, query_counts, reps, d_ind_ptr, d_sq_ptr):
         """S problems in one launch (device pointers in, device outputs); returns average kernel milliseconds."""

@@ -135,6 +135,13 @@ struct lvo_ctx {
   // overwritten map.registered, until the next step completes
   std::vector<size_t> reg_n;
   bool reg_valid = true;
+  // pose uncertainty (LVO_P_*_UNCERTAINTY): raw records [lanes][2] written by k_lm_solve; the derived records of every lane come to a
+  // pinned mirror on the first fetch after unc_epoch moved (every call that can change a raw record bumps it); unc_frame is each
+  // record's frame field, kept on the host (lane_frame of the step that wrote it, -1 otherwise)
+  LvoUncRaw* d_unc = nullptr;
+  lvo_pose_uncertainty* d_unc_out = nullptr; lvo_pose_uncertainty* h_unc = nullptr;
+  std::vector<int64_t> unc_frame;
+  long long unc_epoch = 0, unc_mirror_epoch = -1;
 };
 
 void lvo_set_error(lvo_ctx* ctx, const std::string& msg) { if (ctx) ctx->err = msg; }
@@ -305,6 +312,12 @@ int upload_lane_config(lvo_ctx* c, int lane) {
 }
 // the stand-alone stage calls run their stage for every lane: its probes are this context's own again
 void stage_ran_on_all_lanes(lvo_ctx* c, int gate) { for (char& g : c->probe_gate) g &= ~gate; }
+// lvo_scan_to_scan (stage 0) / lvo_scan_to_map (stage 1) rewrite that stage's pose-uncertainty record of every lane; they keep no frame
+// count, so the records' frame is -1
+void uncertainty_written(lvo_ctx* c, int stage) {
+  for (int l = 0; l < c->lanes; ++l) c->unc_frame[2 * l + stage] = -1;
+  c->unc_epoch++;
+}
 // sweep pointers, counts and lane flags of the step
 int set_inputs(lvo_ctx* c) {
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->d_in_ptr, c->h_in_ptr, sizeof(void*) * c->lanes, cudaMemcpyHostToDevice, c->st));
@@ -490,6 +503,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   c->lane_map_update.assign(L, 1);
   c->probe_gate.assign(L, 0);
   c->reg_n.assign(L, 0);
+  c->unc_frame.assign(2 * (size_t)L, -1);
   c->lane_cfg.assign(L, lvo_lane_config{c->cfg.n_scans, c->cfg.minimum_range, c->cfg.line_res, c->cfg.plane_res, c->cfg.skip_frame});
 
   LVO_TRY(dalloc(c, &c->d_ls, (size_t)L));
@@ -528,13 +542,16 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   memset(&so, 0, sizeof(so));
   so.ls = c->d_ls; so.max_iters = cfg->lm_max_iters; so.huber = cfg->huber;
   so.n_outer = cfg->outer_iters; so.fixpoint_skip = 1;
+  LVO_TRY(dalloc(c, &c->d_unc, 2 * (size_t)L));
+  LVO_TRY(dalloc(c, &c->d_unc_out, 2 * (size_t)L, false)); LVO_TRY(halloc(c, &c->h_unc, 2 * (size_t)L));
+  so.unc = c->d_unc;
   const size_t trace_n = (size_t)L * LVO_MAX_OUTER * (LVO_MAX_LM + 1) * LVO_TRACE_W;
   LVO_TRY(dalloc(c, &c->d_trace[0], trace_n)); LVO_TRY(dalloc(c, &c->d_trace[1], trace_n));
 
   // ---- odometry
   OdoArgs& od = c->odo;
   memset(&od, 0, sizeof(od));
-  od.ls = c->d_ls; od.lanes = L; od.distortion = cfg->distortion; od.full = ex.full; od.lane_flags = ex.lane_flags;
+  od.ls = c->d_ls; od.lanes = L; od.distortion = cfg->distortion; od.full = ex.full; od.lane_flags = ex.lane_flags; od.unc = c->d_unc;
   od.sharp = ex.sharp; od.less_sharp = ex.less_sharp; od.flat = ex.flat; od.less_flat = ex.less_flat;
   od.cap_sharp = c->cap_sharp; od.cap_lsharp = c->cap_lsharp; od.cap_flat = c->cap_flat; od.P = P;
   // per-outer-iteration probe arrays: all LVO_MAX_OUTER iterations only when the parity probes are wanted, else the current and the previous one
@@ -556,7 +573,7 @@ int lvo_create(const lvo_config* cfg, lvo_ctx** out) {
   // ---- mapping
   MapArgs& mp = c->map;
   memset(&mp, 0, sizeof(mp));
-  mp.ls = c->d_ls; mp.lanes = L; mp.lane_flags = ex.lane_flags; mp.lcfg = c->d_lcfg;
+  mp.ls = c->d_ls; mp.lanes = L; mp.lane_flags = ex.lane_flags; mp.lcfg = c->d_lcfg; mp.unc = c->d_unc;
   mp.in_pts[0] = ex.less_sharp; mp.in_pts[1] = ex.less_flat; mp.in_cap[0] = c->cap_lsharp; mp.in_cap[1] = P;
   mp.full = ex.full; mp.P = P; mp.gen = 0; mp.slots = slots;
   mp.knn_reuse = 1;   // default: neighbour sets carried across the outer iterations with a certificate
@@ -730,6 +747,7 @@ int lvo_scan_to_scan(lvo_ctx* c, lvo_cloud_view sharp, lvo_cloud_view less_sharp
   LvoStageTimer* tm = stage_timer_begin(c, true);
   enqueue_odometry(c, tm);
   stage_ran_on_all_lanes(c, LVO_PROBE_GATE_ODO);
+  uncertainty_written(c, 0);
   c->stage_tm.stop(c->st);
   cudaEventRecord(c->ev[3], c->st);
   LVO_TRY(sync_state(c));
@@ -764,6 +782,7 @@ int lvo_scan_to_map(lvo_ctx* c, lvo_cloud_view corner_last, lvo_cloud_view surf_
   LvoStageTimer* tm = stage_timer_begin(c, true);
   enqueue_mapping(c, 0, want_reg, tm);
   stage_ran_on_all_lanes(c, LVO_PROBE_GATE_MAP);
+  uncertainty_written(c, 1);
   c->stage_tm.stop(c->st);
   cudaEventRecord(c->ev[5], c->st);
   LVO_TRY(sync_state(c));
@@ -865,9 +884,12 @@ static int step_enqueue(lvo_ctx* c, int stride, int off_xyz, int max_n) {
   nvtxRangePop();
   for (int l = 0; l < c->lanes; ++l) {
     const int f = lane_flags(c)[l];
+    if (f & LVO_LANE_ACTIVE) c->unc_frame[2 * l] = c->lane_frame[l];       // the frame index of this step
+    if (f & LVO_LANE_MAPS) c->unc_frame[2 * l + 1] = c->lane_frame[l];
     if (f & LVO_LANE_ACTIVE) { c->lane_frame[l]++; c->probe_gate[l] &= ~(LVO_PROBE_GATE_EXTRACT | LVO_PROBE_GATE_ODO); }
     if (f & LVO_LANE_MAPS) c->probe_gate[l] = 0;
   }
+  c->unc_epoch++;
   // the lane states come back on the same stream; lvo_wait only has to synchronise
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->h_ls, c->d_ls, sizeof(LaneState) * c->lanes, cudaMemcpyDeviceToHost, c->st));
   c->pending = true; c->pending_do_map = do_map; c->pending_graph = use_graph;
@@ -1033,6 +1055,7 @@ static int reset_lane(lvo_ctx* c, int lane, const lvo_lane_config* cfg) {
     for (int t = 0; t < 2; ++t)
       LVO_CUDA_OK(c, cudaMemsetAsync(c->map.cube_start[g][t] + (size_t)lane * (LVO_NCUBES + 1), 0, sizeof(unsigned) * (LVO_NCUBES + 1), c->st));
   k_init_lanes<<<1, 64, 0, c->st>>>(c->d_ls, lane, 1);
+  LVO_CUDA_OK(c, cudaMemsetAsync(c->d_unc + 2 * (size_t)lane, 0, 2 * sizeof(LvoUncRaw), c->st));   // both pose-uncertainty records
   if (cfg) { c->lane_cfg[lane] = *cfg; LVO_TRY(upload_lane_config(c, lane)); }
   // and its host copies, so that lvo_get_stats / lvo_lane_status report the new sequence at once
   LVO_CUDA_OK(c, cudaMemcpyAsync(c->h_ls + lane, c->d_ls + lane, sizeof(LaneState), cudaMemcpyDeviceToHost, c->st));
@@ -1042,6 +1065,8 @@ static int reset_lane(lvo_ctx* c, int lane, const lvo_lane_config* cfg) {
   c->lane_frame[lane] = 0;
   c->probe_gate[lane] = 0;   // zero counts: every probe is empty, and in bounds
   c->reg_n[lane] = 0;
+  c->unc_frame[2 * lane] = c->unc_frame[2 * lane + 1] = -1;
+  c->unc_epoch++;
   return LVO_OK;
 }
 extern "C" {
@@ -1275,6 +1300,8 @@ int lvo_lane_load(lvo_ctx* c, int lane, const void* src, size_t n_bytes) {
   c->probe_gate[lane] = LVO_PROBE_GATE_EXTRACT | LVO_PROBE_GATE_ODO | LVO_PROBE_GATE_MAP;
   c->odo_grids_stale = true;
   c->reg_n[lane] = 0;
+  c->unc_frame[2 * lane] = c->unc_frame[2 * lane + 1] = -1;   // gated until the stage runs (probe_gate)
+  c->unc_epoch++;
   return LVO_OK;
 }
 
@@ -1534,8 +1561,37 @@ int lvo_set_odometry_state(lvo_ctx* c, int lane, const lvo_pose* T_last_curr, co
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+}  // extern "C"
+// LVO_P_ODO_UNCERTAINTY / LVO_P_MAP_UNCERTAINTY: one launch of k_pose_uncertainty and one copy bring every lane's records into the
+// pinned mirror when a raw record may have changed since the last fetch; otherwise the mirror answers.  The launch is not counted in
+// lvo_timings::kernel_launches, which keeps reporting the last step or stage call.
+static int fetch_uncertainty(lvo_ctx* c, int lane, int stage, void* out, size_t cap_bytes, size_t* n_bytes) {
+  if (c->probe_gate[lane] & (stage ? LVO_PROBE_GATE_MAP : LVO_PROBE_GATE_ODO)) {
+    lvo_set_error(c, "the lane was loaded from a snapshot and the stage that writes this probe has not run for it since");
+    return LVO_E_STATE;
+  }
+  const size_t bytes = sizeof(lvo_pose_uncertainty);
+  if (n_bytes) *n_bytes = bytes;
+  if (!out) return LVO_OK;  // size query
+  if (cap_bytes < bytes) return LVO_E_CAPACITY;
+  if (c->unc_mirror_epoch != c->unc_epoch) {
+    const int n = 2 * c->lanes;
+    k_pose_uncertainty<<<lvo_div_up(n, 64), 64, 0, c->st>>>(c->d_unc, c->d_unc_out, n);
+    LVO_CUDA_OK(c, cudaGetLastError());
+    LVO_CUDA_OK(c, cudaMemcpyAsync(c->h_unc, c->d_unc_out, bytes * n, cudaMemcpyDeviceToHost, c->st));
+    LVO_CUDA_OK(c, cudaStreamSynchronize(c->st));
+    c->unc_mirror_epoch = c->unc_epoch;
+  }
+  lvo_pose_uncertainty r = c->h_unc[2 * lane + stage];
+  r.frame = c->unc_frame[2 * lane + stage];
+  memcpy(out, &r, bytes);
+  return LVO_OK;
+}
+extern "C" {
+
 int lvo_probe_fetch(lvo_ctx* c, int lane, int what, void* out, size_t cap_bytes, size_t* n_bytes) {
   LVO_ENTER_LANE(c, lane);
+  if (what == LVO_P_ODO_UNCERTAINTY || what == LVO_P_MAP_UNCERTAINTY) return fetch_uncertainty(c, lane, what == LVO_P_MAP_UNCERTAINTY ? 1 : 0, out, cap_bytes, n_bytes);
   LVO_TRY(sync_state(c));
   const LaneState& s = c->h_ls[lane];
   const ExtractArgs& ex = c->ex;

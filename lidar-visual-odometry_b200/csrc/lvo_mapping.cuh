@@ -65,6 +65,7 @@ struct MapArgs {
   int* fit_list;                     // [lanes][in_cap[0] + in_cap[1]] factor slots whose row changed in this outer iteration (k_map_fit_reuse refits them)
   int* fit_cnt;                      // [lanes][LVO_MAX_OUTER] their number per outer iteration (zeroed by k_map_begin)
   float4* registered;                // [lanes][P] or null
+  LvoUncRaw* unc;                    // [lanes][2] pose-uncertainty records (lvo_solver.cuh); k_map_begin clears `solved` of stage 1
 };
 
 __device__ __forceinline__ int cube_index(int i, int j, int k) { return i + LVO_CUBE_W * j + LVO_CUBE_W * LVO_CUBE_H * k; }
@@ -77,6 +78,7 @@ __global__ void k_map_begin(MapArgs a) {
   // gather / stack / refilter / finish / register kernels see no items, and the rebuild carries its map into the other generation
   // unchanged.  Nothing of its state is written, so that its snapshot does not depend on what the other lanes of the context do.
   if (!lane_maps(a.lane_flags, lane)) return;
+  a.unc[2 * lane + 1].solved = 0;   // set again by k_lm_solve unless the map is too small
   if (a.from_odo) { for (int k = 0; k < 4; ++k) s.q_wodom[k] = s.q_w[k]; for (int k = 0; k < 3; ++k) s.t_wodom[k] = s.t_w[k]; }
   // transformAssociateToMap
   quat_mul(s.q_wmap_wodom, s.q_wodom, s.map_x);
@@ -203,7 +205,7 @@ __device__ __forceinline__ void fit_factor(int t, const float4 ori, const float4
         for (int c = 0; c < 3; ++c) cov[r * 3 + c] = cov[r * 3 + c] + z[r] * z[c];
     }
     double w[3], V[9];
-    sym_eigen3_dev(cov, w, V);
+    sym_eigen_dev<3>(cov, w, V);
     if (w[2] > 3 * w[1]) {  // :611
       const double ux = V[0 * 3 + 2], uy = V[1 * 3 + 2], uz = V[2 * 3 + 2];
       fac.type = 0; fac.d = 1.0;

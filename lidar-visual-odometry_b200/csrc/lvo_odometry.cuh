@@ -44,6 +44,7 @@ struct OdoArgs {
   float4* ref;       // [lanes][cap_sharp + cap_flat] feature position (TransformToStart) at its last full association
   float4* guard;     // [lanes][cap_sharp + cap_flat] guard radii of that association: x closest point, y same-ring point, z adjacent-ring point; w != 0: record valid
   int4* sel;         // [lanes][cap_sharp + cap_flat] what that association chose: x closest, y same-ring, z adjacent-ring point (-1: none inside the 5 m gate)
+  LvoUncRaw* unc;    // [lanes][2] pose-uncertainty records (lvo_solver.cuh); k_odo_begin clears `solved` of stage 0
 };
 
 // ---- certified reuse of a correspondence across outer iterations (LVO_OPT_ODO_REUSE) ---------------------------------------------
@@ -107,6 +108,7 @@ __global__ void k_odo_begin(OdoArgs a) {
   for (int o = 0; o < LVO_MAX_OUTER; ++o) { s.stats.odo_corner_corr[o] = 0; s.stats.odo_plane_corr[o] = 0; s.stats.odo_lm_iters[o] = 0; s.stats.odo_final_cost[o] = 0; s.stats.odo_slow[o] = 0; s.stats.odo_certified[o] = 0; }
   for (int k = 0; k < 6; ++k) s.stats.odo_slow_why[k] = 0;
   a.slow_cnt[lane] = 0;
+  a.unc[2 * lane].solved = 0;   // set again by k_lm_solve unless this is the first frame
 }
 
 struct Best { float d; int pos; int j; };

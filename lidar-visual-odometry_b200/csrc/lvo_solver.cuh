@@ -33,39 +33,52 @@
 #define LVO_NACC 28  // 21 + 6 + 1
 
 // ---- small dense routines (double) ---------------------------------------------------------------------------
-// cyclic Jacobi for a symmetric 3x3; eigenvalues ascending in w, eigenvectors in the columns of V (row-major)
-__device__ inline void sym_eigen3_dev(const double M[9], double w[3], double V[9]) {
-  double a[3][3], v[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
-  for (int r = 0; r < 3; ++r) for (int c = 0; c < 3; ++c) a[r][c] = M[r * 3 + c];
+// cyclic Jacobi for a symmetric NxN (N = 3: the line fit; N = 6: the pose information); eigenvalues ascending in w (stable order
+// for ties), eigenvectors in the columns of V (row-major).  tests/uncertainty_oracle.cpp sym_eigen restates it operation for operation.
+template <int N>
+__device__ inline void sym_eigen_dev(const double* M, double* w, double* V) {
+  double a[N][N], v[N][N];
+#pragma unroll
+  for (int r = 0; r < N; ++r)
+#pragma unroll
+    for (int c = 0; c < N; ++c) { a[r][c] = M[r * N + c]; v[r][c] = r == c ? 1.0 : 0.0; }
   for (int sweep = 0; sweep < 64; ++sweep) {
-    const double off = a[0][1] * a[0][1] + a[0][2] * a[0][2] + a[1][2] * a[1][2];
-    const double diag = a[0][0] * a[0][0] + a[1][1] * a[1][1] + a[2][2] * a[2][2];
+    double off = 0.0, diag = 0.0;
+#pragma unroll
+    for (int p = 0; p < N - 1; ++p)
+#pragma unroll
+      for (int q = p + 1; q < N; ++q) off += a[p][q] * a[p][q];
+#pragma unroll
+    for (int p = 0; p < N; ++p) diag += a[p][p] * a[p][p];
     if (off <= 1e-32 * diag || off == 0.0) break;
 #pragma unroll
-    for (int p = 0; p < 2; ++p)
+    for (int p = 0; p < N - 1; ++p)
 #pragma unroll
-      for (int q = p + 1; q < 3; ++q) {
+      for (int q = p + 1; q < N; ++q) {
         if (a[p][q] == 0.0) continue;
         const double theta = (a[q][q] - a[p][p]) / (2.0 * a[p][q]);
         const double t = (theta >= 0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
         const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
 #pragma unroll
-        for (int k = 0; k < 3; ++k) { const double akp = a[k][p], akq = a[k][q]; a[k][p] = c * akp - s * akq; a[k][q] = s * akp + c * akq; }
+        for (int k = 0; k < N; ++k) { const double akp = a[k][p], akq = a[k][q]; a[k][p] = c * akp - s * akq; a[k][q] = s * akp + c * akq; }
 #pragma unroll
-        for (int k = 0; k < 3; ++k) { const double apk = a[p][k], aqk = a[q][k]; a[p][k] = c * apk - s * aqk; a[q][k] = s * apk + c * aqk; }
+        for (int k = 0; k < N; ++k) { const double apk = a[p][k], aqk = a[q][k]; a[p][k] = c * apk - s * aqk; a[q][k] = s * apk + c * aqk; }
 #pragma unroll
-        for (int k = 0; k < 3; ++k) { const double vkp = v[k][p], vkq = v[k][q]; v[k][p] = c * vkp - s * vkq; v[k][q] = s * vkp + c * vkq; }
+        for (int k = 0; k < N; ++k) { const double vkp = v[k][p], vkq = v[k][q]; v[k][p] = c * vkp - s * vkq; v[k][q] = s * vkp + c * vkq; }
       }
   }
-  int o0 = 0, o1 = 1, o2 = 2;
-  double e0 = a[0][0], e1 = a[1][1], e2 = a[2][2];
-  // stable 3-element sort by eigenvalue
-  if (e1 < e0) { double t = e0; e0 = e1; e1 = t; int ti = o0; o0 = o1; o1 = ti; }
-  if (e2 < e1) { double t = e1; e1 = e2; e2 = t; int ti = o1; o1 = o2; o2 = ti; }
-  if (e1 < e0) { double t = e0; e0 = e1; e1 = t; int ti = o0; o0 = o1; o1 = ti; }
-  w[0] = e0; w[1] = e1; w[2] = e2;
-  const int ord[3] = {o0, o1, o2};
-  for (int c = 0; c < 3; ++c) for (int r = 0; r < 3; ++r) V[r * 3 + c] = v[r][ord[c]];
+  // stable insertion sort by eigenvalue
+  double e[N]; int ord[N];
+#pragma unroll
+  for (int i = 0; i < N; ++i) { e[i] = a[i][i]; ord[i] = i; }
+#pragma unroll
+  for (int i = 1; i < N; ++i)
+#pragma unroll
+    for (int j = i; j > 0; --j)
+      if (e[j] < e[j - 1]) { const double te = e[j]; e[j] = e[j - 1]; e[j - 1] = te; const int to = ord[j]; ord[j] = ord[j - 1]; ord[j - 1] = to; }
+#pragma unroll
+  for (int c = 0; c < N; ++c) w[c] = e[c];
+  for (int c = 0; c < N; ++c) for (int r = 0; r < N; ++r) V[r * N + c] = v[r][ord[c]];
 }
 
 // least squares min ||A y - b|| for a 5x3 A by Householder QR (A, b destroyed)
@@ -278,8 +291,19 @@ __device__ __forceinline__ void accumulate_factor(const LvoFactor& f, const doub
   }
 }
 
+// Raw pose-uncertainty record of one (lane, stage), [lanes][2] (stage 0 = odometry, 1 = mapping): the Gauss-Newton information
+// J^T W J of the last executed outer iteration at its final pose, in the solver's tangent u = (delta, dt) (upper triangle, row-major,
+// the 21 accumulators of lm_evaluate), its cost and residual blocks.  Written by k_lm_solve; `solved` cleared by k_odo_begin /
+// k_map_begin for the lanes that run the stage; k_pose_uncertainty derives the lvo_pose_uncertainty fields from it.
+struct LvoUncRaw {
+  double H[21];
+  double cost;
+  int n_factors, solved;
+};
+
 struct SolveArgs {
   LaneState* ls;
+  LvoUncRaw* unc;             // [lanes][2] raw records (stage = which)
   const LvoFactor* factors;   // [lanes][factor_cap]
   int factor_cap;
   int which;                  // 0 = odometry (x = para_q,para_t), 1 = mapping (x = map_x)
@@ -499,6 +523,11 @@ __global__ void __launch_bounds__(LVO_LM_THREADS, LVO_LM_MINB) k_lm_solve(SolveA
     bool fixed = a.fixpoint_skip != 0;
     for (int i = 0; i < 7; ++i) fixed = fixed && __double_as_longlong(c.x[i]) == __double_as_longlong(c.x0[i]);
     const double fc = c.nfactors ? c.cost : 0.0;
+    // c.H is the information at c.x: the initial evaluation's, replaced at every accepted step; a rejected or discarded candidate
+    // leaves both alone
+    LvoUncRaw& u = a.unc[2 * lane + a.which];
+    for (int i = 0; i < 21; ++i) u.H[i] = c.H[i];
+    u.cost = fc; u.n_factors = c.nfactors; u.solved = 1;
     if (a.which == 0) {
       s.stats.odo_lm_iters[a.outer] = c.iter; s.stats.odo_final_cost[a.outer] = fc;
       s.stats.odo_outer_executed = a.outer + 1;
@@ -521,6 +550,61 @@ __global__ void __launch_bounds__(LVO_LM_THREADS, LVO_LM_MINB) k_lm_solve(SolveA
       }
     }
   }
+}
+
+// ---- pose uncertainty (lvo_pose_uncertainty, include/lvo.h) ------------------------------------------------------------------
+// p = (t, theta) = M u with u = (delta, dt) the solver tangent (plus7_dev: q <- [sin|d| d^, cos|d|] q, so theta = 2 delta):
+// information H_p = M^-T H_u M^-1, i.e. the blocks H_tt, H_t,delta / 2, H_delta,delta / 4 reordered (exact scalings by 1/2, 1/4);
+// eigen-decomposition by sym_eigen_dev<6>, each eigenvector with its largest-magnitude entry positive (the first one on ties);
+// covariance V diag(1 / lambda) V^T when lambda_min > 0 and lambda_min >= 1e-14 lambda_max (Ceres' default
+// min_reciprocal_condition_number), else zero.  tests/uncertainty_oracle.cpp (derive_u) restates it operation for operation.
+__device__ inline void pose_uncertainty_derive(const double* Hu21, double* info, double* cov, double* w, double* V, int* pd) {
+  double Hu[6][6];
+  int t = 0;
+#pragma unroll
+  for (int i = 0; i < 6; ++i)
+#pragma unroll
+    for (int j = i; j < 6; ++j) { Hu[i][j] = Hu21[t]; Hu[j][i] = Hu21[t]; ++t; }
+#pragma unroll
+  for (int i = 0; i < 6; ++i)
+#pragma unroll
+    for (int j = 0; j < 6; ++j) info[i * 6 + j] = Hu[i < 3 ? i + 3 : i - 3][j < 3 ? j + 3 : j - 3] * ((i < 3 ? 1.0 : 0.5) * (j < 3 ? 1.0 : 0.5));
+  sym_eigen_dev<6>(info, w, V);
+#pragma unroll
+  for (int c = 0; c < 6; ++c) {
+    int m = 0;
+#pragma unroll
+    for (int r = 1; r < 6; ++r) if (fabs(V[r * 6 + c]) > fabs(V[m * 6 + c])) m = r;
+    if (V[m * 6 + c] < 0.0)
+#pragma unroll
+      for (int r = 0; r < 6; ++r) V[r * 6 + c] = -V[r * 6 + c];
+  }
+  *pd = (w[0] > 0.0 && w[0] >= 1e-14 * w[5]) ? 1 : 0;
+  double inv[6];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) inv[k] = *pd ? 1.0 / w[k] : 0.0;
+#pragma unroll
+  for (int i = 0; i < 6; ++i)
+#pragma unroll
+    for (int j = i; j < 6; ++j) {
+      double s = 0.0;
+#pragma unroll
+      for (int k = 0; k < 6; ++k) s += (V[i * 6 + k] * inv[k]) * V[j * 6 + k];
+      cov[i * 6 + j] = s; cov[j * 6 + i] = s;
+    }
+}
+// One thread per (lane, stage): the derived fields of every record at once (frame is the host's, filled in by lvo_probe_fetch).  A
+// record whose stage did not solve on its last run (first odometry frame, map too small) reports zero information.
+__global__ void k_pose_uncertainty(const LvoUncRaw* __restrict__ raw, lvo_pose_uncertainty* __restrict__ out, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const LvoUncRaw& r = raw[i];
+  lvo_pose_uncertainty& o = out[i];
+  const bool solved = r.solved != 0;
+  double H[21];
+  for (int k = 0; k < 21; ++k) H[k] = solved ? r.H[k] : 0.0;
+  o.frame = -1; o.solved = solved ? 1 : 0; o.n_factors = solved ? r.n_factors : 0; o.reserved = 0; o.cost = solved ? r.cost : 0.0;
+  pose_uncertainty_derive(H, o.information, o.covariance, o.eigenvalues, o.eigenvectors, &o.positive_definite);
 }
 
 // one CTA per lane (max_slots is kept for the call sites; the factor loop is strided over the CTA whatever the count)

@@ -96,6 +96,15 @@ class ScanRegistration {
   std::vector<lvo_point> buf_[5];
 };
 
+namespace detail {
+inline bool covariance(Context& c, int probe, double covariance[36]) {
+  lvo_pose_uncertainty u;
+  c.check(lvo_probe_fetch(c.get(), 0, probe, &u, sizeof(u), nullptr));
+  for (int k = 0; k < 36; ++k) covariance[k] = u.covariance[k];
+  return u.positive_definite != 0;
+}
+}  // namespace detail
+
 class LaserOdometry {
  public:
   explicit LaserOdometry(Context& c) : c_(c) {}
@@ -128,6 +137,10 @@ class LaserOdometry {
     c_.check(lvo_transform_cloud(c_.get(), view_of(laserCloudFullRes), nullptr, 1, &o));
     detail::store(buf_, o.n, laserCloudFullRes);
   }
+  // Covariance of T_last_curr from the last process() (lvo_pose_uncertainty::covariance, row-major 6 x 6 in (tx, ty, tz, rx, ry, rz),
+  // the layout of nav_msgs::Odometry::pose.covariance): all zeros, and false, on the first frame or when the problem does not constrain
+  // every direction (lvo_pose_uncertainty::positive_definite).
+  bool motionCovariance(double covariance[36]) { return detail::covariance(c_, LVO_P_ODO_UNCERTAINTY, covariance); }
 
  private:
   Context& c_;
@@ -164,6 +177,9 @@ class LaserMapping {
   // Localisation in a fixed prior map (lvo_set_lane_map_update): false skips the insertion and re-filter of :737-801 on the
   // following frames, so an imported map is registered against but not changed; true (the default) maps as the reference does.
   void setMapUpdate(bool update) { c_.check(lvo_set_lane_map_update(c_.get(), 0, update ? 1 : 0)); }
+  // Covariance of T_w_curr from the last process(), for the pose.covariance of /aft_mapped_to_init (the reference leaves it zero);
+  // same layout and return value as LaserOdometry::motionCovariance.
+  bool poseCovariance(double covariance[36]) { return detail::covariance(c_, LVO_P_MAP_UNCERTAINTY, covariance); }
 
  private:
   template <class Cloud>

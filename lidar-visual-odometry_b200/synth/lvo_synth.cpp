@@ -34,7 +34,9 @@ struct Scene {
   uint64_t seed;
   double ground_z = -1.73;
   double wall_y = 8.0, seg_len = 4.0;
+  bool features = true;   // false: ground and two flat facades only (a tunnel: translation along x is unobservable)
   double recess(long k, int side) const {
+    if (!features) return 0.0;
     uint64_t h = hash3(seed, (uint64_t)(k + (1l << 40)), (uint64_t)(side + 7));
     int r = (int)(h % 5);
     return r == 0 ? 1.2 : (r == 1 ? 0.6 : 0.0);
@@ -122,6 +124,7 @@ struct Scene {
     if (d[2] < -1e-12) t = (ground_z - o[2]) / d[2];
     double tf = hit_facade(o, d, +1); if (tf < t) t = tf;
     tf = hit_facade(o, d, -1); if (tf < t) t = tf;
+    if (!features) return t;
     double lim = t < 130.0 ? t : 130.0;
     double tp = hit_poles(o, d, lim); if (tp < t) t = tp;
     double tb = hit_boxes(o, d, lim); if (tb < t) t = tb;
@@ -183,13 +186,15 @@ long lvo_synth_rays(int model) { return model == 16 ? 16L * 1800 : 64L * 1875; }
 // ground-truth sensor pose (q xyzw, t) in the frame of sweep 0 of the same sequence.  Returns the number of points,
 // or -1 if cap is too small / the model is unknown.
 // naz = azimuth columns per sweep (0: the model's default).
-static long synth_sweep(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7, bool moving, int naz = 0) {
+static long synth_sweep(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7, bool moving, int naz = 0,
+                        bool features = true) {
   if (model != 16 && model != 64) return -1;
   const int beams = model;
   if (naz == 0) naz = model == 16 ? 1800 : 1875;
   if (naz < 1 || cap < (long)beams * naz) return -1;
   Scene sc;
   sc.seed = 1000ull * (uint64_t)model + 10ull * (uint64_t)seq;
+  sc.features = features;
   Pose P, P0;
   double pa[6], pb[6];
   pose_params(seq, frame, speed, pa);
@@ -263,6 +268,18 @@ long lvo_synth_sweep_moving(int model, int seq, int frame, double speed, float* 
 // that spin slower or fire faster, e.g. a VLP-16 at 5 Hz (~3600 columns).  out[cap] needs model * naz entries.
 long lvo_synth_sweep_res(int model, int seq, int frame, double speed, int naz, float* out_xyzi, long cap, double* gt_pose7) {
   return synth_sweep(model, seq, frame, speed, out_xyzi, cap, gt_pose7, false, naz);
+}
+// Same beam pattern, trajectory and noise as lvo_synth_sweep, cast into the same street with its recesses, poles and boxes removed:
+// the ground plane and two flat facades, parallel to the world x axis.  Translation along the street is unobservable there, the
+// degenerate case of a straight tunnel or corridor.  street_axis3 (optional) gets the world x axis in the sensor frame of sweep 0 (the
+// odometry and map origin).
+long lvo_synth_sweep_tunnel(int model, int seq, int frame, double speed, float* out_xyzi, long cap, double* gt_pose7, double* street_axis3) {
+  if (street_axis3) {
+    Pose P0;
+    pose_of(seq, 0, speed, P0);
+    for (int r = 0; r < 3; ++r) street_axis3[r] = P0.R[0 * 3 + r];   // R0^T e_x
+  }
+  return synth_sweep(model, seq, frame, speed, out_xyzi, cap, gt_pose7, false, 0, false);
 }
 
 }  // extern "C"
